@@ -12,6 +12,13 @@ Nit = 80.  N > 1: the same cube sharded as row stripes, one rank per GPU (strong
 
 --impl reference: the CPU port of the reference path (oracle/, NumPy+BLAS on all host threads) on a
 bounded patch sample of the same workload.
+
+--dump-outputs DIR: after the timed steps, write what the last timed step computed as DIR/<name>.npy (float32), so that
+two builds can be compared output for output on the same seeded inputs.  The GPU arms write the ADMM state a caller
+receives (X.npy, lambda_1.npy, lambda_2.npy); where the three full arrays exceed DUMP_BYTES, the same fixed, seeded
+sample of rows (dump_rows) is written for all three.  The reference arms write Phi_z.npy of their fixed patch sample.
+Two runs of the same build agree to about 1e-7 rel-L2, not bit for bit: the SVT's Gram matrix is summed with fp64
+atomics in whatever order the blocks finish (cfg4 on one B200 at 1000 W: X 8e-9, lambda_2 2e-7).
 """
 from __future__ import annotations
 
@@ -36,6 +43,8 @@ WORKLOADS = {
 }
 K_ATOMS, NIT, BB, STRIDE = 256, 80, 8, 1
 METRIC, UNIT = "ista_patch_iters_per_s", "patch-iters/s"
+DUMP_BYTES = 48 << 20      # --dump-outputs writes at most this much in all
+STATE = ("X", "lambda_1", "lambda_2")
 
 
 # The contract is ONE JSON line on stdout.  Libraries write there too (NCCL prints its version banner on the first
@@ -89,6 +98,39 @@ def make_inputs(workload):
     return Y, pm, D
 
 
+# ---------------------------------------------------------------------------------------------- --dump-outputs
+def dump_rows(R, C):
+    """Rows of the R x C ADMM state that --dump-outputs writes: all of them when X, lambda_1 and lambda_2 fit DUMP_BYTES,
+    else as many as fit, drawn with a fixed seed and sorted (the same rows in every run)."""
+    keep = min(R, DUMP_BYTES // (len(STATE) * C * 4))
+    if keep == R:
+        return np.arange(R)
+    return np.sort(np.random.default_rng(0).choice(R, keep, replace=False))
+
+
+def state_rows(torch, dist, sol, st, rows, rank, world):
+    """X, lambda_1, lambda_2 at the global rows ``rows``, gathered on the host of rank 0 (None on the other ranks).  Each
+    rank contributes the rows it owns; stripes are in rank order, so the gathered rows stay sorted."""
+    mine = rows[(rows >= st.a) & (rows < st.a + sol.rows_owned)] - st.a
+    idx = torch.as_tensor(mine, device=sol.X.device)
+    part = {n: getattr(sol, n).index_select(0, idx).cpu().numpy() for n in STATE}
+    if world == 1:
+        return part
+    parts = [None] * world if rank == 0 else None
+    dist.gather_object(part, parts, dst=0)
+    return {n: np.concatenate([p[n] for p in parts]) for n in STATE} if rank == 0 else None
+
+
+def write_outputs(out_dir, arrays):
+    arrays = {n: np.ascontiguousarray(a, dtype=np.float32) for n, a in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_BYTES:
+        raise SystemExit(f"bench.py: --dump-outputs would write {total} bytes, more than {DUMP_BYTES}")
+    os.makedirs(out_dir, exist_ok=True)
+    for n, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{n}.npy"), a)
+
+
 # ---------------------------------------------------------------------------------------------- CPU arm
 CPU_SAMPLE_ROWS = 192      # FIXED sample: the first 192 unfolded rows = 185 patch row starts x ALL column starts
 
@@ -122,13 +164,13 @@ def cpu_sample(Y):
 def cpu_pass(sub, D):
     """ONE pass of the oracle port (NumPy restatement of main_LRS_PnP.py:259-303, BLAS on all host threads) over the
     sample: im2col of the observed and current matrices, step constants, Nit masked soft-ISTA iterations, Phi_z.
-    Returns (patches, seconds)."""
+    Returns (patches, seconds, Phi_z)."""
     from oracle import lrs_oracle as orc
 
     oprm = orc.Params(Nit=NIT, bb=BB, slidingDis=STRIDE, step="spectral")
     t0 = time.perf_counter()
     phi, _ = orc.sparse_step(sub, np.zeros_like(sub), sub, D, oprm)
-    return phi.shape[1], time.perf_counter() - t0
+    return phi.shape[1], time.perf_counter() - t0, phi
 
 
 def sample_text(P_s, rows, C):
@@ -144,7 +186,7 @@ def cpu_patch_iters_per_s(Y, D, budget_s=15.0):
     cpu_pass(sub, D)
     times, t_end = [], time.perf_counter() + budget_s
     while True:
-        P_s, dt = cpu_pass(sub, D)
+        P_s, dt, _ = cpu_pass(sub, D)
         times.append(dt)
         if time.perf_counter() + dt > t_end:
             break
@@ -161,9 +203,11 @@ def run_reference(args, rank):
     threads = use_all_host_threads()
     times, P_s = [], 0
     for i in range(args.warmup + args.steps):
-        P_s, dt = cpu_pass(sub, D)
+        P_s, dt, phi = cpu_pass(sub, D)
         if i >= args.warmup:
             times.append(dt)
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, {"Phi_z": phi})
     mean = float(np.mean(times))
     val = P_s * NIT / mean
     R, C = Y.shape
@@ -388,6 +432,10 @@ def run_ours(args, rank, world, local_rank):
     sol.validate()
     launches = int(L.lrs_launch_count() - launches0)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        state = state_rows(torch, dist, sol, st, dump_rows(R, C), rank, world)
+        if rank == 0:
+            write_outputs(args.dump_outputs, state)
     ms = torch.tensor([e0.elapsed_time(e1)], device=dev, dtype=torch.float64)
     kms = torch.tensor([float(np.mean([a.elapsed_time(b) for a, b in kern_ev]))], device=dev, dtype=torch.float64)
     if world > 1:
@@ -525,8 +573,8 @@ def cfg1_cpu_pass(Y, D):
     from oracle import literal_loop as ll, lrs_oracle as orc
 
     blocks, _, _, _ = orc.get_image_block(Y, CFG1_BB, CFG1_BB)
-    _, dt = ll.sparse_step_literal(blocks, blocks, D, 0.1, CFG1_NIT, "spectral", patches=np.array(CFG1_SAMPLE))
-    return len(CFG1_SAMPLE), dt
+    phi, dt = ll.sparse_step_literal(blocks, blocks, D, 0.1, CFG1_NIT, "spectral", patches=np.array(CFG1_SAMPLE))
+    return len(CFG1_SAMPLE), dt, phi
 
 
 def run_cfg1_reference(args, rank):
@@ -536,9 +584,11 @@ def run_cfg1_reference(args, rank):
     threads = use_all_host_threads()
     times = []
     for i in range(args.warmup + args.steps):
-        P_s, dt = cfg1_cpu_pass(Y, D)
+        P_s, dt, phi = cfg1_cpu_pass(Y, D)
         if i >= args.warmup:
             times.append(dt)
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, {"Phi_z": phi})
     mean = float(np.mean(times))
     val = P_s * CFG1_NIT / mean
     sample = f"{P_s} of the 144 patches (indices {list(CFG1_SAMPLE)}) x {CFG1_NIT} iterations per pass, literal per-patch loop with one SVD per patch"
@@ -597,7 +647,7 @@ def run_cfg1_ours(args):
     sampler.start()
     launches0 = L.lrs_launch_count()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    reps = max(args.steps, 1)
+    reps = args.steps
     e0.record()
     for _ in range(reps):
         one_step()
@@ -607,6 +657,8 @@ def run_cfg1_ours(args):
     clocks = sampler.stop()
     if not bool(torch.isfinite(sol.X).all()):
         raise SystemExit("bench.py: non-finite ADMM state")
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, {n: getattr(sol, n).cpu().numpy() for n in STATE})
     ms_per_step = e0.elapsed_time(e1) / reps
     kms = float(np.mean([a.elapsed_time(b) for a, b in kern_ev]))
     # end to end: host buffers in, a fresh solver, one outer iteration, X back on the host
@@ -637,7 +689,7 @@ def run_cfg1_ours(args):
     if not args.no_cpu:
         threads = use_all_host_threads()
         cfg1_cpu_pass(Y, D)
-        P_s, dt = cfg1_cpu_pass(Y, D)
+        P_s, dt, _ = cfg1_cpu_pass(Y, D)
         cpu = {"value": P_s * CFG1_NIT / dt, "unit": UNIT, "cores": threads, "kind": "port",
                "sample": f"{P_s} of the 144 patches x {CFG1_NIT} iterations, literal per-patch loop with one SVD per patch (B0)"}
     emit({
@@ -677,7 +729,11 @@ def main():
     ap.add_argument("--range-mb", type=int, default=None,
                     help="experiment: size (MiB) of each of the two Phi_z range buffers (default: SparseCoder.CHUNK_BYTES)")
     ap.add_argument("--cpu-seconds", type=float, default=15.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed as DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     claim_stdout()                                  # stdout carries the one JSON line and nothing else
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

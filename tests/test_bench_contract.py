@@ -62,6 +62,39 @@ def test_bench_state_schedule_stays_finite_on_the_oracle():
     assert g[-1] > 100 * g[1] and all(g[i + 1] > 1.5 * g[i] for i in range(5, 11))
 
 
+def test_reference_arm_dumps_its_last_pass(tmp_path):
+    """--dump-outputs: the reference arm writes the Phi_z of its last timed pass over the fixed sample, in float32."""
+    import numpy as np
+
+    import bench
+    from oracle import lrs_oracle as orc
+
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--workload", "mini",
+                          "--steps", "1", "--warmup", "0", "--dump-outputs", str(tmp_path)], capture_output=True, text=True,
+                         timeout=300)
+    assert out.returncode == 0, out.stderr[-2000:]
+    phi = np.load(tmp_path / "Phi_z.npy")
+    Y, _, D = bench.make_inputs("mini")
+    sub = bench.cpu_sample(Y)
+    oprm = orc.Params(Nit=bench.NIT, bb=bench.BB, slidingDis=bench.STRIDE, step="spectral")
+    want, _ = orc.sparse_step(sub, np.zeros_like(sub), sub, D, oprm)
+    assert phi.dtype == np.float32 and phi.shape == want.shape
+    assert np.linalg.norm(phi - want) <= 1e-6 * np.linalg.norm(want)
+
+
+def test_dump_row_sample_is_fixed_and_fits():
+    import numpy as np
+
+    import bench
+
+    for R, C in ((262144, 191), (1048576, 224)):
+        rows = bench.dump_rows(R, C)
+        assert len(rows) * C * 4 * len(bench.STATE) <= bench.DUMP_BYTES and len(rows) > 10000
+        assert np.all(np.diff(rows) > 0) and rows[-1] < R
+        assert np.array_equal(rows, bench.dump_rows(R, C))
+    assert np.array_equal(bench.dump_rows(4096, 32), np.arange(4096))         # small states are written whole
+
+
 def test_reference_arm_other_ranks_exit_silently():
     """Under torchrun (N > 1) rank 0 alone runs the CPU reference arm; the other ranks exit 0 without work."""
     env = dict(os.environ, RANK="1", LOCAL_RANK="1", WORLD_SIZE="2")

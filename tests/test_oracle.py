@@ -29,8 +29,11 @@ def test_index_kat_bit_exact(golden):
         assert np.array_equal(x, g[f"c{ci}_x"]), (R, C, bb, s)
         assert np.array_equal(y, g[f"c{ci}_y"]), (R, C, bb, s)
         assert orc.idx_mat(R, C, bb, s).sum() == g[f"c{ci}_idxsum"][0]
-        blocks, x2, y2, _ = orc.get_image_block(g[f"c{ci}_X"], bb, s)
+        blocks, x2, y2, idx = orc.get_image_block(g[f"c{ci}_X"], bb, s)
         assert blocks.dtype == np.float32 and x2.dtype == np.int64
+        # the reference's x, y are the argwhere of its 0/1 idx_Mat: with the stored sum they fix every 1 of idx_Mat
+        assert idx.shape == (R - bb + 1, C - bb + 1) and np.isin(idx, (0, 1)).all()
+        assert (idx[g[f"c{ci}_x"], g[f"c{ci}_y"]] == 1).all() and idx.sum() == g[f"c{ci}_idxsum"][0] == len(x)
         if f"c{ci}_blocks" in g:
             assert np.array_equal(blocks, g[f"c{ci}_blocks"])
         else:

@@ -68,7 +68,10 @@ def _problem(H=10, W=9):
     return Y, MtM, D, prm
 
 
-def _worker(rank, world, port, iters, out_dir, H=10, W=9):
+DUMP_TEST_BYTES = 30 * 3 * 14 * 4          # bench.DUMP_BYTES that makes the 90 x 14 state of _problem() a 30-row sample
+
+
+def _worker(rank, world, port, iters, out_dir, H=10, W=9, dump=False):
     os.environ["MASTER_ADDR"] = "127.0.0.1"
     os.environ["MASTER_PORT"] = str(port)
     dist.init_process_group("gloo", rank=rank, world_size=world)
@@ -82,7 +85,17 @@ def _worker(rank, world, port, iters, out_dir, H=10, W=9):
         sol = solver.LRSPnP(Yl, Ml, D, prm, stripe=st, backend=be)
         sol.run(iters)
         np.savez(os.path.join(out_dir, f"rank{rank}.npz"), X=sol.X.numpy()[:st.rows_owned], a=st.a,
-                 l1=sol.lambda_1.numpy()[:st.rows_owned], halo_X=sol.X.numpy()[st.rows_owned:])
+                 l1=sol.lambda_1.numpy()[:st.rows_owned], l2=sol.lambda_2.numpy()[:st.rows_owned],
+                 halo_X=sol.X.numpy()[st.rows_owned:])
+        if dump:                                         # what bench.py --dump-outputs gathers on N ranks
+            import bench
+
+            bench.DUMP_BYTES = DUMP_TEST_BYTES
+            got = bench.state_rows(torch, dist, sol, st, bench.dump_rows(*Y.shape), rank, world)
+            if rank == 0:
+                np.savez(os.path.join(out_dir, "dump.npz"), **got)
+            else:
+                assert got is None
     finally:
         dist.destroy_process_group()
 
@@ -115,6 +128,29 @@ def test_sharded_equals_unsharded(world, tmp_path):
     err = np.linalg.norm(X - ref.X) / np.linalg.norm(ref.X)
     assert err < 2e-5, err
     assert np.linalg.norm(l1 - ref.lambda_1) / np.linalg.norm(ref.lambda_1) < 1e-4
+
+
+def test_bench_dump_gathers_sampled_rows_over_stripes(tmp_path, monkeypatch):
+    """bench.py --dump-outputs on N ranks: the fixed row sample (forced here by a small DUMP_BYTES) is gathered on rank 0
+    from the stripes that own its rows, the last rank's trailing bb-1 rows included, in row order and unchanged."""
+    import bench
+
+    world = 3
+    mp.spawn(_worker, args=(world, _free_port(), 2, str(tmp_path), 10, 9, True), nprocs=world, join=True)
+    Y, _, _, prm = _problem()
+    R, C = Y.shape
+    monkeypatch.setattr(bench, "DUMP_BYTES", DUMP_TEST_BYTES)
+    rows = bench.dump_rows(R, C)
+    assert len(rows) == 30 and rows[-1] >= R - (prm.bb - 1)
+    full = {n: np.full_like(Y, np.nan) for n in bench.STATE}
+    for r in range(world):
+        z = np.load(tmp_path / f"rank{r}.npz")
+        a = int(z["a"])
+        for n, key in zip(bench.STATE, ("X", "l1", "l2")):
+            full[n][a:a + z[key].shape[0]] = z[key]
+    got = np.load(tmp_path / "dump.npz")
+    for n in bench.STATE:
+        assert got[n].dtype == np.float32 and np.array_equal(got[n], full[n][rows]), n
 
 
 def test_stripes_as_narrow_as_the_halo(tmp_path):

@@ -50,7 +50,7 @@ extern "C" {
 
 /* engines of lrs_sparse_step_fused_f32 */
 #define LRS_ENGINE_AUTO 0
-#define LRS_ENGINE_SIMT 1   /* fp32 FFMA kernel (any K multiple of 16 up to 256)          */
+#define LRS_ENGINE_SIMT 1   /* fp32 FFMA kernel (K in {64,128,192,256})                   */
 #define LRS_ENGINE_TC 2     /* tcgen05/TMEM kernel, 3-pass fp16 split (n = 64, K in {64,128,192,256}) */
 /* OR-ed into `engine`: the tcgen05 kernel's CTAs CLAIM their work items from a device counter instead of being dealt them,
  * for a launch that shares the GPU with another kernel (CTAs that start late take fewer items).  Costs ~4 % in cycles

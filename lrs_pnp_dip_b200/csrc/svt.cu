@@ -257,6 +257,7 @@ __global__ void __launch_bounds__(64) spectral_table_kernel(const double* __rest
         __syncthreads();
         double nrm2 = 0.0;
         for (int i = 0; i < n; ++i) nrm2 += red[i];                 // every thread: same order, same value
+        __syncthreads();                                            // all reads of red[] done before it is rewritten below
         if (nrm2 <= 0.0) {
             lam = 0.0;
             break;

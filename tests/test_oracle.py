@@ -275,3 +275,28 @@ def test_svt_through_the_b_form_of_a_one_sided_jacobi_sweep():
         got = Z.astype(np.float64) @ W
         want = orc.svt(Z, tau)
         assert np.linalg.norm(got - want) <= 1e-5 * np.linalg.norm(want)
+
+
+# ---------------------------------------------------------------- helpers of tests/test_kernel_edges.py (CPU self-checks)
+def test_de_bruijn_rows_carry_every_row_pattern_once():
+    """The de Bruijn row mask of the fused-step edge test: its 2^n row starts see every n-row validity pattern once."""
+    from tests.test_kernel_edges import de_bruijn_rows, row_patterns
+
+    for n in (3, 8):
+        rows = de_bruijn_rows(n)
+        assert rows.shape == ((1 << n) + n - 1,)
+        pats = row_patterns(rows, np.arange(1 << n), bb=n)
+        assert sorted(pats.tolist()) == list(range(1 << n)), n
+
+
+def test_svt_fp64_restatement_vs_svd():
+    """The fp64 SVT restatement (Gram matrix, eigh, max(1 - tau/sigma, 0), recomposition) equals U soft(S, tau) V^T of an
+    fp64 SVD, with tau at 0, mid-spectrum, exactly at a singular value and above the largest one."""
+    from tests.test_kernel_edges import svt_fp64
+
+    rng = np.random.default_rng(5)
+    Z = rng.standard_normal((300, 5)) @ rng.standard_normal((5, 17)) + 0.05 * rng.standard_normal((300, 17))
+    U, S, Vt = np.linalg.svd(Z, full_matrices=False)
+    for tau in (0.0, float(np.median(S)), float(S[2]), 2.0 * float(S[0])):
+        want = (U * np.maximum(S - tau, 0.0)) @ Vt
+        assert np.abs(svt_fp64(Z, tau) - want).max() <= 1e-10 * np.abs(Z).max(), tau

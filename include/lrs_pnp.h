@@ -118,6 +118,26 @@ size_t lrs_spectral_table_workspace_bytes(int bb);
 int lrs_spectral_table_f32(const float* D_dev, int K, int bb, int step, float* table_dev, void* workspace_dev,
                            size_t workspace_bytes, lrs_stream_t stream);
 
+/* Per-patch step constants for ANY mask (bb <= 8), in two stages; the caller merges equal words in between
+ * (ops.patch_step_constants).  Together they replace np.linalg.norm(H, 2)**2 with H = D minus the patch's missing rows
+ * (main_LRS_PnP.py:134, :276-289), paid per patch per outer iteration in the reference, by one value per distinct mask
+ * pattern per dictionary; the result feeds a_patch_dev of lrs_sparse_step_fused_f32 or a_dev of lrs_ista_pnp_f32.
+ *
+ * words_dev[p - p_begin] for the patches p in [p_begin, p_end) (reference order): bit k set iff element k of the patch
+ * (window row k % bb, column k / bb) is observed, Yobs != 0.0f as in the fused kernels (-0.0 missing, NaN observed).
+ * Any stride. */
+int lrs_patch_mask_words_u64(const float* Yobs_dev, int64_t R, int64_t C, int bb, int s, int64_t p_begin, int64_t p_end,
+                             uint64_t* words_dev, lrs_stream_t stream);
+/* a_dev[i] for each pattern word words_dev[i] (bit k = row k of D [n, K], n <= 64): LRS_STEP_SPECTRAL lambda_max of
+ * G[S,S], G = D D^T in fp64 (fp64 Lanczos), LRS_STEP_FROB4 4 tr G[S,S]; the empty pattern gives exactly 0.  Equal words
+ * give bit-identical values.  count_dev: NULL -> all max_count words; else a device int64 holding how many of the
+ * max_count words to process (the launch is sized for max_count and reads the count on the device: no host
+ * synchronisation). */
+size_t lrs_spectral_patterns_workspace_bytes(int n);
+int lrs_spectral_patterns_f32(const float* D_dev, int n, int K, const uint64_t* words_dev, int64_t max_count,
+                              const int64_t* count_dev, int step, float* a_dev, void* workspace_dev, size_t workspace_bytes,
+                              lrs_stream_t stream);
+
 /* ---- batched soft-ISTA on explicit patch matrices ------------------------------------------- */
 /* For every patch p: alpha=0; repeat Nit: alpha <- soft(alpha + D^T(m.*(y - D alpha))/a_p, lambda/(2 a_p))
  * with m = (blocks_copy[:,p] != 0)  [row deletion of main_LRS_PnP.py:276-289 in masked form],

@@ -43,6 +43,9 @@ SIGNATURES = {
     "lrs_step_frob4_f32": (_int, [_p, _p, _int, _int, _i64, _p, _p]),
     "lrs_spectral_table_workspace_bytes": (C.c_size_t, [_int]),
     "lrs_spectral_table_f32": (_int, [_p, _int, _int, _int, _p, _p, C.c_size_t, _p]),
+    "lrs_patch_mask_words_u64": (_int, [_p, _i64, _i64, _int, _int, _i64, _i64, _p, _p]),
+    "lrs_spectral_patterns_workspace_bytes": (C.c_size_t, [_int]),
+    "lrs_spectral_patterns_f32": (_int, [_p, _int, _int, _p, _i64, _p, _int, _p, _p, C.c_size_t, _p]),
     "lrs_ista_workspace_bytes": (C.c_size_t, [_int, _int, _i64]),
     "lrs_ista_soft_f32": (_int, [_p, _p, _p, _p, _f, _int, _int, _int, _i64, _p, _p, _p, C.c_size_t, _p]),
     "lrs_ista_pnp_f32": (_int, [_p, _p, _p, _p, _f, _int, _int, _int, _i64, _int, _f, _p, _p, _p, C.c_size_t, _p]),

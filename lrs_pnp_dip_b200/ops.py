@@ -229,6 +229,65 @@ def row_pattern_table(D: torch.Tensor, bb: int, step: str) -> torch.Tensor:
 
 _TABLE_CACHE: dict = {}
 
+# patches whose words are merged in one pass of patch_step_constants: bounds its transient memory (~80 B per patch of a
+# pass: the words, the sort's keys, indices and scratch, the group numbers and representatives) whatever P is
+PATCH_CONSTANTS_CHUNK = 1 << 25
+
+
+def patch_step_constants(Y_observed, D, bb: int, s: int, step: str = "spectral", p_begin: int = 0,
+                         p_end: Optional[int] = None):
+    """a[p] = ||M_p D||_2^2 (``step='spectral'``, np.linalg.norm(H, 2)**2 of main_LRS_PnP.py:134) or 4||M_p D||_F^2
+    (``'frob4'``) for the patches p in [p_begin, p_end) of the observed matrix, M_p = the patch's own observed entries
+    (``Y_observed != 0``, main_LRS_PnP.py:276-289), for ANY mask, bb <= 8.
+
+    Each patch's validity is one 64-bit word (lrs_patch_mask_words_u64).  The word IS the pattern, so equal patterns are
+    merged exactly, on the device and without a host synchronisation: sort, mark where a run of equal words starts,
+    cumsum for the group number, scatter one representative per group.  lrs_spectral_patterns_f32 then runs once per
+    distinct word (it reads the number of groups on the device) and the values are gathered back to the patches."""
+    bb, s = int(bb), int(s)
+    if not 1 <= bb <= 8:
+        raise ValueError(f"per-patch step constants pack a patch's mask into 64 bits: bb <= 8 (got bb = {bb})")
+    mode = {"spectral": _lib.STEP_SPECTRAL, "frob4": _lib.STEP_FROB4}.get(step)
+    if mode is None:
+        raise ValueError(f"unknown step mode {step!r}")
+    Y, src, was_np = _to_dev(Y_observed)
+    if Y.dim() != 2:
+        raise ValueError("Y_observed must be a 2-D (pixels x bands) matrix")
+    R, C = Y.shape
+    Dd = torch.as_tensor(D).to(device=Y.device, dtype=torch.float32).contiguous()
+    n, K = Dd.shape
+    if n != bb * bb:
+        raise ValueError(f"dictionary has {n} rows, bb² = {bb * bb}")
+    P = patch_count(R, C, bb, s)
+    p_end = P if p_end is None else int(p_end)
+    p_begin = int(p_begin)
+    if not 0 <= p_begin <= p_end <= P:
+        raise ValueError(f"patch range [{p_begin}, {p_end}) outside [0, {P}]")
+    L = lib()
+    with torch.cuda.device(Y.device):
+        a = torch.empty(p_end - p_begin, dtype=torch.float32, device=Y.device)
+        ws_bytes = L.lrs_spectral_patterns_workspace_bytes(n)
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=Y.device)
+        for c0 in range(p_begin, p_end, PATCH_CONSTANTS_CHUNK):
+            c1 = min(p_end, c0 + PATCH_CONSTANTS_CHUNK)
+            m = c1 - c0
+            words = torch.empty(m, dtype=torch.int64, device=Y.device)
+            check(L.lrs_patch_mask_words_u64(ptr(Y), R, C, bb, s, c0, c1, ptr(words), stream_ptr()), "lrs_patch_mask_words_u64")
+            sw, order = torch.sort(words)                  # int64 order of the uint64 words: any order groups equal words
+            del words
+            start = torch.ones(m, dtype=torch.bool, device=Y.device)
+            torch.ne(sw[1:], sw[:-1], out=start[1:])
+            group = torch.cumsum(start, 0, dtype=torch.int64).sub_(1)     # group number of each sorted word
+            del start
+            uniq = torch.empty_like(sw).scatter_(0, group, sw)    # the words of a group are equal: any writer is right
+            count = group[-1:] + 1                                 # number of distinct words, stays on the device
+            vals = torch.empty(m, dtype=torch.float32, device=Y.device)
+            check(L.lrs_spectral_patterns_f32(ptr(Dd), n, K, ptr(uniq), m, ptr(count), mode, ptr(vals), ptr(ws), ws_bytes,
+                                              stream_ptr()), "lrs_spectral_patterns_f32")
+            a[c0 - p_begin:c1 - p_begin].index_copy_(0, order, vals.index_select(0, group))
+            del sw, order, group, uniq, vals
+    return _back(a, src, was_np)
+
 
 def _row_pattern_table(D: torch.Tensor, bb: int, step: str) -> torch.Tensor:
     n, K = D.shape

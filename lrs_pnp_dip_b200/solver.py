@@ -42,7 +42,14 @@ def _on(t):
 @dataclass
 class Params:
     """Hyper-parameters, SURVEY Appendix C.  Defaults = main_LRS_PnP.py:218-238;
-    DIP variants: mu_1 = mu_2 = 0.1, Nit = 100, step = 'frob4' (main_LRS_PnP_DIP_pro.py:324-341,190)."""
+    DIP variants: mu_1 = mu_2 = 0.1, Nit = 100, step = 'frob4' (main_LRS_PnP_DIP_pro.py:324-341,190).
+
+    ``step`` — the ISTA step constant a_p of each patch:
+      'spectral'        ||M_p D||_2^2 (main_LRS_PnP.py:134).  On the fused engines it comes from the 256-entry row-pattern
+                        table, which needs masks replicated over the bands (per-element masks are refused).
+      'spectral_patch'  the same value from each patch's own 64-bit validity pattern, for ANY mask (bb <= 8): one fp64
+                        Lanczos run per distinct pattern at construction (ops.patch_step_constants), 4 B per patch kept.
+      'frob4'           4||M_p D||_F^2 (main_LRS_PnP_DIP_pro.py:190), a different step rule."""
     gamma: float = 0.5
     mu_1: float = 0.15
     mu_2: float = 0.15 * 6
@@ -162,6 +169,9 @@ class SparseCoder:
                 self.validate()
 
     def _init(self, Y_observed: torch.Tensor, D: torch.Tensor, prm: Params, engine: str):
+        if prm.step == "spectral_patch" and prm.bb > 8:
+            raise ValueError(f"step='spectral_patch' packs a patch's mask into 64 bits and needs bb <= 8 (got bb = {prm.bb}); "
+                             "use step='spectral' for explicit patch matrices")
         _lib.require_cuda()
         if Y_observed.device.type != "cuda" or D.device.type != "cuda":
             raise _lib.LrsError("SparseCoder needs CUDA tensors")
@@ -189,11 +199,17 @@ class SparseCoder:
                 self._bad_event = torch.cuda.Event()
                 self._bad_event.record()
                 self.a_table = ops.row_pattern_table(self.D, prm.bb, "spectral")
+            elif prm.step == "spectral_patch":
+                # any mask: one value per patch (the kernels' a_patch_dev, indexed by the global patch number)
+                self.a_patch = ops.patch_step_constants(self.Y, self.D, prm.bb, prm.slidingDis, "spectral")
             elif prm.step != "frob4":
                 raise ValueError(prm.step)
         else:
             self.blocks_copy = ops.im2col(self.Y, prm.bb, prm.slidingDis)
-            self.a_patch = ops.step_constants(self.blocks_copy, self.D, prm.step)
+            if prm.step == "spectral_patch":
+                self.a_patch = ops.patch_step_constants(self.Y, self.D, prm.bb, prm.slidingDis, "spectral")
+            else:
+                self.a_patch = ops.step_constants(self.blocks_copy, self.D, prm.step)
 
     def validate(self, wait: bool = True) -> None:
         """Raise if the construction-time mask test failed.  ``wait=False`` only looks at a verdict that has
@@ -208,7 +224,8 @@ class SparseCoder:
         self._bad_event = None
         if bool(self._bad_host):
             raise _lib.LrsError("spectral step constants on the fused path need band-replicated masks "
-                                "(one validity flag per unfolded row); use step='frob4'")
+                                "(one validity flag per unfolded row); use step='spectral_patch' (the same spectral "
+                                "constant per patch, for any mask) or step='frob4' (a different step rule)")
 
     def phi_z(self, X: torch.Tensor, lambda_1: Optional[torch.Tensor]) -> torch.Tensor:
         """Phi_z [n, P] of main_LRS_PnP.py:259-303 for V = X + lambda_1/mu_1."""

@@ -68,11 +68,29 @@ def pixel_mask(H: int, W: int, kind: str = "bernoulli", keep: float = 0.5, seed:
     return m.reshape(-1).astype(np.uint8)
 
 
+def band_mask(H: int, W: int, B: int, keep: float = 0.7, band_frac: float = 0.25, dead_frac: float = 0.05,
+              seed: int = 5) -> np.ndarray:
+    """Per-element 0/1 mask ``[H, W, B]`` (uint8) with band-dependent missing data: a per-pixel Bernoulli(``keep``) mask
+    replicated over the bands, and in a random ``band_frac`` of the bands, each its own random ``dead_frac`` of the
+    image columns dropped (dead detector lines / stripes that affect only some bands).  Not band-replicated, but an 8 x 8
+    patch meets at most one dead column per band, so the distinct patch patterns stay moderate in number."""
+    rng = np.random.default_rng(seed)
+    m = np.repeat((rng.random((H, W)) < keep)[:, :, None], B, axis=2)
+    bands = np.flatnonzero(rng.random(B) < band_frac)
+    for b in bands:
+        m[:, rng.random(W) < dead_frac, b] = False
+    return m.astype(np.uint8)
+
+
 def observe(noisy: np.ndarray, pix_mask: np.ndarray) -> np.ndarray:
     """Apply the mask the way the reference detects it: missing entries are
     exactly 0.0 (main_LRS_PnP.py:276-278), and an observed exact zero is nudged
-    to 1e-12 so that ``== 0`` ⇔ masked."""
+    to 1e-12 so that ``== 0`` ⇔ masked.  ``pix_mask``: per pixel ``[H*W]``
+    (replicated over the bands), or per element ``[H*W, B]`` / ``[H, W, B]``."""
     Y = noisy.astype(F32).copy()
     Y[Y == 0] = F32(1e-12)
-    Y[pix_mask == 0, :] = 0
+    if pix_mask.ndim == 1:
+        Y[pix_mask == 0, :] = 0
+    else:
+        Y[pix_mask.reshape(Y.shape) == 0] = 0
     return Y

@@ -110,14 +110,6 @@ int lrs_axpy_f32(const float* x_dev, const float* l_dev, float c, float* out_dev
 int lrs_step_frob4_f32(const float* blocks_copy_dev, const float* D_dev, int n, int K, int64_t P, float* a_dev,
                        lrs_stream_t stream);
 
-/* table_dev[2^bb] (bb <= 8): step constant for every validity pattern of a patch's bb pixel rows (bit i = row r+i
- * observed; band-replicated masks, main_LRS_PnP.py:188-192): LRS_STEP_SPECTRAL ||M D||_2^2 (main_LRS_PnP.py:134) or
- * LRS_STEP_FROB4 (main_LRS_PnP_DIP_pro.py:190).  Replaces one SVD per patch per outer iteration by one table per
- * dictionary; feeds a_table_dev of lrs_sparse_step_fused_f32. */
-size_t lrs_spectral_table_workspace_bytes(int bb);
-int lrs_spectral_table_f32(const float* D_dev, int K, int bb, int step, float* table_dev, void* workspace_dev,
-                           size_t workspace_bytes, lrs_stream_t stream);
-
 /* Per-patch step constants for ANY mask (bb <= 8), in two stages; the caller merges equal words in between
  * (ops.patch_step_constants).  Together they replace np.linalg.norm(H, 2)**2 with H = D minus the patch's missing rows
  * (main_LRS_PnP.py:134, :276-289), paid per patch per outer iteration in the reference, by one value per distinct mask
@@ -132,7 +124,9 @@ int lrs_patch_mask_words_u64(const float* Yobs_dev, int64_t R, int64_t C, int bb
  * G[S,S], G = D D^T in fp64 (fp64 Lanczos), LRS_STEP_FROB4 4 tr G[S,S]; the empty pattern gives exactly 0.  Equal words
  * give bit-identical values.  count_dev: NULL -> all max_count words; else a device int64 holding how many of the
  * max_count words to process (the launch is sized for max_count and reads the count on the device: no host
- * synchronisation). */
+ * synchronisation).
+ * Run on the 2^bb row-pattern words (bit k set iff bit k % bb of the row pattern is set: band-replicated masks,
+ * main_LRS_PnP.py:188-192), it also fills a_table_dev of lrs_sparse_step_fused_f32: one table per dictionary. */
 size_t lrs_spectral_patterns_workspace_bytes(int n);
 int lrs_spectral_patterns_f32(const float* D_dev, int n, int K, const uint64_t* words_dev, int64_t max_count,
                               const int64_t* count_dev, int step, float* a_dev, void* workspace_dev, size_t workspace_bytes,

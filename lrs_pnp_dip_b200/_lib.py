@@ -41,8 +41,6 @@ SIGNATURES = {
     "lrs_soft_f32": (_int, [_p, _f, _p, _i64, _p]),
     "lrs_axpy_f32": (_int, [_p, _p, _f, _p, _i64, _p]),
     "lrs_step_frob4_f32": (_int, [_p, _p, _int, _int, _i64, _p, _p]),
-    "lrs_spectral_table_workspace_bytes": (C.c_size_t, [_int]),
-    "lrs_spectral_table_f32": (_int, [_p, _int, _int, _int, _p, _p, C.c_size_t, _p]),
     "lrs_patch_mask_words_u64": (_int, [_p, _i64, _i64, _int, _int, _i64, _i64, _p, _p]),
     "lrs_spectral_patterns_workspace_bytes": (C.c_size_t, [_int]),
     "lrs_spectral_patterns_f32": (_int, [_p, _int, _int, _p, _i64, _p, _int, _p, _p, C.c_size_t, _p]),

@@ -387,7 +387,7 @@ extern "C" {
 
 const char* lrs_last_error(void) { return lrs::g_err.c_str(); }
 
-int lrs_version(void) { return 101; }
+int lrs_version(void) { return 102; }
 
 uint64_t lrs_launch_count(void) { return (uint64_t)lrs::g_launches.load(); }
 

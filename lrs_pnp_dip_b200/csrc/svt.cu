@@ -204,102 +204,3 @@ int lrs_svt_apply_f32(const float* X_dev, const float* L_dev, float c, const flo
 }
 
 }  // extern "C"
-
-// ------------------------------------------------------------------------------------------------
-// Step-constant table for the fused sparse step (band-replicated masks): for each of the 2^bb validity patterns of
-// a patch's pixel rows, a = ||M D||_2^2 = lambda_max(M (D D^T) M)  (np.linalg.norm(H,2)**2, main_LRS_PnP.py:134) or
-// 4 ||M D||_F^2 (main_LRS_PnP_DIP_pro.py:190).  The reference pays an SVD per patch per outer iteration; here it is
-// one 2^bb-entry table per dictionary.  n = bb^2 <= 64.  fp64 power iteration on the n x n masked Gram matrix: the
-// Rayleigh quotient's error is sum_i (l1 - li) c_i^2, so near-degenerate top eigenvalues do not hurt its accuracy.
-// ------------------------------------------------------------------------------------------------
-namespace lrs {
-
-__global__ void __launch_bounds__(256) ddt_kernel(const float* __restrict__ D, int n, int K, double* __restrict__ G) {
-    for (int e = threadIdx.x + blockIdx.x * blockDim.x; e < n * n; e += blockDim.x * gridDim.x) {
-        int i = e / n, j = e % n;
-        double s = 0.0;
-        for (int k = 0; k < K; ++k) s = fma((double)D[(int64_t)i * K + k], (double)D[(int64_t)j * K + k], s);
-        G[e] = s;
-    }
-}
-
-__global__ void __launch_bounds__(64) spectral_table_kernel(const double* __restrict__ G0, int n, int bb, int frob4,
-                                                            float* __restrict__ table) {
-    __shared__ double G[64 * 65];
-    __shared__ double v[64], w[64], red[64];
-    const int pat = blockIdx.x, t = threadIdx.x;
-    const bool valid_t = t < n && ((pat >> (t % bb)) & 1);          // element k of a patch sits in pixel row k % bb
-    for (int e = t; e < n * n; e += 64) {
-        int i = e / n, j = e % n;
-        bool ok = ((pat >> (i % bb)) & 1) && ((pat >> (j % bb)) & 1);
-        G[i * 65 + j] = ok ? G0[e] : 0.0;
-    }
-    __syncthreads();
-    if (frob4) {
-        red[t] = valid_t ? G[t * 65 + t] : 0.0;
-        __syncthreads();
-        if (t == 0) {
-            double s = 0.0;
-            for (int i = 0; i < n; ++i) s += red[i];
-            table[pat] = (float)(4.0 * s);
-        }
-        return;
-    }
-    v[t] = valid_t ? 1.0 + 0.01 * t : 0.0;
-    __syncthreads();
-    double lam = 0.0, lam_prev = -1.0;
-    for (int it = 0; it < 40000; ++it) {
-        double s = 0.0;
-        if (t < n)
-            for (int j = 0; j < n; ++j) s = fma(G[t * 65 + j], v[j], s);
-        w[t] = t < n ? s : 0.0;
-        red[t] = t < n ? s * s : 0.0;
-        __syncthreads();
-        double nrm2 = 0.0;
-        for (int i = 0; i < n; ++i) nrm2 += red[i];                 // every thread: same order, same value
-        __syncthreads();                                            // all reads of red[] done before it is rewritten below
-        if (nrm2 <= 0.0) {
-            lam = 0.0;
-            break;
-        }
-        const double inv = rsqrt(nrm2);
-        // Rayleigh quotient of the previous (unit) iterate: v^T G v = v . w
-        red[t] = t < n ? v[t] * w[t] : 0.0;
-        __syncthreads();
-        double rq = 0.0;
-        for (int i = 0; i < n; ++i) rq += red[i];
-        __syncthreads();
-        v[t] = w[t] * inv;
-        __syncthreads();
-        if (it > 0) lam = rq;
-        if ((it & 31) == 31) {
-            if (fabs(lam - lam_prev) <= 1e-13 * fabs(lam)) break;
-            lam_prev = lam;
-        }
-    }
-    if (t == 0) table[pat] = (float)(lam > 0.0 ? lam : 0.0);
-}
-
-}  // namespace lrs
-
-extern "C" size_t lrs_spectral_table_workspace_bytes(int bb) { return bb > 0 && bb <= 8 ? (size_t)64 * 64 * sizeof(double) : 0; }
-
-extern "C" int lrs_spectral_table_f32(const float* D_dev, int K, int bb, int step, float* table_dev, void* workspace_dev,
-                                      size_t workspace_bytes, lrs_stream_t stream) {
-    const char* fn = "lrs_spectral_table_f32";
-    if (!D_dev || !table_dev || K <= 0) return lrs::fail_arg(fn, "bad arguments");
-    if (bb < 1 || bb > 8) return lrs::fail_arg(fn, "row-pattern tables exist for bb <= 8 (n <= 64)");
-    if (step != LRS_STEP_SPECTRAL && step != LRS_STEP_FROB4) return lrs::fail_arg(fn, "unknown step mode");
-    if (!workspace_dev || workspace_bytes < lrs_spectral_table_workspace_bytes(bb)) {
-        lrs::set_error(std::string(fn) + ": workspace smaller than lrs_spectral_table_workspace_bytes()");
-        return LRS_E_WORKSPACE;
-    }
-    const int n = bb * bb;
-    double* G = (double*)workspace_dev;
-    cudaStream_t st = (cudaStream_t)stream;
-    lrs::ddt_kernel<<<16, 256, 0, st>>>(D_dev, n, K, G);
-    LRS_CHECK_LAUNCH(fn);
-    lrs::spectral_table_kernel<<<1 << bb, 64, 0, st>>>(G, n, bb, step == LRS_STEP_FROB4, table_dev);
-    LRS_CHECK_LAUNCH(fn);
-    return LRS_OK;
-}

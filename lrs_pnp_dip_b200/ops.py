@@ -234,6 +234,26 @@ _TABLE_CACHE: dict = {}
 PATCH_CONSTANTS_CHUNK = 1 << 25
 
 
+_STEP_MODES = {"spectral": _lib.STEP_SPECTRAL, "frob4": _lib.STEP_FROB4}
+
+
+def _spectral_patterns(D: torch.Tensor, words: torch.Tensor, step: str, count: Optional[torch.Tensor] = None):
+    """a[i] = the step constant of pattern word words[i] (int64 view of the uint64 word, bit k = row k of the contiguous
+    fp32 dictionary D) by lrs_spectral_patterns_f32, on the current stream.  ``count``: a device int64 holding how many
+    leading words to process (the rest of a is left unwritten), None = all of them."""
+    mode = _STEP_MODES.get(step)
+    if mode is None:
+        raise ValueError(f"unknown step mode {step!r}")
+    n, K = D.shape
+    L = lib()
+    ws_bytes = L.lrs_spectral_patterns_workspace_bytes(n)
+    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=D.device)
+    a = torch.empty(words.numel(), dtype=torch.float32, device=D.device)
+    check(L.lrs_spectral_patterns_f32(ptr(D), n, K, ptr(words), words.numel(), ptr(count), mode, ptr(a), ptr(ws), ws_bytes,
+                                      stream_ptr()), "lrs_spectral_patterns_f32")
+    return a
+
+
 def patch_step_constants(Y_observed, D, bb: int, s: int, step: str = "spectral", p_begin: int = 0,
                          p_end: Optional[int] = None):
     """a[p] = ||M_p D||_2^2 (``step='spectral'``, np.linalg.norm(H, 2)**2 of main_LRS_PnP.py:134) or 4||M_p D||_F^2
@@ -247,15 +267,14 @@ def patch_step_constants(Y_observed, D, bb: int, s: int, step: str = "spectral",
     bb, s = int(bb), int(s)
     if not 1 <= bb <= 8:
         raise ValueError(f"per-patch step constants pack a patch's mask into 64 bits: bb <= 8 (got bb = {bb})")
-    mode = {"spectral": _lib.STEP_SPECTRAL, "frob4": _lib.STEP_FROB4}.get(step)
-    if mode is None:
+    if step not in _STEP_MODES:
         raise ValueError(f"unknown step mode {step!r}")
     Y, src, was_np = _to_dev(Y_observed)
     if Y.dim() != 2:
         raise ValueError("Y_observed must be a 2-D (pixels x bands) matrix")
     R, C = Y.shape
     Dd = torch.as_tensor(D).to(device=Y.device, dtype=torch.float32).contiguous()
-    n, K = Dd.shape
+    n = Dd.shape[0]
     if n != bb * bb:
         raise ValueError(f"dictionary has {n} rows, bb² = {bb * bb}")
     P = patch_count(R, C, bb, s)
@@ -266,8 +285,6 @@ def patch_step_constants(Y_observed, D, bb: int, s: int, step: str = "spectral",
     L = lib()
     with torch.cuda.device(Y.device):
         a = torch.empty(p_end - p_begin, dtype=torch.float32, device=Y.device)
-        ws_bytes = L.lrs_spectral_patterns_workspace_bytes(n)
-        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=Y.device)
         for c0 in range(p_begin, p_end, PATCH_CONSTANTS_CHUNK):
             c1 = min(p_end, c0 + PATCH_CONSTANTS_CHUNK)
             m = c1 - c0
@@ -281,27 +298,23 @@ def patch_step_constants(Y_observed, D, bb: int, s: int, step: str = "spectral",
             del start
             uniq = torch.empty_like(sw).scatter_(0, group, sw)    # the words of a group are equal: any writer is right
             count = group[-1:] + 1                                 # number of distinct words, stays on the device
-            vals = torch.empty(m, dtype=torch.float32, device=Y.device)
-            check(L.lrs_spectral_patterns_f32(ptr(Dd), n, K, ptr(uniq), m, ptr(count), mode, ptr(vals), ptr(ws), ws_bytes,
-                                              stream_ptr()), "lrs_spectral_patterns_f32")
+            vals = _spectral_patterns(Dd, uniq, step, count)
             a[c0 - p_begin:c1 - p_begin].index_copy_(0, order, vals.index_select(0, group))
             del sw, order, group, uniq, vals
     return _back(a, src, was_np)
 
 
 def _row_pattern_table(D: torch.Tensor, bb: int, step: str) -> torch.Tensor:
-    n, K = D.shape
-    L = lib()
-    ws_bytes = L.lrs_spectral_table_workspace_bytes(bb)
-    if ws_bytes == 0:
+    """The pattern values of the 2^bb row-pattern words: row pattern r is the word with bit k set iff bit k % bb of r
+    is set (element k of a patch sits in pixel row k % bb), the word of a patch whose rows are observed in all bands
+    or in none."""
+    if not 1 <= bb <= 8:
         raise _lib.LrsError(f"row-pattern step-constant tables exist for bb <= 8 (got bb = {bb})")
-    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=D.device)
-    table = torch.empty(1 << bb, dtype=torch.float32, device=D.device)
-    mode = {"spectral": _lib.STEP_SPECTRAL, "frob4": _lib.STEP_FROB4}[step]
     with torch.cuda.device(D.device):
-        check(L.lrs_spectral_table_f32(ptr(D.contiguous()), K, bb, mode, ptr(table), ptr(ws), ws_bytes, stream_ptr()),
-              "lrs_spectral_table_f32")
-    return table
+        r = torch.arange(1 << bb, dtype=torch.int64, device=D.device)
+        k = torch.arange(bb * bb, dtype=torch.int64, device=D.device)
+        words = (((r[:, None] >> (k % bb)) & 1) << k).sum(1)      # distinct bits: the sum is their OR (bit 63 = sign)
+        return _spectral_patterns(D.contiguous(), words, step)
 
 
 # ------------------------------------------------------------------ ista

@@ -111,11 +111,18 @@ def _near_degenerate_top():
     return ((U * s) @ V.T).astype(np.float32)
 
 
+def _dominant_top():
+    D = synth.synthetic_dictionary(64, 256, seed=4)
+    D[:, :40] += 0.6 * D[:, [0]]                            # coherent atoms: a dominant singular value
+    return D
+
+
 TABLE_DICTIONARIES = {
     **{f"gaussian-K{K}": (lambda K=K: synth.synthetic_dictionary(64, K, seed=K)) for K in (64, 128, 192, 256)},
     "orthonormal-rows": _orthonormal_rows,
     "near-degenerate-top": _near_degenerate_top,
     "coherent": _coherent_dictionary,
+    "dominant-top": _dominant_top,
     "rank-16": lambda: synth.synthetic_dictionary(64, 16, seed=16),
     "scale-2^-20": lambda: synth.synthetic_dictionary(64, 256, seed=3) * np.float32(2.0 ** -20),
     "scale-2^20": lambda: synth.synthetic_dictionary(64, 256, seed=3) * np.float32(2.0 ** 20),
@@ -124,8 +131,8 @@ TABLE_DICTIONARIES = {
 
 @pytest.mark.parametrize("name", list(TABLE_DICTIONARIES))
 def test_step_constant_table_every_pattern(lrs, name):
-    """lrs_spectral_table_f32 for all 256 row-validity patterns against np.linalg.norm(D[valid], 2)**2 and 4||D[valid]||_F^2
-    in fp64; the empty pattern gives exactly 0."""
+    """The row-pattern table (lrs_spectral_patterns_f32 on the 256 row-pattern words) for all 256 row-validity patterns
+    against np.linalg.norm(D[valid], 2)**2 and 4||D[valid]||_F^2 in fp64; the empty pattern gives exactly 0."""
     D = TABLE_DICTIONARIES[name]()
     Dd = cu(D)
     tab_s = ops._row_pattern_table(Dd, 8, "spectral").cpu().numpy()
@@ -150,6 +157,23 @@ def test_step_constant_table_is_repeatable(lrs, name):
         first = ops._row_pattern_table(Dd, 8, step)
         for _ in range(2):
             assert torch.equal(ops._row_pattern_table(Dd, 8, step), first), step
+
+
+def test_step_constant_table_built_without_host_sync(lrs):
+    """Building the solver in the table mode, with the table not yet cached, does not synchronise with the host."""
+    H, W, B = 12, 12, 20
+    _, noisy = synth.synthetic_cube(H, W, B, rank=4, seed=1)
+    Y = synth.observe(noisy, synth.pixel_mask(H, W, keep=0.6, seed=2))
+    Yd, Md, Dd = cu(Y), cu((Y != 0).astype(np.float32)), cu(synth.synthetic_dictionary(64, 256, seed=0))
+    prm = lrs.Params(bb=8, slidingDis=1, step="spectral")
+    ops._TABLE_CACHE.clear()
+    torch.cuda.synchronize()
+    torch.cuda.set_sync_debug_mode("error")
+    try:
+        sol = lrs.LRSPnP(Yd, Md, Dd, prm)
+    finally:
+        torch.cuda.set_sync_debug_mode(0)
+    assert sol.be.coder.a_table is not None and len(ops._TABLE_CACHE) == 1
 
 
 # ================================================================ B. fused sparse step at the geometry edges

@@ -14,7 +14,7 @@ import torch
 import lrs_pnp_dip_b200 as lrs
 from lrs_pnp_dip_b200 import _lib, ops, synth
 from oracle import lrs_oracle as orc
-from tests.test_kernel_edges import FUSED_GEOMS, TABLE_DICTIONARIES, rel
+from tests.test_kernel_edges import FUSED_GEOMS, TABLE_DICTIONARIES, rel, row_patterns
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 gpu = pytest.mark.gpu
@@ -128,8 +128,8 @@ def _check_close(got, ref, tol=2e-6):
 @pytest.mark.parametrize("name", list(TABLE_DICTIONARIES))
 def test_pattern_values_every_dictionary(name):
     """Single elements (= ||D_i||^2), the full pattern (= ||D||_2^2), the empty pattern (exactly 0), all 256
-    band-replicated patterns (also against the row-pattern table) and random patterns at keep 0.5 / 0.9: spectral and
-    frob4 within 2e-6 of fp64."""
+    band-replicated patterns (equal, bit for bit, to the row-pattern table) and random patterns at keep 0.5 / 0.9:
+    spectral and frob4 within 2e-6 of fp64."""
     D = TABLE_DICTIONARIES[name]()
     rng = np.random.default_rng(1)
     k_rows = np.arange(64) % 8
@@ -148,8 +148,7 @@ def test_pattern_values_every_dictionary(name):
     nz = ref > 0
     _check_close(a[nz], ref[nz])
     assert np.all(a[~nz] == 0.0)
-    table = ops._row_pattern_table(cu(D), 8, "spectral").cpu().numpy().astype(np.float64)
-    _check_close(a[65:65 + 256][1:], table[1:])
+    assert np.array_equal(a[65:65 + 256], ops._row_pattern_table(cu(D), 8, "spectral").cpu().numpy())
     f = patterns_dev(D, words, "frob4")
     fref = frob4_fp64(D, mask)
     _check_close(f[fref > 0], fref[fref > 0])
@@ -258,13 +257,19 @@ def test_sparse_step_per_element_masks_vs_oracle(kind, s):
 
 @gpu
 def test_spectral_patch_equals_table_on_replicated_masks():
-    """On band-replicated masks the per-patch constants and the 256-entry table give the same sparse step (<= 1e-5)."""
+    """On band-replicated masks every patch's constant equals, bit for bit, the 256-entry table's entry for the patch's
+    row pattern, and the two give the same sparse step (<= 1e-5: the kernels' table and per-patch paths round
+    differently)."""
     X, L, Y, _ = _cube_inputs("replicated", H=10, W=16, B=24, seed=4)
     D = synth.synthetic_dictionary(64, 256, seed=2)
-    out = {}
+    sc, out = {}, {}
     for step in ("spectral", "spectral_patch"):
         prm = lrs.Params(mu_1=MU1, lambda_ista=LAM, Nit=NIT, bb=8, slidingDis=1, step=step)
-        out[step] = lrs.SparseCoder(cu(Y), cu(D), prm).phi_z(cu(X), cu(L)).cpu().numpy()
+        sc[step] = lrs.SparseCoder(cu(Y), cu(D), prm)
+        out[step] = sc[step].phi_z(cu(X), cu(L)).cpu().numpy()
+    xs, _ = orc.patch_index(Y.shape[0], Y.shape[1], 8, 1)
+    table = sc["spectral"].a_table.cpu().numpy()
+    assert np.array_equal(sc["spectral_patch"].a_patch.cpu().numpy(), table[row_patterns(Y[:, 0] != 0, xs)])
     assert rel(out["spectral_patch"], out["spectral"]) <= 1e-5
 
 

@@ -43,10 +43,7 @@ __device__ __forceinline__ void split_h(float x, __half& h1, __half& h2) {
     h2 = __float2half_rn(x - __half2float(h1));
 }
 
-// 1-D bulk copy global -> shared (TMA engine, SASS UBLKCP), completion counted in bytes on an mbarrier
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
+// 1-D bulk copy global -> shared (TMA engine, SASS UBLKCP), completion counted in bytes on an mbarrier (mbar_expect_tx)
 __device__ __forceinline__ void bulk_g2s(uint32_t dst_smem, const void* src, uint32_t bytes, uint64_t* bar) {
     asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst_smem),
                  "l"(src), "r"(bytes), "r"(smem_u32(bar))
@@ -464,7 +461,6 @@ bool ista_tc_enabled() {
 // launch with the programmatic-stream-serialization attribute (see pdl_wait above)
 template <class... KArgs, class... Args>
 static cudaError_t launch_chained(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args... args) {
-    static const bool plain = getenv("LRS_ISTA_NO_PDL") != nullptr;
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = grid;
     cfg.blockDim = block;
@@ -474,7 +470,7 @@ static cudaError_t launch_chained(void (*kern)(KArgs...), dim3 grid, dim3 block,
     at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     at[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = at;
-    cfg.numAttrs = plain ? 0 : 1;
+    cfg.numAttrs = 1;
     return cudaLaunchKernelEx(&cfg, kern, KArgs(args)...);
 }
 

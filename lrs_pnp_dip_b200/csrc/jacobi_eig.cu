@@ -26,10 +26,13 @@
 #include <vector>
 
 #include "common.cuh"
+#include "tc_common.cuh"
 
 namespace cg = cooperative_groups;
 
 namespace lrs {
+using namespace tc;
+
 namespace {
 
 constexpr int JC = 8;              // CTAs per cluster (portable maximum)
@@ -143,8 +146,7 @@ __device__ __forceinline__ float rotate_pair(double* __restrict__ p, double* __r
 }
 
 // ---- distributed-shared-memory plumbing: bulk copies between the shared memories of two CTAs of the cluster (TMA engine),
-// completion counted in bytes on an mbarrier of the DESTINATION CTA ----
-__device__ __forceinline__ uint32_t jsmem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
+// completion counted in bytes on an mbarrier of the DESTINATION CTA (mbar_expect_tx) ----
 __device__ __forceinline__ uint32_t map_to_rank(uint32_t local_smem_addr, int rank) {
     uint32_t r;
     asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(local_smem_addr), "r"(rank));
@@ -154,24 +156,6 @@ __device__ __forceinline__ void bulk_s2s(uint32_t dst_cluster, uint32_t src_cta,
     asm volatile("cp.async.bulk.shared::cluster.shared::cta.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst_cluster),
                  "r"(src_cta), "r"(bytes), "r"(bar_cluster)
                  : "memory");
-}
-__device__ __forceinline__ void jbar_init(uint64_t* bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(jsmem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void jbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(jsmem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void jbar_wait(uint64_t* bar, uint32_t parity) {
-    uint32_t ok = 0;
-    while (!ok) {
-        asm volatile(
-            "{\n\t.reg .pred p;\n\t"
-            "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-            "selp.u32 %0, 1, 0, p;\n\t}"
-            : "=r"(ok)
-            : "r"(jsmem_u32(bar)), "r"(parity)
-            : "memory");
-    }
 }
 
 // status[0] = sweeps run, status[1] = 1 if the last sweep still rotated by more than the stopping angle (not converged),
@@ -215,9 +199,9 @@ __global__ void __cluster_dims__(JC, 1, 1) __launch_bounds__(JT, 1)
     }
     if (tid == 0) {
         my_max = 0;
-        jbar_init(&bar[0], 1);
-        jbar_init(&bar[1], 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init(&bar[0], 1);
+        mbar_init(&bar[1], 1);
+        mbar_fence_init();
     }
     // ||G||_F^2 (every CTA computes the same sum in the same order): scale of the dead-column floor
     double floor2;
@@ -282,14 +266,14 @@ __global__ void __cluster_dims__(JC, 1, 1) __launch_bounds__(JT, 1)
                     for (int pr = 0; pr < JC; ++pr) cl.map_shared_rank(&max_cos2[0][0], pr)[(sweep & 1) * JC + rank] = my_max;
                     my_max = 0;
                 }
-                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // the rotations' stores -> copy engine
-                jbar_expect_tx(&bar[nph], 2 * slot_bytes);
-                bulk_s2s(map_to_rank(jsmem_u32(slot(nph, top_slot)), top_to), jsmem_u32(top), slot_bytes,
-                         map_to_rank(jsmem_u32(&bar[nph]), top_to));
-                bulk_s2s(map_to_rank(jsmem_u32(slot(nph, bot_slot)), bot_to), jsmem_u32(bot), slot_bytes,
-                         map_to_rank(jsmem_u32(&bar[nph]), bot_to));
+                fence_async_smem();                                // the rotations' stores -> copy engine
+                mbar_expect_tx(&bar[nph], 2 * slot_bytes);
+                bulk_s2s(map_to_rank(smem_u32(slot(nph, top_slot)), top_to), smem_u32(top), slot_bytes,
+                         map_to_rank(smem_u32(&bar[nph]), top_to));
+                bulk_s2s(map_to_rank(smem_u32(slot(nph, bot_slot)), bot_to), smem_u32(bot), slot_bytes,
+                         map_to_rank(smem_u32(&bar[nph]), bot_to));
             }
-            jbar_wait(&bar[nph], uses[nph] & 1);                   // step 4
+            mbar_wait(&bar[nph], uses[nph] & 1);                   // step 4
             ++uses[nph];
             cl.barrier_arrive();
             armed = true;

@@ -53,40 +53,11 @@ constexpr int NCG = NEPI / 4;                  // column groups per TMEM lane qu
 constexpr int CW = 64 / NCG;                   // columns (of a 64-column chunk) and pixels per epilogue thread
 constexpr int NPX = 16 / NCG;                  // pixels of every 16-pixel GEMM-B k-step owned by one epilogue thread
 static_assert(NPX == 8, "the residual epilogue moves its pixels with 8-column TMEM loads and 16-byte stores");
-constexpr int FIRST_EPI = (NEPI == 8) ? 4 : 2; // first epilogue warp (keeps warp % 4 == TMEM lane quarter)
+constexpr int FIRST_EPI = 4;                   // first epilogue warp (keeps warp % 4 == TMEM lane quarter)
 constexpr int NTHREADS = 32 * (FIRST_EPI + NEPI);
-#ifndef LRS_WG0_REGS
-#define LRS_WG0_REGS 88
-#define LRS_EPI_REGS 208
-#endif
-#ifndef LRS_B1_EARLY
-#define LRS_B1_EARLY 0       // k-steps of GEMM-B's second atom half issued during the residual phase (see the MMA issuer)
-#endif
-#ifndef LRS_MASK_FOLD
-#define LRS_MASK_FOLD 1      // 1: band-replicated masks folded into the residual constants (no per-element selects)
-#endif
-#ifndef LRS_TAIL_SPLIT
-#define LRS_TAIL_SPLIT 1     // 1: the last soft-threshold chunk is released to GEMM-A in two 16-atom halves per column group
-#endif
-#ifndef LRS_SPLIT_FHFMA
-#define LRS_SPLIT_FHFMA 1    // 1: low fp16 piece through the mixed-precision FMA (FHFMA)
-#endif
-#ifndef LRS_RES_PREFETCH
-#define LRS_RES_PREFETCH 0   // 1: residual phase requests the next quarter's accumulators one quarter ahead
-#endif
-#ifndef LRS_DEFER_ARRIVE
-#define LRS_DEFER_ARRIVE 1   // 1: soft chunk j is signalled from the middle of chunk j+1 (hides the TMEM store latency)
-#endif
-#ifndef LRS_SOFT_XORSIGN
-#define LRS_SOFT_XORSIGN 1   // 1: clamp through min.xorsign.abs (one FMNMX.XORSIGN per element)
-#endif
-#ifndef LRS_SOFT_SAT
-#define LRS_SOFT_SAT 0       // 1 / 2: soft threshold through fma.sat on the FMA pipe (see SoftSat; both measured, neither adopted)
-#endif
-#define LRS_STR2(x) #x
-#define LRS_STR(x) LRS_STR2(x)
-static_assert(128 * LRS_WG0_REGS + 256 * LRS_EPI_REGS <= 384 * 168, "register budget of one CTA per SM");
-static_assert(FIRST_EPI == 4 && NEPI == 8, "setmaxnreg works on warpgroups: warps 0-3 give registers to warps 4-11");
+// setmaxnreg works on warpgroups: warps 0-3 give registers to warps 4-11
+constexpr int WG0_REGS = 88, EPI_REGS = 208;
+static_assert(128 * WG0_REGS + 256 * EPI_REGS <= 384 * 168, "register budget of one CTA per SM");
 constexpr int MAXCHUNK = 4;                    // soft-threshold / GEMM-A pipeline: K/64 chunks of 64 atoms, K <= 256
 constexpr uint32_t COL_ALPHA = 0;    // [0,256)   fp32 state / GEMM-B accumulator
 constexpr uint32_t COL_ACC = 256;    // [256,320) a1 D1 + a2 D1 ; [320,384) a1 D2
@@ -103,13 +74,11 @@ constexpr float S_R = 0.25f;         // residual pieces = fp16(r / 4)  (S_R * S_
 // D pieces in shared memory, one copy for both GEMMs (bytes):
 //   (k%8)*2 + (i%8)*16 + (8*piece + i/8)*128 + (k/8)*2048       i = pixel (row of D), k = atom
 constexpr uint32_t D_SMEM_BYTES = 64 * 1024;
-// GEMM-B variant: residual pieces as the A operand from SHARED memory (SS form) and the 256 atoms in two N = 128
+// GEMM-B takes the residual pieces as the A operand from SHARED memory (SS form) and the 256 atoms in two N = 128
 // halves, so that the soft-threshold of the first half overlaps the MMAs of the second (an N = 128 MMA with A in
-// shared memory runs at its 64-cycle MAC floor; with A in TMEM it would cost 88).  false = A from TMEM, N = 256.
-constexpr bool B_SS = true;
-static_assert(B_SS, "the TMEM-operand GEMM-B variant (v2) was removed with the shared k-step mapping");
+// shared memory runs at its 64-cycle MAC floor; with A in TMEM it would cost 88).
 // residual pieces in shared memory, K-major A operand (bytes): (k%8)*2 + (m%8)*16 + (m/8)*128 + (k/8)*2048 + piece*16384
-constexpr uint32_t R_SMEM_BYTES = B_SS ? 32 * 1024 : 0;
+constexpr uint32_t R_SMEM_BYTES = 32 * 1024;
 constexpr uint32_t R_SK = 2048, R_SM = 128, R_PIECE = 16 * 1024;
 constexpr uint32_t D_SK = 2048, D_SI = 128;
 // Next tile's patch values, gathered by the otherwise idle warps 1..3 while the current tile iterates:
@@ -119,8 +88,8 @@ constexpr int NLOAD = 32 * (FIRST_EPI - 1);   // loader threads
 
 struct __align__(8) Shared {
     uint64_t bar_R[4];        // epilogue -> MMA: residual pieces of pixel quarter ks are in shared memory (NEPI warps)
-    uint64_t bar_B[2];        // MMA -> epilogue: GEMM-B complete for atom half h (h = 0 only when !B_SS)      (commit)
-    uint64_t bar_S[MAXCHUNK];   // epilogue -> MMA: soft-thresholded state pieces of chunk j are staged     (16 warps)
+    uint64_t bar_B[2];        // MMA -> epilogue: GEMM-B complete for atom half h                              (commit)
+    uint64_t bar_S[MAXCHUNK];   // epilogue -> MMA: soft-thresholded state pieces of chunk j are staged     (NEPI warps)
     uint64_t bar_A[MAXCHUNK];   // MMA -> epilogue: GEMM-A of chunk j complete (staging free / Da final)    (commit)
     uint64_t bar_T[2];        // epilogue -> MMA: first / second 16-atom halves of the LAST chunk are staged (NEPI warps)
     uint64_t bar_G_full;      // loader -> epilogue: the gathered values of the next tile are in shared memory (loader warps)
@@ -171,17 +140,12 @@ __device__ __forceinline__ uint64_t fma2(uint64_t a, uint64_t b, uint64_t c) {
 __device__ __forceinline__ void split_pair(float x0, float x1, uint32_t& p1, uint32_t& p2) {
     __half2 h = __floats2half2_rn(x0, x1);
     float l0, l1;
-#if LRS_SPLIT_FHFMA
     // x - fp16(x) with the mixed-precision FMA of sm_100 (fma.rn.f32.f16 -> FHFMA): one instruction per element instead of
     // a conversion and half a packed subtract; the difference is exact either way
     const unsigned short hl = __half_as_ushort(__low2half(h)), hh = __half_as_ushort(__high2half(h));
     const unsigned short m1 = 0xBC00;   // -1.0 in fp16
     asm("fma.rn.f32.f16 %0, %1, %2, %3;" : "=f"(l0) : "h"(hl), "h"(m1), "f"(x0));
     asm("fma.rn.f32.f16 %0, %1, %2, %3;" : "=f"(l1) : "h"(hh), "h"(m1), "f"(x1));
-#else
-    float2 f = __half22float2(h);
-    upk2(sub2(pk2(x0, x1), pk2(f.x, f.y)), l0, l1);
-#endif
     __half2 l = __floats2half2_rn(l0, l1);
     p1 = pack_h2(h);
     p2 = pack_h2(l);
@@ -190,53 +154,14 @@ __device__ __forceinline__ void split_pair(float x0, float x1, uint32_t& p1, uin
 // soft(g, T) = g - clamp(g, -T, T) for a pair.  clamp(g, -T, T) = sign(g) min(|g|, T) is ONE instruction per element
 // (min.xorsign.abs -> FMNMX.XORSIGN: magnitude min(|g|, |T|), sign = sign(g) xor sign(T), T >= 0), then one packed
 // subtract: three instructions per pair, exact (|g| <= T gives g - g = 0; beyond it g -/+ T is the single rounding of
-// sign(g)(|g| - T), soft.m:4).  LRS_SOFT_XORSIGN = 0 keeps the two-min/max form (five instructions per pair).
+// sign(g)(|g| - T), soft.m:4).  The two-min/max form takes five instructions per pair; the fma.sat forms on the FMA pipe
+// were either inexact in the dead zone or slower (DESIGN.md 4.4).
 __device__ __forceinline__ void soft_pair(float g0, float g1, float T, float& x0, float& x1) {
-#if LRS_SOFT_XORSIGN
     float t0, t1;
     asm("min.xorsign.abs.f32 %0, %1, %2;" : "=f"(t0) : "f"(g0), "f"(T));
     asm("min.xorsign.abs.f32 %0, %1, %2;" : "=f"(t1) : "f"(g1), "f"(T));
-#else
-    const float t0 = fminf(fmaxf(g0, -T), T), t1 = fminf(fmaxf(g1, -T), T);
-#endif
     upk2(sub2(pk2(g0, g1), pk2(t0, t1)), x0, x1);
 }
-// The same through the FMA pipe (the min/max form runs on the half-rate ALU pipe that bounds the epilogue).
-//   LRS_SOFT_SAT = 2 (exact): with s = 2^-40, sat(g s - T s) = max(g - T, 0) s and sat(-g s - T s) = max(-g - T, 0) s — one
-//     rounding of g -/+ T each, as in sign(g) max(|g| - T, 0) (scaling by a power of two commutes with the rounding; |g| < 2^40
-//     is far beyond what the fp16 pieces can carry) — so soft(g, T) = (pos - neg) 2^40 bit for bit, exact zeros included:
-//     four FFMA.SAT, one FADD2 and one FMUL2 per pair.
-//   LRS_SOFT_SAT = 1 (inexact in the dead zone): clamp(g, -T, T) = (sat(g / 2T + 1/2) - 1/2) 2T, soft = (g + T) - 2T sat(..):
-//     two FFMA.SAT, one FADD2, one FFMA2 per pair, but |g| < T leaves a residue of order 2^-24 T instead of an exact zero
-//     (an all-zero solution comes back as noise) — measured only 0.2 % faster than the exact min/max form; kept for the record.
-struct SoftSat {
-#if LRS_SOFT_SAT == 2
-    float s, nTs;
-    uint64_t up2;
-    __device__ __forceinline__ explicit SoftSat(float T) : s(9.094947017729282e-13f), nTs(-T * 9.094947017729282e-13f),
-                                                          up2(pk2(1099511627776.0f, 1099511627776.0f)) {}
-    __device__ __forceinline__ void operator()(float g0, float g1, float& x0, float& x1) const {
-        float p0, p1, n0, n1;
-        asm("fma.rn.sat.f32 %0, %1, %2, %3;" : "=f"(p0) : "f"(g0), "f"(s), "f"(nTs));
-        asm("fma.rn.sat.f32 %0, %1, %2, %3;" : "=f"(p1) : "f"(g1), "f"(s), "f"(nTs));
-        asm("fma.rn.sat.f32 %0, %1, %2, %3;" : "=f"(n0) : "f"(g0), "f"(-s), "f"(nTs));
-        asm("fma.rn.sat.f32 %0, %1, %2, %3;" : "=f"(n1) : "f"(g1), "f"(-s), "f"(nTs));
-        uint64_t d = sub2(pk2(p0, p1), pk2(n0, n1)), r;
-        asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(d), "l"(up2));
-        upk2(r, x0, x1);
-    }
-#else
-    float inv2T;
-    uint64_t T2, m2T2;
-    __device__ __forceinline__ explicit SoftSat(float T) : inv2T(T > 0.f ? 0.5f / T : 0.f), T2(pk2(T, T)), m2T2(pk2(-2.f * T, -2.f * T)) {}
-    __device__ __forceinline__ void operator()(float g0, float g1, float& x0, float& x1) const {
-        float s0, s1;
-        asm("fma.rn.sat.f32 %0, %1, %2, 0f3F000000;" : "=f"(s0) : "f"(g0), "f"(inv2T));
-        asm("fma.rn.sat.f32 %0, %1, %2, 0f3F000000;" : "=f"(s1) : "f"(g1), "f"(inv2T));
-        upk2(fma2(pk2(s0, s1), m2T2, add2(pk2(g0, g1), T2)), x0, x1);
-    }
-#endif
-};
 
 template <int N> __device__ __forceinline__ void tmem_ldN(uint32_t a, uint32_t* r) {
     if constexpr (N == 8) tmem_ld8(a, r);
@@ -461,8 +386,8 @@ __global__ void __launch_bounds__(NTHREADS, 1) sparse_fused_tc_kernel(FusedParam
     const uint32_t tbase = sh.tmem_base;
     // warp-specialised register budget: the MMA / gather warpgroup (warps 0-3) gives registers to the two epilogue
     // warpgroups (168 each at launch: 128*88 + 256*208 = 384*168; 56/224 .. 104/200 measure the same within noise)
-    if (warp < 4) asm volatile("setmaxnreg.dec.sync.aligned.u32 " LRS_STR(LRS_WG0_REGS) ";");
-    else asm volatile("setmaxnreg.inc.sync.aligned.u32 " LRS_STR(LRS_EPI_REGS) ";");
+    if (warp < 4) asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(WG0_REGS));
+    else asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(EPI_REGS));
 
     if (warp == 0) {
         // ================================ MMA issuer ================================
@@ -510,49 +435,41 @@ __global__ void __launch_bounds__(NTHREADS, 1) sparse_fused_tc_kernel(FusedParam
                 {
                     const uint32_t idescB128 = make_idesc_f16(128, KH, /*b_mn_major=*/true);
                     const uint64_t descR0 = make_smem_desc(smem_u32(Rsm), /*lbo=*/R_SK, /*sbo=*/R_SM);
-                    // Issue order of the 8 (atom half, k-step) groups of 3 MMAs.  Half 0 takes every k-step as soon as its
-                    // residual quarter is staged (its completion releases the first soft-threshold chunks); LRS_B1_EARLY
-                    // k-steps of half 1 are slotted into the tensor-pipe gaps of the residual phase instead of all
-                    // running between bar_B[0] and the first GEMM-A chunk.
-                    constexpr int NE = LRS_B1_EARLY;
-                    static_assert(NE >= 0 && NE <= 3, "LRS_B1_EARLY");
+                    // Half 0 takes every k-step as soon as its residual quarter is staged (its completion releases the first
+                    // soft-threshold chunks), then half 1 runs all four k-steps.
 #pragma unroll
-                    for (int step = 0; step < 8; ++step) {
-                        // schedule: h0k0, [h1k0 .. h1k(NE-1) interleaved after h0k0 .. h0k(NE-1)], rest of half 0, rest of half 1
-                        int half, ks;
-                        if (step < 2 * NE) { half = step & 1; ks = step >> 1; }
-                        else if (step < 4 + NE) { half = 0; ks = step - NE; }
-                        else { half = 1; ks = step - 4; }
-                        if (half == 0) {
-                            long long w0 = TSTAMP();
-                            mbar_wait(&sh.bar_R[ks], par);
-                            if (DBG) dbg[1 + ks] += clock64() - w0;
-                            tc_fence_after();
+                    for (int half = 0; half < 2; ++half) {
+#pragma unroll
+                        for (int ks = 0; ks < 4; ++ks) {
+                            if (half == 0) {
+                                long long w0 = TSTAMP();
+                                mbar_wait(&sh.bar_R[ks], par);
+                                if (DBG) dbg[1 + ks] += clock64() - w0;
+                                tc_fence_after();
+                            }
+                            const uint64_t d1 = descB0 + (uint64_t)(((0 * 8 + 2 * ks) * D_SI + half * (KH / 8) * D_SK) >> 4);
+                            const uint64_t d2 = descB0 + (uint64_t)(((1 * 8 + 2 * ks) * D_SI + half * (KH / 8) * D_SK) >> 4);
+                            const uint64_t r1 = descR0 + (uint64_t)((2 * ks * R_SK) >> 4);
+                            const uint64_t r2 = descR0 + (uint64_t)((R_PIECE + 2 * ks * R_SK) >> 4);
+                            const uint32_t acc = tbase + COL_ALPHA + KH * half;
+                            if (leader) {
+                                mma_f16_ss(acc, r1, d1, idescB128, !(it == 0 && ks == 0));
+                                mma_f16_ss(acc, r2, d1, idescB128, true);
+                                mma_f16_ss(acc, r1, d2, idescB128, true);
+                            }
+                            __syncwarp();
+                            if (ks == 3 && leader) mma_commit(&sh.bar_B[half]);     // last group of the half
+                            __syncwarp();
                         }
-                        const uint64_t d1 = descB0 + (uint64_t)(((0 * 8 + 2 * ks) * D_SI + half * (KH / 8) * D_SK) >> 4);
-                        const uint64_t d2 = descB0 + (uint64_t)(((1 * 8 + 2 * ks) * D_SI + half * (KH / 8) * D_SK) >> 4);
-                        const uint64_t r1 = descR0 + (uint64_t)((2 * ks * R_SK) >> 4);
-                        const uint64_t r2 = descR0 + (uint64_t)((R_PIECE + 2 * ks * R_SK) >> 4);
-                        const uint32_t acc = tbase + COL_ALPHA + KH * half;
-                        if (leader) {
-                            mma_f16_ss(acc, r1, d1, idescB128, !(it == 0 && ks == 0));
-                            mma_f16_ss(acc, r2, d1, idescB128, true);
-                            mma_f16_ss(acc, r1, d2, idescB128, true);
-                        }
-                        __syncwarp();
-                        if (step == 3 + NE && leader) mma_commit(&sh.bar_B[0]);     // last group of half 0
-                        if (step == 7 && leader) mma_commit(&sh.bar_B[1]);
-                        __syncwarp();
                     }
                 }
                 // ---- GEMM-A: Da = state D^T, chunk by chunk as the soft-threshold epilogue releases them ----
 #pragma unroll
                 for (int j = 0; j < NCHUNK; ++j) {
                     const uint32_t stg = tbase + ((j & 1) ? COL_STG1 : COL_STG0);
-                    // TAIL: the last chunk is released in two halves (k-steps {0,2}, then {1,3}: each column group stages its
+                    // the last chunk is released in two halves (k-steps {0,2}, then {1,3}: each column group stages its
                     // first 16 atoms, then its last 16), so only two k-steps of MMAs remain after the soft threshold ends
-                    constexpr bool TAIL = LRS_TAIL_SPLIT != 0;
-                    if (TAIL && j == NCHUNK - 1) {
+                    if (j == NCHUNK - 1) {
 #pragma unroll
                         for (int h = 0; h < 2; ++h) {
                             long long w1 = TSTAMP();
@@ -585,9 +502,9 @@ __global__ void __launch_bounds__(NTHREADS, 1) sparse_fused_tc_kernel(FusedParam
                             mma_f16_ts(tbase + COL_ACC, stg + 32 + 8 * ks, d, idescA64, true);               // a2 D1
                         }
                     }
-                    // staging-release commits are only needed when chunks share staging buffers; the last chunk always
-                    // signals "Da complete"
-                    if ((j == NCHUNK - 1 || j + 2 < NCHUNK) && leader) mma_commit(&sh.bar_A[j]);
+                    // staging-release commits are only needed when chunks share staging buffers (the last chunk, above,
+                    // signals "Da complete")
+                    if (j + 2 < NCHUNK && leader) mma_commit(&sh.bar_A[j]);
                     __syncwarp();
                 }
                 if (DBG) dbg[10] += 1;
@@ -667,7 +584,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) sparse_fused_tc_kernel(FusedParam
 #pragma unroll
             for (int c = 0; c < NPX / 2; ++c)
                 nc2m[c] = pk2(((mbits >> (2 * c)) & 1u) ? -c2 : 0.f, ((mbits >> (2 * c + 1)) & 1u) ? -c2 : 0.f);
-            const SoftSat softsat(Tn);
             if (DBG) ed[7] += clock64() - tp0;
 
             for (int it = 0; it < Nit; ++it, ++gi) {
@@ -683,58 +599,43 @@ __global__ void __launch_bounds__(NTHREADS, 1) sparse_fused_tc_kernel(FusedParam
                 // FOLD: band-replicated masks (validity depends on the window row only), so the mask is folded into four
                 // packed constants nc2m[row pair] = -c2 .* m and into y' itself: r = y'm - (c2 m) Da needs no per-element
                 // select (the selects run on the half-rate ALU pipe that bounds the epilogue).
-                {
-                    // LRS_RES_PREFETCH: the accumulators of quarter ks+1 are requested before quarter ks is processed
-                    uint32_t ba[2][NPX], bb[2][NPX];
-                    if (LRS_RES_PREFETCH && it > 0) {
-                        tmem_ld8(lane_addr + COL_ACC + NPX * cg, ba[0]);
-                        tmem_ld8(lane_addr + COL_ACC + 64 + NPX * cg, bb[0]);
-                    }
 #pragma unroll
-                    for (int ks = 0; ks < 4; ++ks) {             // pixel quarter = GEMM-B k-step; my NPX pixels of it
-                        uint32_t p1[NPX / 2], p2[NPX / 2];
-                        if (it > 0) {
-                            uint32_t* b0 = ba[LRS_RES_PREFETCH ? (ks & 1) : 0];
-                            uint32_t* b1 = bb[LRS_RES_PREFETCH ? (ks & 1) : 0];
-                            if (!LRS_RES_PREFETCH) {
-                                tmem_ld8(lane_addr + COL_ACC + 16 * ks + NPX * cg, b0);
-                                tmem_ld8(lane_addr + COL_ACC + 64 + 16 * ks + NPX * cg, b1);
-                            }
-                            tmem_wait_ld();
-                            if (LRS_RES_PREFETCH && ks < 3) {
-                                tmem_ld8(lane_addr + COL_ACC + 16 * (ks + 1) + NPX * cg, ba[(ks + 1) & 1]);
-                                tmem_ld8(lane_addr + COL_ACC + 64 + 16 * (ks + 1) + NPX * cg, bb[(ks + 1) & 1]);
-                            }
+                for (int ks = 0; ks < 4; ++ks) {             // pixel quarter = GEMM-B k-step; my NPX pixels of it
+                    uint32_t p1[NPX / 2], p2[NPX / 2];
+                    if (it > 0) {
+                        uint32_t b0[NPX], b1[NPX];
+                        tmem_ld8(lane_addr + COL_ACC + 16 * ks + NPX * cg, b0);
+                        tmem_ld8(lane_addr + COL_ACC + 64 + 16 * ks + NPX * cg, b1);
+                        tmem_wait_ld();
 #pragma unroll
-                            for (int c = 0; c < NPX / 2; ++c) {
-                                const int e = NPX * ks + 2 * c;
-                                const uint64_t sm2 = add2(pk2(__uint_as_float(b0[2 * c]), __uint_as_float(b0[2 * c + 1])),
-                                                          pk2(__uint_as_float(b1[2 * c]), __uint_as_float(b1[2 * c + 1])));
-                                float r0, r1;
-                                upk2(fma2(FOLD ? nc2m[c] : nc2, sm2, pk2(ysc[e], ysc[e + 1])), r0, r1);
-                                if (!FOLD) {
-                                    r0 = ((mbits >> e) & 1u) ? r0 : 0.f;
-                                    r1 = ((mbits >> (e + 1)) & 1u) ? r1 : 0.f;
-                                }
-                                split_pair(r0, r1, p1[c], p2[c]);
+                        for (int c = 0; c < NPX / 2; ++c) {
+                            const int e = NPX * ks + 2 * c;
+                            const uint64_t sm2 = add2(pk2(__uint_as_float(b0[2 * c]), __uint_as_float(b0[2 * c + 1])),
+                                                      pk2(__uint_as_float(b1[2 * c]), __uint_as_float(b1[2 * c + 1])));
+                            float r0, r1;
+                            upk2(fma2(FOLD ? nc2m[c] : nc2, sm2, pk2(ysc[e], ysc[e + 1])), r0, r1);
+                            if (!FOLD) {
+                                r0 = ((mbits >> e) & 1u) ? r0 : 0.f;
+                                r1 = ((mbits >> (e + 1)) & 1u) ? r1 : 0.f;
                             }
-                        } else {
-#pragma unroll
-                            for (int c = 0; c < NPX / 2; ++c) {
-                                const int e = NPX * ks + 2 * c;
-                                split_pair(ysc[e], ysc[e + 1], p1[c], p2[c]);   // y' is stored masked
-                            }
+                            split_pair(r0, r1, p1[c], p2[c]);
                         }
-                        // my 8 pixels = k-group 2ks + cg of my row m: one 16-byte store per piece (a warp covers 512 contiguous
-                        // bytes per store: conflict-free), then publish to the async proxy
-                        uint8_t* rrow = Rsm + (uint32_t)(m >> 3) * R_SM + (uint32_t)(m & 7) * 16 + (uint32_t)(NCG * ks + cg) * R_SK;
-                        *reinterpret_cast<uint4*>(rrow) = make_uint4(p1[0], p1[1], p1[2], p1[3]);
-                        *reinterpret_cast<uint4*>(rrow + R_PIECE) = make_uint4(p2[0], p2[1], p2[2], p2[3]);
-                        fence_async_smem();
-                        tc_fence_before();
-                        __syncwarp();
-                        if (lane == 0) mbar_arrive(&sh.bar_R[ks]);
+                    } else {
+#pragma unroll
+                        for (int c = 0; c < NPX / 2; ++c) {
+                            const int e = NPX * ks + 2 * c;
+                            split_pair(ysc[e], ysc[e + 1], p1[c], p2[c]);   // y' is stored masked
+                        }
                     }
+                    // my 8 pixels = k-group 2ks + cg of my row m: one 16-byte store per piece (a warp covers 512 contiguous
+                    // bytes per store: conflict-free), then publish to the async proxy
+                    uint8_t* rrow = Rsm + (uint32_t)(m >> 3) * R_SM + (uint32_t)(m & 7) * 16 + (uint32_t)(NCG * ks + cg) * R_SK;
+                    *reinterpret_cast<uint4*>(rrow) = make_uint4(p1[0], p1[1], p1[2], p1[3]);
+                    *reinterpret_cast<uint4*>(rrow + R_PIECE) = make_uint4(p2[0], p2[1], p2[2], p2[3]);
+                    fence_async_smem();
+                    tc_fence_before();
+                    __syncwarp();
+                    if (lane == 0) mbar_arrive(&sh.bar_R[ks]);
                 }
                 // ---- soft threshold, 4 chunks of 64 atoms; my CW columns of each.  The load of chunk j+1 is in
                 //      flight while chunk j is processed. ----
@@ -751,20 +652,19 @@ __global__ void __launch_bounds__(NTHREADS, 1) sparse_fused_tc_kernel(FusedParam
                     uint32_t* gn = (j & 1) ? ga : gb;
                     uint32_t p1[CW / 2], p2[CW / 2];
                     const uint32_t col = COL_ALPHA + 64 * j + CW * cg;
-                    if (B_SS && j == FIRST_B1_CHUNK) {  // first chunk with atoms of the second GEMM-B half: no prefetch across it
+                    if (j == FIRST_B1_CHUNK) {  // first chunk with atoms of the second GEMM-B half: no prefetch across it
                         mbar_wait(&sh.bar_B[1], par);
                         tc_fence_after();
                         tmem_ldN<CW>(lane_addr + col, g);
                     }
                     tmem_wait_ld();
-                    if (j + 1 < NCHUNK && !(B_SS && j + 1 == FIRST_B1_CHUNK)) tmem_ldN<CW>(lane_addr + col + 64, gn);
+                    if (j + 1 < NCHUNK && j + 1 != FIRST_B1_CHUNK) tmem_ldN<CW>(lane_addr + col + 64, gn);
                     const uint32_t stg = (j & 1) ? COL_STG1 : COL_STG0;
                     auto soft_pairs = [&](int c_lo, int c_hi) {
 #pragma unroll
                         for (int c = c_lo; c < c_hi; ++c) {
                             float x0, x1;
-                            if (LRS_SOFT_SAT) softsat(__uint_as_float(g[2 * c]), __uint_as_float(g[2 * c + 1]), x0, x1);
-                            else soft_pair(__uint_as_float(g[2 * c]), __uint_as_float(g[2 * c + 1]), Tn, x0, x1);
+                            soft_pair(__uint_as_float(g[2 * c]), __uint_as_float(g[2 * c + 1]), Tn, x0, x1);
                             g[2 * c] = __float_as_uint(x0);
                             g[2 * c + 1] = __float_as_uint(x1);
                             split_pair(x0 * S_ALPHA, x1 * S_ALPHA, p1[c], p2[c]);
@@ -778,17 +678,17 @@ __global__ void __launch_bounds__(NTHREADS, 1) sparse_fused_tc_kernel(FusedParam
                             tc_fence_after();
                         }
                     };
-                    // LRS_DEFER_ARRIVE: chunk j's "staged" signal is given in the middle of chunk j+1's arithmetic, when its TMEM
-                    // stores have landed, instead of stalling on tcgen05.wait::st right after issuing them
+                    // chunk j's "staged" signal is given in the middle of chunk j+1's arithmetic, when its TMEM stores have
+                    // landed, instead of stalling on tcgen05.wait::st right after issuing them
                     auto flush_pending = [&]() {
-                        if (LRS_DEFER_ARRIVE && j > 0) {
+                        if (j > 0) {
                             tmem_wait_st();
                             tc_fence_before();
                             __syncwarp();
                             if (lane == 0) mbar_arrive(&sh.bar_S[j - 1]);
                         }
                     };
-                    if (LRS_TAIL_SPLIT && j == NCHUNK - 1) {
+                    if (j == NCHUNK - 1) {
                         // last chunk: my first 16 atoms (k-step 2 cg), then my last 16 (k-step 2 cg + 1), each released on its
                         // own barrier, so that only two k-steps of GEMM-A remain when the soft threshold ends
                         static_assert(CW == 32, "the tail split stages 16-atom halves with x16 / x8 TMEM stores");
@@ -815,12 +715,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) sparse_fused_tc_kernel(FusedParam
                         tmem_stN<CW>(lane_addr + col, g);
                         tmem_stN<CW / 2>(lane_addr + stg + (CW / 2) * cg, p1);
                         tmem_stN<CW / 2>(lane_addr + stg + 32 + (CW / 2) * cg, p2);
-                        if (!LRS_DEFER_ARRIVE || j == NCHUNK - 1) {
-                            tmem_wait_st();
-                            tc_fence_before();
-                            __syncwarp();
-                            if (lane == 0) mbar_arrive(&sh.bar_S[j]);
-                        }
                     }
                 }
                 if (DBG) ed[6] += clock64() - ts0;
@@ -955,7 +849,7 @@ template <int K>
 static int launch_tc(const FusedParams& prm, bool dynamic_tiles, cudaStream_t st) {
     const char* fn = "lrs_sparse_step_fused_f32";
     const size_t smem = D_SMEM_BYTES + R_SMEM_BYTES + G_SMEM_BYTES + sizeof(Shared);
-    const bool fold = LRS_MASK_FOLD && prm.a_table != nullptr && prm.a_patch == nullptr;
+    const bool fold = prm.a_table != nullptr && prm.a_patch == nullptr;
     using Kern = void (*)(FusedParams, TilePlan);
     auto pick = [&](auto dbg_c, bool dyn) -> Kern {
         constexpr bool DBGV = decltype(dbg_c)::value;

@@ -1,6 +1,7 @@
-// sm_100a primitives used by the tcgen05 engine: mbarrier, TMEM allocation, tcgen05.mma (kind::tf32,
-// A from shared memory or TMEM), tcgen05.ld/st, commit and fences, plus the shared-memory matrix
-// descriptor and instruction descriptor encoders (no-swizzle canonical layouts).
+// sm_100a primitives used by the tcgen05 engines and the cluster eigensolver: mbarrier, TMEM allocation, tcgen05.mma
+// (kind::f16 and kind::tf32, A from shared memory or TMEM), tcgen05.ld/st, commit and fences, plus the shared-memory
+// matrix descriptor and instruction descriptor encoders (no-swizzle canonical layouts).  The kind::tf32 wrappers are
+// used only by the diagnostics probe (tc_probe.cu).
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -17,6 +18,10 @@ __device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
 __device__ __forceinline__ void mbar_fence_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
 __device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
     asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
+}
+// arrive and expect `bytes` more of bulk-copy (complete_tx) traffic in the current phase
+__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
+    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
 }
 __device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
     uint32_t ok;
@@ -178,12 +183,6 @@ __device__ __forceinline__ void tmem_st32(uint32_t taddr, const uint32_t* r) {
         "r"(r[19]), "r"(r[20]), "r"(r[21]), "r"(r[22]), "r"(r[23]), "r"(r[24]), "r"(r[25]), "r"(r[26]), "r"(r[27]),
         "r"(r[28]), "r"(r[29]), "r"(r[30]), "r"(r[31])
         : "memory");
-}
-
-// fp32 -> (hi, lo) with hi = the value the tensor core sees when it drops the 13 low mantissa bits
-__device__ __forceinline__ void split_tf32(float x, float& hi, float& lo) {
-    hi = __uint_as_float(__float_as_uint(x) & 0xFFFFE000u);
-    lo = x - hi;  // exact
 }
 
 }  // namespace tc

@@ -25,6 +25,11 @@
  *    work is enqueued asynchronously on it; no hidden device synchronisation.
  *  - There is no CPU fallback: without a CUDA device every compute entry point
  *    fails with LRS_E_CUDA.
+ *  - Batched forms (*_batch_*) serve B cubes of ONE geometry (same R, C, bb,
+ *    s): every per-cube array is [B, ...] contiguous, cube b at offset b times
+ *    the per-cube size, 1 <= B <= LRS_MAX_BATCH.  Slice b of a batched result
+ *    is what the single-cube entry point gives for cube b (each single-cube
+ *    entry point is the B = 1 call of the same launcher).
  */
 #ifndef LRS_PNP_H_
 #define LRS_PNP_H_
@@ -40,6 +45,8 @@ extern "C" {
 #define LRS_E_ARG (-1)       /* invalid argument / unsupported shape */
 #define LRS_E_CUDA (-2)      /* CUDA runtime error (message has the cudaError string) */
 #define LRS_E_WORKSPACE (-3) /* workspace too small */
+
+#define LRS_MAX_BATCH 65535 /* largest cube count of a batched entry point (the cube is a grid dimension) */
 
 #define LRS_STEP_SPECTRAL 0 /* a = ||H||_2^2        main_LRS_PnP.py:134, ista.m:15 */
 #define LRS_STEP_FROB4 1    /* a = 4*||H||_F^2      main_LRS_PnP_DIP_pro.py:190     */
@@ -84,6 +91,12 @@ int lrs_im2col_f32(const float* X_dev, const float* L_dev, float mu, int64_t R, 
  * sequential loop main_LRS_PnP.py:332-339).  Deterministic gather, no atomics. */
 int lrs_col2im_accum_f32(const float* blocks_dev, int64_t R, int64_t C, int bb, int s, float* imout_dev,
                          lrs_stream_t stream);
+/* Batched im2col / col2im: X_dev, L_dev (may be NULL), imout_dev [B, R, C]; blocks_dev [n, B*P] with cube b in columns
+ * [b*P, (b+1)*P).  The overlap sum of a cube keeps the sequential fp32 order of lrs_col2im_accum_f32. */
+int lrs_im2col_batch_f32(const float* X_dev, const float* L_dev, float mu, int64_t B, int64_t R, int64_t C, int bb, int s,
+                         float* blocks_dev, lrs_stream_t stream);
+int lrs_col2im_accum_batch_f32(const float* blocks_dev, int64_t B, int64_t R, int64_t C, int bb, int s, float* imout_dev,
+                               lrs_stream_t stream);
 /* The same overlap sum fed one RANGE of column starts at a time (bb = 8, s = 1): blocks_dev holds only the patches
  * p in [ci_begin*nR, ci_end*nR) (nR = R-bb+1 row starts; [n, (ci_end-ci_begin)*nR] row-major — what
  * lrs_sparse_step_fused_f32 writes for that patch range) and imout_dev carries the running sum.  Patch order is
@@ -178,26 +191,45 @@ int lrs_admm_update_f32(const float* Y_dev, const float* MtM_dev, const float* i
                         float* lam1_dev, float* lam2_dev, float* X_out_dev, float gamma, float mu_1, float mu_2,
                         int64_t rows, int64_t row_offset, int64_t R_total, int64_t C, int bb, int s,
                         lrs_stream_t stream);
+/* The same update for B whole cubes [B, R, C] of one geometry (Weight and lam1sum shared). */
+int lrs_admm_update_batch_f32(const float* Y_dev, const float* MtM_dev, const float* imout_dev, const float* U_dev,
+                              float* lam1_dev, float* lam2_dev, float* X_out_dev, float gamma, float mu_1, float mu_2, int64_t B,
+                              int64_t R, int64_t C, int bb, int s, lrs_stream_t stream);
 
 /* ---- low-rank proximal step (SVT, main_LRS_PnP.py:118-124) via the band Gram matrix ------------ */
 /* G[C,C] (fp64, device, accumulated INTO — caller zeroes) += Z^T Z with Z = X + c*L (L may be NULL). */
 int lrs_gram_f64(const float* X_dev, const float* L_dev, float c, int64_t R, int64_t C, double* G_dev,
                  lrs_stream_t stream);
+/* G[B,C,C] += Z_b^T Z_b for the B cubes Z_b = X_b + c*L_b of [B, R, C] arrays (caller zeroes G). */
+int lrs_gram_batch_f64(const float* X_dev, const float* L_dev, float c, int64_t B, int64_t R, int64_t C, double* G_dev,
+                       lrs_stream_t stream);
 /* Symmetric eigen-decomposition of the band Gram matrix (fp64, symmetric positive semi-definite, 1 <= C <= 256) in ONE
  * launch: one-sided Jacobi over a thread-block cluster (csrc/jacobi_eig.cu) — replaces the eigh / SVD of
  * main_LRS_PnP.py:119 without a host synchronisation.  Outputs: lam_dev[C] eigenvalues (unsorted), Bt_dev[C*C] with row k
  * = lambda_k * v_k (the eigenvector scaled by its eigenvalue; "B form"), status_dev[3] = {sweeps run, 1 if not converged,
  * 1 if an eigenvalue is not finite}. */
 int lrs_sym_eig_jacobi_f64(const double* G_dev, int C, double* lam_dev, double* Bt_dev, int* status_dev, lrs_stream_t stream);
+/* B independent problems in one launch (one cluster each; clusters need not be co-resident): G_dev [B,C,C], lam_dev [B,C],
+ * Bt_dev [B,C,C], status_dev [B,3]. */
+int lrs_sym_eig_jacobi_batch_f64(const double* G_dev, int64_t B, int C, double* lam_dev, double* Bt_dev, int* status_dev,
+                                 lrs_stream_t stream);
 /* W[C,C] (f32) = V diag(max(1 - tau/sigma_k, 0)) V^T on the leading C x C block, sigma_k = sqrt(max(evals[k], 0)):
  * the shrinkage of main_LRS_PnP.py:121-123 on the n_eig >= C eigenpairs of the (possibly zero-bordered) Gram matrix.
  * V[i,k] is read at V_dev[i*v_row_stride + k*v_col_stride] (eigenvectors in columns, either storage order).
  * b_form != 0: column k holds lambda_k * v_k as lrs_sym_eig_jacobi_f64 returns it (v_row_stride = 1, v_col_stride = C). */
 int lrs_svt_weights_f64(const double* evals_dev, const double* V_dev, int64_t v_row_stride, int64_t v_col_stride, int C,
                         int n_eig, double tau, int b_form, float* W_dev, lrs_stream_t stream);
+/* B weight matrices W_dev [B,C,C]: eigenvalues of cube b at evals_dev + b*n_eig, its eigenvectors at
+ * V_dev + b*v_batch_stride (the strides above within a cube). */
+int lrs_svt_weights_batch_f64(const double* evals_dev, const double* V_dev, int64_t v_batch_stride, int64_t v_row_stride,
+                              int64_t v_col_stride, int64_t B, int C, int n_eig, double tau, int b_form, float* W_dev,
+                              lrs_stream_t stream);
 /* U[R,C] = (X + c*L) * W, W [C,C] f32 = V diag(max(1 - tau/sigma, 0)) V^T from the caller's eigh. */
 int lrs_svt_apply_f32(const float* X_dev, const float* L_dev, float c, const float* W_dev, int64_t R, int64_t C,
                       float* U_dev, lrs_stream_t stream);
+/* U_b = (X_b + c*L_b) * W_b for B cubes: X, L, U [B, R, C], W [B, C, C]. */
+int lrs_svt_apply_batch_f32(const float* X_dev, const float* L_dev, float c, const float* W_dev, int64_t B, int64_t R,
+                            int64_t C, float* U_dev, lrs_stream_t stream);
 
 #ifdef __cplusplus
 }

@@ -20,6 +20,7 @@ ENGINE_AUTO, ENGINE_SIMT, ENGINE_TC = 0, 1, 2
 ENGINES = {"auto": ENGINE_AUTO, "simt": ENGINE_SIMT, "tc": ENGINE_TC}
 ENGINE_DYNAMIC_TILES = 0x100          # OR-ed into the engine: work items claimed dynamically (include/lrs_pnp.h)
 DENOISERS = {"soft": 0, "nlm": 1, "identity": 2}
+MAX_BATCH = 65535                     # LRS_MAX_BATCH: largest cube count of the batched entry points
 
 _p = C.c_void_p
 _i64 = C.c_int64
@@ -36,6 +37,8 @@ SIGNATURES = {
     "lrs_patch_index_i64": (_int, [_i64, _i64, _int, _int, _p, _p, _p, _p]),
     "lrs_im2col_f32": (_int, [_p, _p, _f, _i64, _i64, _int, _int, _p, _p]),
     "lrs_col2im_accum_f32": (_int, [_p, _i64, _i64, _int, _int, _p, _p]),
+    "lrs_im2col_batch_f32": (_int, [_p, _p, _f, _i64, _i64, _i64, _int, _int, _p, _p]),
+    "lrs_col2im_accum_batch_f32": (_int, [_p, _i64, _i64, _i64, _int, _int, _p, _p]),
     "lrs_col2im_accum_range_f32": (_int, [_p, _i64, _i64, _int, _int, _i64, _i64, _p, _p]),
     "lrs_coverage_weight_f32": (_int, [_i64, _i64, _int, _int, _p, _p]),
     "lrs_soft_f32": (_int, [_p, _f, _p, _i64, _p]),
@@ -50,10 +53,15 @@ SIGNATURES = {
     "lrs_sparse_step_fused_f32": (_int, [_p, _p, _f, _p, _p, _int, _p, _p, _f, _int, _i64, _i64, _int, _int, _i64,
                                          _i64, _p, _int, _p]),
     "lrs_admm_update_f32": (_int, [_p, _p, _p, _p, _p, _p, _p, _f, _f, _f, _i64, _i64, _i64, _i64, _int, _int, _p]),
+    "lrs_admm_update_batch_f32": (_int, [_p, _p, _p, _p, _p, _p, _p, _f, _f, _f, _i64, _i64, _i64, _int, _int, _p]),
     "lrs_gram_f64": (_int, [_p, _p, _f, _i64, _i64, _p, _p]),
+    "lrs_gram_batch_f64": (_int, [_p, _p, _f, _i64, _i64, _i64, _p, _p]),
     "lrs_sym_eig_jacobi_f64": (_int, [_p, _int, _p, _p, _p, _p]),
+    "lrs_sym_eig_jacobi_batch_f64": (_int, [_p, _i64, _int, _p, _p, _p, _p]),
     "lrs_svt_weights_f64": (_int, [_p, _p, _i64, _i64, _int, _int, C.c_double, _int, _p, _p]),
+    "lrs_svt_weights_batch_f64": (_int, [_p, _p, _i64, _i64, _i64, _i64, _int, _int, C.c_double, _int, _p, _p]),
     "lrs_svt_apply_f32": (_int, [_p, _p, _f, _p, _i64, _i64, _p, _p]),
+    "lrs_svt_apply_batch_f32": (_int, [_p, _p, _f, _p, _i64, _i64, _i64, _p, _p]),
 }
 
 # diagnostics build only (include/lrs_pnp_diag.h, csrc/liblrs_pnp_diag.so): never loaded by the product path

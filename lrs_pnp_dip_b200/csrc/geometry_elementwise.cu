@@ -52,14 +52,19 @@ __global__ void idx_mat_kernel(Geom g, float* __restrict__ m) {
 }
 
 // ------------------------------------------------------------------------------------------------
-// im2col: blocks[(i + bb*j)*P + p] = V[(rs+i)*C + cs + j],  V = X (+ L/mu)
+// im2col: blocks[(i + bb*j)*ld + p] = V[(rs+i)*C + cs + j],  V = X (+ L/mu)
 // thread = (patch p, window column j); loops the bb rows.  Writes are coalesced along p.
+// Batch: cube b = blockIdx.z reads X, L at b*R*C and writes columns [b*P, (b+1)*P) of blocks [n, ld] (ld = B*P).
 // ------------------------------------------------------------------------------------------------
 __global__ void im2col_kernel(Geom g, const float* __restrict__ X, const float* __restrict__ L, float mu,
-                              float* __restrict__ blocks) {
+                              float* __restrict__ blocks, int64_t ld) {
     int64_t p = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     int j = blockIdx.y;
     if (p >= g.P) return;
+    const int64_t cube = (int64_t)blockIdx.z * g.R * g.C;
+    X += cube;
+    if (L) L += cube;
+    blocks += (int64_t)blockIdx.z * g.P;
     int64_t ci, ri;
     if (g.P <= 0x7fffffffLL) {  // 32-bit division on the common sizes
         const unsigned nr = (unsigned)g.row.n, pu = (unsigned)p;
@@ -73,7 +78,7 @@ __global__ void im2col_kernel(Geom g, const float* __restrict__ X, const float* 
     const int bb = g.bb;
     const float* src = X + rs * g.C + cs + j;
     const float* lsrc = L ? L + rs * g.C + cs + j : nullptr;
-    float* dst = blocks + (int64_t)(bb * j) * g.P + p;
+    float* dst = blocks + (int64_t)(bb * j) * ld + p;
     for (int i = 0; i < bb; ++i) {
         float v = __ldg(src);
         if (lsrc) {
@@ -82,7 +87,7 @@ __global__ void im2col_kernel(Geom g, const float* __restrict__ X, const float* 
         }
         *dst = v;
         src += g.C;
-        dst += g.P;
+        dst += ld;
     }
 }
 
@@ -92,9 +97,13 @@ __global__ void im2col_kernel(Geom g, const float* __restrict__ X, const float* 
 // out, 512 contiguous bytes per row.
 template <int IM2COL_TILE>
 __global__ void __launch_bounds__(256) im2col_s1_kernel(Geom g, const float* __restrict__ X, const float* __restrict__ L,
-                                                        float mu, float* __restrict__ blocks) {
+                                                        float mu, float* __restrict__ blocks, int64_t ld) {
     extern __shared__ float win[];   // [(TILE + bb - 1)][bb + 1]
-    const int bb = g.bb, ld = bb + 1;
+    const int64_t cube = (int64_t)blockIdx.z * g.R * g.C;    // batch: as im2col_kernel
+    X += cube;
+    if (L) L += cube;
+    blocks += (int64_t)blockIdx.z * g.P;
+    const int bb = g.bb, wld = bb + 1;
     const int64_t ri0 = blockIdx.x * (int64_t)IM2COL_TILE, ci = blockIdx.y;
     const int64_t nR = g.row.n;
     const int np = (int)(nR - ri0 < IM2COL_TILE ? nR - ri0 : IM2COL_TILE);   // patches of this tile
@@ -104,19 +113,19 @@ __global__ void __launch_bounds__(256) im2col_s1_kernel(Geom g, const float* __r
         const int64_t src = (ri0 + wr) * g.C + ci + wc;
         float v = __ldg(X + src);
         if (L) v = __fadd_rn(v, __fdiv_rn(__ldg(L + src), mu));
-        win[wr * ld + wc] = v;
+        win[wr * wld + wc] = v;
     }
     __syncthreads();
     const int m = threadIdx.x % IM2COL_TILE, h = threadIdx.x / IM2COL_TILE, nh = blockDim.x / IM2COL_TILE;
     if (m >= np) return;
     float* dst = blocks + ci * nR + ri0 + m;
     for (int j = 0; j < bb; ++j) {                               // element k = i + bb*j = row i, column j of the patch
-        float* d = dst + (int64_t)(bb * j + h) * g.P;
-        const float* w = win + (m + h) * ld + j;
+        float* d = dst + (int64_t)(bb * j + h) * ld;
+        const float* w = win + (m + h) * wld + j;
         for (int i = h; i < bb; i += nh) {
             __stcs(d, *w);                                       // written once, read by a later kernel: stream it
-            d += nh * g.P;
-            w += nh * ld;
+            d += nh * ld;
+            w += nh * wld;
         }
     }
 }
@@ -129,12 +138,13 @@ __global__ void __launch_bounds__(256) im2col_s1_kernel(Geom g, const float* __r
 // memory so the store runs along c.
 // ------------------------------------------------------------------------------------------------
 // Sum, in ascending row-start order, of the regular row starts [rlo, rhi] (+ the appended last start) of one column
-// start.  `pc` points at blocks[(bb*j)*P + ci*nR]; consecutive row starts are one pointer step apart, so the walk
-// costs an add per load (the kernel is instruction-issue bound otherwise: measured 56 instructions per load).
-__device__ __forceinline__ float col2im_column(const Geom& g, const float* __restrict__ pc, int64_t r, int64_t rlo,
+// start.  `pc` points at blocks[(bb*j)*ld + ci*nR] (ld = leading dimension of blocks); consecutive row starts are one
+// pointer step apart, so the walk costs an add per load (the kernel is instruction-issue bound otherwise: measured 56
+// instructions per load).
+__device__ __forceinline__ float col2im_column(const Geom& g, int64_t ld, const float* __restrict__ pc, int64_t r, int64_t rlo,
                                                int64_t nreg, bool rapp, float sum) {
-    const int64_t step = 1 - (int64_t)g.row.s * g.P;
-    const float* pr = pc + (r - rlo * g.row.s) * g.P + rlo;
+    const int64_t step = 1 - (int64_t)g.row.s * ld;
+    const float* pr = pc + (r - rlo * g.row.s) * ld + rlo;
     int64_t b = 0;
     for (; b + 8 <= nreg; b += 8) {  // 8 independent loads in flight, then the adds in patch order
         float v[8];
@@ -148,7 +158,7 @@ __device__ __forceinline__ float col2im_column(const Geom& g, const float* __res
         sum = __fadd_rn(sum, __ldg(pr));
         pr += step;
     }
-    if (rapp) sum = __fadd_rn(sum, __ldg(pc + (r - g.row.last) * g.P + g.row.n_reg));
+    if (rapp) sum = __fadd_rn(sum, __ldg(pc + (r - g.row.last) * ld + g.row.n_reg));
     return sum;
 }
 
@@ -161,14 +171,17 @@ __device__ __forceinline__ float col2im_column(const Geom& g, const float* __res
 // the range contains its first covering column start.  Patch order is column-start-outer, so feeding the ranges in
 // ascending order reproduces the association of the sequential loop (main_LRS_PnP.py:332-339) bit for bit while only one
 // range of Phi_z exists at a time.  Only output columns [ci_begin, ci_end + BB - 1) are touched.
+// Batch (whole range only): cube b = blockIdx.z sums columns [b*P, (b+1)*P) of blocks [n, ld] into out + b*R*C.
 template <int BB, int JU, int MINB>
-__global__ void __launch_bounds__(256, MINB) col2im_s1_kernel(Geom g, const float* __restrict__ blocks, float* __restrict__ out,
-                                                              int64_t ci_begin, int64_t ci_end) {
+__global__ void __launch_bounds__(256, MINB) col2im_s1_kernel(Geom g, const float* __restrict__ blocks, int64_t ld,
+                                                              float* __restrict__ out, int64_t ci_begin, int64_t ci_end) {
     __shared__ float tile[32][33];
     const int64_t r0 = blockIdx.x * 32LL, c0 = ci_begin + blockIdx.y * 32LL;
     const int tx = threadIdx.x, ty = threadIdx.y;  // blockDim = (32, 8)
-    const int64_t nR = g.row.n, nC = g.col.n, P = (ci_end - ci_begin) * nR;
-    const int64_t step = 1 - P, cstep = nR - (int64_t)BB * P;
+    const int64_t nR = g.row.n, nC = g.col.n;
+    blocks += (int64_t)blockIdx.z * (ci_end - ci_begin) * nR;
+    out += (int64_t)blockIdx.z * g.R * g.C;
+    const int64_t step = 1 - ld, cstep = nR - (int64_t)BB * ld;
     const int64_t c_end = ci_end + BB - 1 < g.C ? ci_end + BB - 1 : g.C;   // one past the last output column touched
     for (int cc = ty; cc < 32; cc += 8) {
         const int64_t r = r0 + tx, c = c0 + cc;
@@ -179,7 +192,7 @@ __global__ void __launch_bounds__(256, MINB) col2im_s1_kernel(Geom g, const floa
             const int64_t clo = clo_all > ci_begin ? clo_all : ci_begin, chi = chi_all < ci_end - 1 ? chi_all : ci_end - 1;
             const int nreg = (int)(rhi - rlo + 1), ncol = (int)(chi - clo + 1);
             if (clo > clo_all) sum = out[r * g.C + c];        // earlier ranges already added this element's first patches
-            const float* pc = blocks + ((r - rlo) + (int64_t)BB * (c - clo)) * P + (clo - ci_begin) * nR + rlo;
+            const float* pc = blocks + ((r - rlo) + (int64_t)BB * (c - clo)) * ld + (clo - ci_begin) * nR + rlo;
             if (nreg == BB) {
                 int j = 0;
                 for (; j + JU <= ncol; j += JU) {   // JU column starts = JU*BB independent loads in flight
@@ -223,9 +236,12 @@ __global__ void __launch_bounds__(256, MINB) col2im_s1_kernel(Geom g, const floa
 }
 
 template <int TR, int TC, int TY>
-__global__ void __launch_bounds__(TR * TY, 1536 / (TR * TY)) col2im_kernel(Geom g, const float* __restrict__ blocks, float* __restrict__ out) {
+__global__ void __launch_bounds__(TR * TY, 1536 / (TR * TY)) col2im_kernel(Geom g, const float* __restrict__ blocks, int64_t ld,
+                                                                           float* __restrict__ out) {
     __shared__ float tile[TC][TR + 1];
     int64_t r0 = blockIdx.x * (int64_t)TR, c0 = blockIdx.y * (int64_t)TC;
+    blocks += (int64_t)blockIdx.z * g.P;                   // batch: as col2im_s1_kernel
+    out += (int64_t)blockIdx.z * g.R * g.C;
     int tx = threadIdx.x, ty = threadIdx.y;  // blockDim = (TR, TY)
     for (int cc = ty; cc < TC; cc += TY) {
         int64_t r = r0 + tx, c = c0 + cc;
@@ -237,15 +253,15 @@ __global__ void __launch_bounds__(TR * TY, 1536 / (TR * TY)) col2im_kernel(Geom 
             g.col.cover(c, clo, chi, capp);
             const int64_t nreg = rhi - rlo + 1 > 0 ? rhi - rlo + 1 : 0;
             // regular column starts ci = clo..chi: j = c - ci*s; next ci: j -= s
-            const float* pc = blocks + ((int64_t)g.bb * (c - clo * g.col.s)) * g.P + clo * g.row.n;
-            const int64_t cstep = g.row.n - (int64_t)g.bb * g.col.s * g.P;
+            const float* pc = blocks + ((int64_t)g.bb * (c - clo * g.col.s)) * ld + clo * g.row.n;
+            const int64_t cstep = g.row.n - (int64_t)g.bb * g.col.s * ld;
             for (int64_t ci = clo; ci <= chi; ++ci) {
-                sum = col2im_column(g, pc, r, rlo, nreg, rapp, sum);
+                sum = col2im_column(g, ld, pc, r, rlo, nreg, rapp, sum);
                 pc += cstep;
             }
             if (capp)
-                sum = col2im_column(g, blocks + ((int64_t)g.bb * (c - g.col.last)) * g.P + g.col.n_reg * g.row.n, r, rlo, nreg,
-                                    rapp, sum);
+                sum = col2im_column(g, ld, blocks + ((int64_t)g.bb * (c - g.col.last)) * ld + g.col.n_reg * g.row.n, r, rlo,
+                                    nreg, rapp, sum);
         }
         tile[cc][tx] = sum;
     }
@@ -328,6 +344,14 @@ __global__ void admm_update_kernel(Geom g, const float* __restrict__ Y, const fl
     const int64_t r0 = (int64_t)blockIdx.x * ADMM_RPT;                   // ADMM_RPT unfolded rows per block row
     const int64_t c = blockIdx.y * (int64_t)blockDim.x + threadIdx.x;    // bands along the threads (coalesced)
     if (c >= g.C) return;
+    const int64_t cube = (int64_t)blockIdx.z * rows * g.C;               // batch: cube b = blockIdx.z, geometry shared
+    Y += cube;
+    M += cube;
+    IM += cube;
+    U += cube;
+    lam1 += cube;
+    lam2 += cube;
+    Xo += cube;
     const int wc = g.col.count(c);
     float l1[ADMM_RPT], l2[ADMM_RPT], im[ADMM_RPT], u[ADMM_RPT], y[ADMM_RPT], m[ADMM_RPT], l1s[ADMM_RPT];
     int W[ADMM_RPT], wmax = 0;
@@ -379,6 +403,67 @@ __global__ void admm_update_kernel(Geom g, const float* __restrict__ Y, const fl
 
 static inline unsigned blocks_for(int64_t n, int threads) { return (unsigned)((n + threads - 1) / threads); }
 
+// Launchers shared by the single-cube entry points (B = 1) and their batched forms: B cubes of one geometry, [B, R, C]
+// contiguous, cube b in grid z.
+static int im2col_launch(const char* fn, const float* X_dev, const float* L_dev, float mu, int64_t B, int64_t R, int64_t C,
+                         int bb, int s, float* blocks_dev, cudaStream_t st) {
+    Geom g;
+    if (!make_geom(R, C, bb, s, g)) return fail_arg(fn, "need 0 < bb <= min(R,C) and s > 0");
+    if (B < 1 || B > LRS_MAX_BATCH) return fail_arg(fn, "need 1 <= B <= LRS_MAX_BATCH");
+    if (!X_dev || !blocks_dev) return fail_arg(fn, "null pointer");
+    if (L_dev && mu == 0.0f) return fail_arg(fn, "mu must be non-zero");
+    // 256 row starts per block: measured 4.2-4.5 TB/s at cfg 4 (128: 3.9-4.3, 64: 3.3-3.5; thread-per-patch gather: 2.2)
+    constexpr int tile = 256;
+    const size_t win_bytes = (size_t)(tile + bb - 1) * (bb + 1) * sizeof(float);
+    const int64_t ld = B * g.P;
+    if (s == 1 && win_bytes <= 48 * 1024 && g.col.n <= 65535) {
+        im2col_s1_kernel<tile><<<dim3(blocks_for(g.row.n, tile), (unsigned)g.col.n, (unsigned)B), 256, win_bytes, st>>>(
+            g, X_dev, L_dev, mu, blocks_dev, ld);
+    } else {
+        dim3 grid(blocks_for(g.P, 128), bb, (unsigned)B);
+        im2col_kernel<<<grid, 128, 0, st>>>(g, X_dev, L_dev, mu, blocks_dev, ld);
+    }
+    LRS_CHECK_LAUNCH(fn);
+    return LRS_OK;
+}
+
+static int col2im_launch(const char* fn, const float* blocks_dev, int64_t B, int64_t R, int64_t C, int bb, int s,
+                         float* imout_dev, cudaStream_t st) {
+    Geom g;
+    if (!make_geom(R, C, bb, s, g)) return fail_arg(fn, "need 0 < bb <= min(R,C) and s > 0");
+    if (B < 1 || B > LRS_MAX_BATCH) return fail_arg(fn, "need 1 <= B <= LRS_MAX_BATCH");
+    if (!blocks_dev || !imout_dev) return fail_arg(fn, "null pointer");
+    dim3 grid(blocks_for(R, 32), blocks_for(C, 32), (unsigned)B);
+    if (grid.y > 65535) return fail_arg(fn, "C too large");
+    const int64_t ld = B * g.P;
+    // measured at cfg 4 (B200): generic kernel 3.9 ms; stride-1 kernel 2.2-2.6 ms; two or four column starts in flight
+    // per thread, 8 blocks/SM with 32 registers, or longer row tiles (128x8, 256x4) are all slower
+    if (s == 1 && bb == 8)
+        col2im_s1_kernel<8, 1, 6><<<grid, dim3(32, 8), 0, st>>>(g, blocks_dev, ld, imout_dev, 0, g.col.n);
+    else col2im_kernel<32, 32, 8><<<grid, dim3(32, 8), 0, st>>>(g, blocks_dev, ld, imout_dev);
+    LRS_CHECK_LAUNCH(fn);
+    return LRS_OK;
+}
+
+static int admm_update_launch(const char* fn, const float* Y_dev, const float* MtM_dev, const float* imout_dev,
+                              const float* U_dev, float* lam1_dev, float* lam2_dev, float* X_out_dev, float gamma, float mu_1,
+                              float mu_2, int64_t B, int64_t rows, int64_t row_offset, int64_t R_total, int64_t C, int bb, int s,
+                              cudaStream_t st) {
+    Geom g;
+    if (!make_geom(R_total, C, bb, s, g)) return fail_arg(fn, "need 0 < bb <= min(R,C) and s > 0");
+    if (B < 1 || B > LRS_MAX_BATCH) return fail_arg(fn, "need 1 <= B <= LRS_MAX_BATCH");
+    if (rows < 0 || row_offset < 0 || row_offset + rows > R_total) return fail_arg(fn, "row stripe outside the matrix");
+    if (rows == 0) return LRS_OK;
+    if (!Y_dev || !MtM_dev || !imout_dev || !U_dev || !lam1_dev || !lam2_dev || !X_out_dev) return fail_arg(fn, "null pointer");
+    const int threads = C >= 256 ? 256 : (int)((C + 31) / 32 * 32);
+    dim3 grid((unsigned)((rows + ADMM_RPT - 1) / ADMM_RPT), blocks_for(C, threads), (unsigned)B);
+    if (rows > 2147483647LL || grid.y > 65535) return fail_arg(fn, "matrix too large");
+    admm_update_kernel<<<grid, threads, 0, st>>>(g, Y_dev, MtM_dev, imout_dev, U_dev, lam1_dev, lam2_dev, X_out_dev, gamma, mu_1,
+                                                 mu_2, rows, row_offset);
+    LRS_CHECK_LAUNCH(fn);
+    return LRS_OK;
+}
+
 }  // namespace lrs
 
 using namespace lrs;
@@ -387,7 +472,7 @@ extern "C" {
 
 const char* lrs_last_error(void) { return lrs::g_err.c_str(); }
 
-int lrs_version(void) { return 102; }
+int lrs_version(void) { return 103; }
 
 uint64_t lrs_launch_count(void) { return (uint64_t)lrs::g_launches.load(); }
 
@@ -424,38 +509,22 @@ int lrs_patch_index_i64(int64_t R, int64_t C, int bb, int s, int64_t* x_index_de
 
 int lrs_im2col_f32(const float* X_dev, const float* L_dev, float mu, int64_t R, int64_t C, int bb, int s,
                    float* blocks_dev, lrs_stream_t stream) {
-    Geom g;
-    if (!make_geom(R, C, bb, s, g)) return fail_arg("lrs_im2col_f32", "need 0 < bb <= min(R,C) and s > 0");
-    if (!X_dev || !blocks_dev) return fail_arg("lrs_im2col_f32", "null pointer");
-    if (L_dev && mu == 0.0f) return fail_arg("lrs_im2col_f32", "mu must be non-zero");
-    // 256 row starts per block: measured 4.2-4.5 TB/s at cfg 4 (128: 3.9-4.3, 64: 3.3-3.5; thread-per-patch gather: 2.2)
-    constexpr int tile = 256;
-    const size_t win_bytes = (size_t)(tile + bb - 1) * (bb + 1) * sizeof(float);
-    if (s == 1 && win_bytes <= 48 * 1024 && g.col.n <= 65535) {
-        im2col_s1_kernel<tile><<<dim3(blocks_for(g.row.n, tile), (unsigned)g.col.n), 256, win_bytes, (cudaStream_t)stream>>>(
-            g, X_dev, L_dev, mu, blocks_dev);
-    } else {
-        dim3 grid(blocks_for(g.P, 128), bb);
-        im2col_kernel<<<grid, 128, 0, (cudaStream_t)stream>>>(g, X_dev, L_dev, mu, blocks_dev);
-    }
-    LRS_CHECK_LAUNCH("lrs_im2col_f32");
-    return LRS_OK;
+    return im2col_launch("lrs_im2col_f32", X_dev, L_dev, mu, 1, R, C, bb, s, blocks_dev, (cudaStream_t)stream);
+}
+
+int lrs_im2col_batch_f32(const float* X_dev, const float* L_dev, float mu, int64_t B, int64_t R, int64_t C, int bb, int s,
+                         float* blocks_dev, lrs_stream_t stream) {
+    return im2col_launch("lrs_im2col_batch_f32", X_dev, L_dev, mu, B, R, C, bb, s, blocks_dev, (cudaStream_t)stream);
 }
 
 int lrs_col2im_accum_f32(const float* blocks_dev, int64_t R, int64_t C, int bb, int s, float* imout_dev,
                          lrs_stream_t stream) {
-    Geom g;
-    if (!make_geom(R, C, bb, s, g)) return fail_arg("lrs_col2im_accum_f32", "need 0 < bb <= min(R,C) and s > 0");
-    if (!blocks_dev || !imout_dev) return fail_arg("lrs_col2im_accum_f32", "null pointer");
-    dim3 grid(blocks_for(R, 32), blocks_for(C, 32));
-    if (grid.y > 65535) return fail_arg("lrs_col2im_accum_f32", "C too large");
-    // measured at cfg 4 (B200): generic kernel 3.9 ms; stride-1 kernel 2.2-2.6 ms; two or four column starts in flight
-    // per thread, 8 blocks/SM with 32 registers, or longer row tiles (128x8, 256x4) are all slower
-    if (s == 1 && bb == 8)
-        col2im_s1_kernel<8, 1, 6><<<grid, dim3(32, 8), 0, (cudaStream_t)stream>>>(g, blocks_dev, imout_dev, 0, g.col.n);
-    else col2im_kernel<32, 32, 8><<<grid, dim3(32, 8), 0, (cudaStream_t)stream>>>(g, blocks_dev, imout_dev);
-    LRS_CHECK_LAUNCH("lrs_col2im_accum_f32");
-    return LRS_OK;
+    return col2im_launch("lrs_col2im_accum_f32", blocks_dev, 1, R, C, bb, s, imout_dev, (cudaStream_t)stream);
+}
+
+int lrs_col2im_accum_batch_f32(const float* blocks_dev, int64_t B, int64_t R, int64_t C, int bb, int s, float* imout_dev,
+                               lrs_stream_t stream) {
+    return col2im_launch("lrs_col2im_accum_batch_f32", blocks_dev, B, R, C, bb, s, imout_dev, (cudaStream_t)stream);
 }
 
 int lrs_col2im_accum_range_f32(const float* blocks_dev, int64_t R, int64_t C, int bb, int s, int64_t ci_begin, int64_t ci_end,
@@ -469,7 +538,8 @@ int lrs_col2im_accum_range_f32(const float* blocks_dev, int64_t R, int64_t C, in
     const int64_t c_end = ci_end + bb - 1 < C ? ci_end + bb - 1 : C;
     dim3 grid(blocks_for(R, 32), blocks_for(c_end - ci_begin, 32));
     if (grid.y > 65535) return fail_arg(fn, "C too large");
-    col2im_s1_kernel<8, 1, 6><<<grid, dim3(32, 8), 0, (cudaStream_t)stream>>>(g, blocks_dev, imout_dev, ci_begin, ci_end);
+    col2im_s1_kernel<8, 1, 6><<<grid, dim3(32, 8), 0, (cudaStream_t)stream>>>(g, blocks_dev, (ci_end - ci_begin) * g.row.n,
+                                                                              imout_dev, ci_begin, ci_end);
     LRS_CHECK_LAUNCH(fn);
     return LRS_OK;
 }
@@ -532,20 +602,15 @@ int lrs_admm_update_f32(const float* Y_dev, const float* MtM_dev, const float* i
                         float* lam1_dev, float* lam2_dev, float* X_out_dev, float gamma, float mu_1, float mu_2,
                         int64_t rows, int64_t row_offset, int64_t R_total, int64_t C, int bb, int s,
                         lrs_stream_t stream) {
-    Geom g;
-    if (!make_geom(R_total, C, bb, s, g)) return fail_arg("lrs_admm_update_f32", "need 0 < bb <= min(R,C) and s > 0");
-    if (rows < 0 || row_offset < 0 || row_offset + rows > R_total)
-        return fail_arg("lrs_admm_update_f32", "row stripe outside the matrix");
-    if (rows == 0) return LRS_OK;
-    if (!Y_dev || !MtM_dev || !imout_dev || !U_dev || !lam1_dev || !lam2_dev || !X_out_dev)
-        return fail_arg("lrs_admm_update_f32", "null pointer");
-    const int threads = C >= 256 ? 256 : (int)((C + 31) / 32 * 32);
-    dim3 grid((unsigned)((rows + ADMM_RPT - 1) / ADMM_RPT), blocks_for(C, threads));
-    if (rows > 2147483647LL || grid.y > 65535) return fail_arg("lrs_admm_update_f32", "matrix too large");
-    admm_update_kernel<<<grid, threads, 0, (cudaStream_t)stream>>>(g, Y_dev, MtM_dev, imout_dev, U_dev, lam1_dev, lam2_dev,
-                                                                  X_out_dev, gamma, mu_1, mu_2, rows, row_offset);
-    LRS_CHECK_LAUNCH("lrs_admm_update_f32");
-    return LRS_OK;
+    return admm_update_launch("lrs_admm_update_f32", Y_dev, MtM_dev, imout_dev, U_dev, lam1_dev, lam2_dev, X_out_dev, gamma,
+                              mu_1, mu_2, 1, rows, row_offset, R_total, C, bb, s, (cudaStream_t)stream);
+}
+
+int lrs_admm_update_batch_f32(const float* Y_dev, const float* MtM_dev, const float* imout_dev, const float* U_dev,
+                              float* lam1_dev, float* lam2_dev, float* X_out_dev, float gamma, float mu_1, float mu_2, int64_t B,
+                              int64_t R, int64_t C, int bb, int s, lrs_stream_t stream) {
+    return admm_update_launch("lrs_admm_update_batch_f32", Y_dev, MtM_dev, imout_dev, U_dev, lam1_dev, lam2_dev, X_out_dev,
+                              gamma, mu_1, mu_2, B, R, 0, R, C, bb, s, (cudaStream_t)stream);
 }
 
 }  // extern "C"

@@ -44,6 +44,7 @@ struct EpiGradientPlain {
 };
 struct EpiStore {
     __device__ __forceinline__ void slice(int64_t) {}
+    __device__ __forceinline__ void cube(int64_t off) { out += off; }     // batch of sgemm_kernel
     float* out;
     __device__ __forceinline__ void operator()(int64_t m, int64_t p, int64_t ld, float acc) const { out[m * ld + p] = acc; }
 };
@@ -60,6 +61,10 @@ struct LoadAxpy {  // Z = X + c*L on the fly (SVT input, main_LRS_PnP.py:315)
     const float* X;
     const float* L;
     float c;
+    __device__ __forceinline__ void cube(int64_t off) {
+        X += off;
+        if (L) L += off;
+    }
     __device__ __forceinline__ float operator()(int64_t o) const {
         float v = __ldg(X + o);
         if (L) v = __fadd_rn(v, __fmul_rn(c, __ldg(L + o)));
@@ -68,9 +73,13 @@ struct LoadAxpy {  // Z = X + c*L on the fly (SVT input, main_LRS_PnP.py:315)
 };
 
 // C[M,N] = op(A)[M,Kd] * B[Kd,N];  A stored row-major [M,Kd] (TRANS_A=false) or [Kd,M] (true).
+// Batch: grid.z = problem z, A and C shifted by z * ac_stride, B by z * b_stride.
 template <bool TRANS_A, class ALoad, class Epi>
 __global__ void __launch_bounds__(256) sgemm_kernel(ALoad aload, const float* __restrict__ B, int64_t M, int64_t N,
-                                                    int64_t Kd, Epi epi) {
+                                                    int64_t Kd, Epi epi, int64_t ac_stride, int64_t b_stride) {
+    aload.cube((int64_t)blockIdx.z * ac_stride);
+    epi.cube((int64_t)blockIdx.z * ac_stride);
+    B += (int64_t)blockIdx.z * b_stride;
     __shared__ float As[BK][BM + 4];
     __shared__ float Bs[BK][BN + 4];
     const int tid = threadIdx.x;
@@ -301,10 +310,10 @@ __global__ void nlm_column_kernel(const float* __restrict__ G, const float* __re
 
 template <bool TRANS_A, class ALoad, class Epi>
 static int launch_gemm(const char* fn, ALoad al, const float* B, int64_t M, int64_t N, int64_t Kd, Epi epi,
-                       cudaStream_t st) {
-    dim3 grid((unsigned)((N + BN - 1) / BN), (unsigned)((M + BM - 1) / BM));
+                       cudaStream_t st, int64_t batch, int64_t ac_stride, int64_t b_stride) {
+    dim3 grid((unsigned)((N + BN - 1) / BN), (unsigned)((M + BM - 1) / BM), (unsigned)batch);
     if (grid.y > 65535) return fail_arg(fn, "matrix too tall for this engine");
-    sgemm_kernel<TRANS_A, ALoad, Epi><<<grid, 256, 0, st>>>(al, B, M, N, Kd, epi);
+    sgemm_kernel<TRANS_A, ALoad, Epi><<<grid, 256, 0, st>>>(al, B, M, N, Kd, epi, ac_stride, b_stride);
     note_launch();
     return check_cuda(fn, cudaGetLastError());
 }
@@ -337,8 +346,9 @@ static int launch_gemm(const char* fn, LoadPlain al, const float* B, int64_t M, 
     return check_cuda(fn, cudaGetLastError());
 }
 
-// U[R,C] = (X + c L) W   — the recomposition GEMM of the Gram-based SVT (svt.cu declares it).
-int svt_apply_impl(const float* X, const float* L, float c, const float* W, int64_t R, int64_t C, float* U,
+// U[R,C] = (X + c L) W   — the recomposition GEMM of the Gram-based SVT (svt.cu declares it); for B cubes
+// ([B, R, C] X, L, U and [B, C, C] W) cube b is grid z.
+int svt_apply_impl(const float* X, const float* L, float c, const float* W, int64_t B, int64_t R, int64_t C, float* U,
                    cudaStream_t st) {
     // rows of Z play "M", W is the [Kd,N] operand
     dim3 grid((unsigned)((C + BN - 1) / BN), 1);
@@ -346,7 +356,8 @@ int svt_apply_impl(const float* X, const float* L, float c, const float* W, int6
     for (int64_t r0 = 0; r0 < R; r0 += rows_per_launch) {
         int64_t rows = R - r0 < rows_per_launch ? R - r0 : rows_per_launch;
         LoadAxpy al{X + r0 * C, L ? L + r0 * C : nullptr, c};
-        int rc = launch_gemm<false>("lrs_svt_apply_f32", al, W, rows, C, C, EpiStore{U + r0 * C}, st);
+        int rc = launch_gemm<false>(B > 1 ? "lrs_svt_apply_batch_f32" : "lrs_svt_apply_f32", al, W, rows, C, C,
+                                    EpiStore{U + r0 * C}, st, B, R * C, C * C);
         if (rc != LRS_OK) return rc;
     }
     return LRS_OK;

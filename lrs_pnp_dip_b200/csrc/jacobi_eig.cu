@@ -170,6 +170,9 @@ __device__ __forceinline__ void bulk_s2s(uint32_t dst_cluster, uint32_t src_cta,
 //   4. wait for the incoming slots (own mbarrier), arm the cluster barrier, switch phase.
 // The stopping rule needs no verification sweep: Jacobi converges quadratically, so a sweep whose largest rotated cosine
 // was below 3e-5 leaves cosines of order 1e-9.
+//
+// Batch: cluster q = blockIdx.x / JC solves problem q (G at q*n*n, lam at q*n, Bt at q*n*n, status at q*3).  Clusters
+// never communicate, so they need not be resident at the same time: a batch larger than the GPU runs in waves.
 template <int JROWS>
 __global__ void __cluster_dims__(JC, 1, 1) __launch_bounds__(JT, 1)
     jacobi_eig_kernel(const double* __restrict__ G, int n, int w, double tol2, double stop2, int max_sweeps,
@@ -182,6 +185,11 @@ __global__ void __cluster_dims__(JC, 1, 1) __launch_bounds__(JT, 1)
     __shared__ double fro[JT / 32];
     cg::cluster_group cl = cg::this_cluster();
     const int rank = (int)cl.block_rank();
+    const int64_t prob = blockIdx.x / JC;
+    G += prob * n * n;
+    lam += prob * n;
+    Bt += prob * n * n;
+    status += prob * 3;
     const int tid = threadIdx.x, nthr = blockDim.x, warp = tid >> 5, lane = tid & 31;
     const size_t slot_sz = (size_t)w * n, slot_stride = slot_sz + 2;
     const uint32_t slot_bytes = (uint32_t)(slot_stride * sizeof(double));
@@ -320,15 +328,14 @@ __global__ void __cluster_dims__(JC, 1, 1) __launch_bounds__(JT, 1)
 
 using namespace lrs;
 
-extern "C" int lrs_sym_eig_jacobi_f64(const double* G_dev, int C, double* lam_dev, double* Bt_dev, int* status_dev,
-                                      lrs_stream_t stream) {
-    const char* fn = "lrs_sym_eig_jacobi_f64";
+static int jacobi_launch(const char* fn, const double* G_dev, int64_t B, int C, double* lam_dev, double* Bt_dev, int* status_dev,
+                         cudaStream_t st) {
     if (C < 1 || C > JNB * JMAXW) return fail_arg(fn, "need 1 <= C <= 256");
+    if (B < 1 || B > LRS_MAX_BATCH) return fail_arg(fn, "need 1 <= B <= LRS_MAX_BATCH");
     if (!G_dev || !lam_dev || !Bt_dev || !status_dev) return fail_arg(fn, "null pointer");
     const int w = jacobi_block_width(C);                           // even slot size: the exchange moves 16-byte words
     if (w > JMAXW) return fail_arg(fn, "need 1 <= C <= 256");
     const size_t smem = (size_t)4 * ((size_t)w * C + 2) * sizeof(double);
-    cudaStream_t st = (cudaStream_t)stream;
     // rotate pairs whose cosine exceeds 1e-11; stop after a sweep whose largest rotated cosine was below 3e-5 (quadratic
     // convergence: what is left is of order 1e-9, two decades below what the fp32 weights W can resolve); 30 sweeps is far beyond the 7-9 a Gram matrix takes (14 for a spectrum
     // graded over 10 decades; exactly rank-deficient or degenerate matrices converge linearly in this parallel order: 17-22)
@@ -336,9 +343,9 @@ extern "C" int lrs_sym_eig_jacobi_f64(const double* G_dev, int C, double* lam_de
     auto launch = [&](auto kern) -> int {
         int rc = check_cuda(fn, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         if (rc != LRS_OK) return rc;
-        rc = check_cuda(fn, cudaMemsetAsync(status_dev, 0, 3 * sizeof(int), st));
+        rc = check_cuda(fn, cudaMemsetAsync(status_dev, 0, (size_t)B * 3 * sizeof(int), st));
         if (rc != LRS_OK) return rc;
-        kern<<<JC, 32 * we, smem, st>>>(G_dev, C, w, 1e-22, 1e-9, 30, lam_dev, Bt_dev, status_dev);
+        kern<<<(unsigned)(B * JC), 32 * we, smem, st>>>(G_dev, C, w, 1e-22, 1e-9, 30, lam_dev, Bt_dev, status_dev);
         return LRS_OK;
     };
     const int rows = (C + 31) / 32;                    // rows of a column per lane
@@ -347,6 +354,16 @@ extern "C" int lrs_sym_eig_jacobi_f64(const double* G_dev, int C, double* lam_de
     if (rc != LRS_OK) return rc;
     note_launch();
     return check_cuda(fn, cudaGetLastError());
+}
+
+extern "C" int lrs_sym_eig_jacobi_f64(const double* G_dev, int C, double* lam_dev, double* Bt_dev, int* status_dev,
+                                      lrs_stream_t stream) {
+    return jacobi_launch("lrs_sym_eig_jacobi_f64", G_dev, 1, C, lam_dev, Bt_dev, status_dev, (cudaStream_t)stream);
+}
+
+extern "C" int lrs_sym_eig_jacobi_batch_f64(const double* G_dev, int64_t B, int C, double* lam_dev, double* Bt_dev,
+                                            int* status_dev, lrs_stream_t stream) {
+    return jacobi_launch("lrs_sym_eig_jacobi_batch_f64", G_dev, B, C, lam_dev, Bt_dev, status_dev, (cudaStream_t)stream);
 }
 
 #ifdef LRS_DIAGNOSTICS

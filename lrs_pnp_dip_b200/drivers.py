@@ -4,7 +4,10 @@ hard-coded ``/home/s1809498/...`` paths:
     python -m lrs_pnp_dip_b200.drivers lrs_pnp  --data-dir <ref>/data --image img5 --mask fourth_mask
     python -m lrs_pnp_dip_b200.drivers lrs_pnp_dip --net skip   --reference-root <ref> ...
     python -m lrs_pnp_dip_b200.drivers lrs_pnp_dip --net 1lip   --reference-root <ref> ...
+    python -m lrs_pnp_dip_b200.drivers lrs_pnp_batch --data-dir <ref>/data [--pairs base:fourth_mask,img2:second_mask]
 
+``lrs_pnp_batch`` runs the same loop for many (image, mask) pairs at once (:class:`LRSPnPBatch`, one kernel of each
+kind per outer iteration for all cubes): by default every bundled image against each of the four distinct masks.
 ``lrs_pnp`` is main_LRS_PnP.py:159-451 (ADMM with the sparse step, SVT and the closed-form X update on the
 GPU, metrics printed per outer iteration).  ``lrs_pnp_dip`` is main_LRS_PnP_DIP_pro.py / _1-LiP.py: the same
 loop with the low-rank step replaced by a deep image prior that stays the REFERENCE's own PyTorch module
@@ -23,19 +26,40 @@ from __future__ import annotations
 import argparse
 import os
 import sys
-from typing import Callable, Optional
+from typing import Callable, List, Optional, Tuple
 
 import numpy as np
 import torch
 
 from . import matio, metrics, synth
-from .solver import LRSPnP, Params
+from .solver import LRSPnP, LRSPnPBatch, Params
 
 PAIRS = {"base": ("low_rank_sparsity_noisy.mat", "low_rank_sparsity_clean.mat", "low_rank_sparsity_mask.mat"),
          "img2": ("low_rank_sparsity_noisy_img2.mat", "low_rank_sparsity_clean_img2.mat", "second_mask.mat"),
          "img3": ("low_rank_sparsity_noisy_img3.mat", "low_rank_sparsity_clean_img3.mat", "third_mask.mat"),
          "img4": ("low_rank_sparsity_noisy_img4.mat", "low_rank_sparsity_clean_img4.mat", "fourth_mask.mat"),
          "img5": ("low_rank_sparsity_noisy_img5.mat", "low_rank_sparsity_clean_img5.mat", "fourth_mask.mat")}
+
+
+# the distinct masks of PAIRS (img5 shares img4's fourth mask), in the order of the images that own them
+BATCH_MASKS = ("low_rank_sparsity_mask", "second_mask", "third_mask", "fourth_mask")
+
+
+def batch_pairs(spec: Optional[str] = None) -> List[Tuple[str, str]]:
+    """(image, mask) pairs of ``lrs_pnp_batch``: ``spec`` = "image:mask,image:mask,..." (mask names with or without
+    ``.mat``), or None = every image of PAIRS against each of BATCH_MASKS (5 x 4 = 20 cubes, image-major)."""
+    if spec is None:
+        return [(img, m) for img in PAIRS for m in BATCH_MASKS]
+    out = []
+    for item in spec.split(","):
+        img, sep, m = item.strip().partition(":")
+        m = m[:-4] if m.endswith(".mat") else m
+        if not sep or img not in PAIRS or m not in BATCH_MASKS:
+            raise ValueError(f"bad pair {item!r}: expected image:mask with image in {sorted(PAIRS)} and mask in {BATCH_MASKS}")
+        out.append((img, m))
+    if not out:
+        raise ValueError("no (image, mask) pair given")
+    return out
 
 
 def load_case(data_dir: str, image: str, mask: Optional[str] = None):
@@ -155,6 +179,39 @@ def run(noisy: np.ndarray, clean: np.ndarray, msk: np.ndarray, D: np.ndarray, pr
     return sol, history
 
 
+def load_pair(data_dir: str, image: str, mask: str):
+    """Cube (image, mask) of a batch: the image's observed cube with the pixels missing in ``mask`` also zeroed
+    (:func:`synth.cross_masked`) → (Y [R, C], MtM [R, C], clean cube [1, B, d2, d3])."""
+    noisy, clean, _ = load_case(data_dir, image)
+    msk = np.asarray(matio.loadmat_any(os.path.join(data_dir, mask + ".mat"))["msk"], dtype=np.uint8)
+    Y, MtM = synth.cross_masked(matio.unfold_cube(noisy), matio.unfold_mask(msk, 1)[:, 0])
+    return Y, MtM, clean
+
+
+def run_batch(cases, D: np.ndarray, prm: Params, iteration_num: int, engine: str = "auto", device="cuda", log=print):
+    """The outer loop for a batch of cubes of one shape: ``cases`` = [(label, Y [R, C], MtM [R, C], clean [1, B, d2, d3])],
+    e.g. from :func:`batch_pairs` / :func:`load_pair`.  One :class:`LRSPnPBatch` runs them together; MPSNR / MSSIM of every
+    cube are logged after each outer iteration.  Returns (solver, history) with history[it][b] = {mpsnr, mssim}."""
+    dev = torch.device(device)
+    labels = [c[0] for c in cases]
+    Y = np.stack([c[1] for c in cases])
+    MtM = np.stack([c[2] for c in cases])
+    cleans = [torch.from_numpy(np.asarray(c[3], dtype=np.float32)).to(dev) for c in cases]
+    _, _, d2, d3 = cases[0][3].shape
+    sol = LRSPnPBatch(Y, MtM, D, prm, engine=engine, device=dev)
+    history = []
+    for itr in range(iteration_num):
+        sol.step()
+        rec = []
+        for b, lab in enumerate(labels):
+            img = metrics.fold(sol.X[b], d2, d3)
+            rec.append(dict(cube=lab, mpsnr=metrics.mpsnr(cleans[b], img), mssim=metrics.ssim(cleans[b], img)))
+        history.append(rec)
+        log(f"Outer-Loop Iteration {itr}: " + "  ".join(f"{r['cube']} {r['mpsnr']:.4f}/{r['mssim']:.4f}" for r in rec))
+    sol.validate()
+    return sol, history
+
+
 def main(argv=None):
     ap = argparse.ArgumentParser(prog="lrs_pnp_dip_b200.drivers", description=__doc__.split("\n\n")[0])
     sub = ap.add_subparsers(dest="cmd", required=True)
@@ -172,6 +229,14 @@ def main(argv=None):
             p.add_argument("--net", default="skip", choices=["skip", "1lip"])
             p.add_argument("--reference-root", required=True)
             p.add_argument("--dip-iterations", type=int, default=5000)
+    p = sub.add_parser("lrs_pnp_batch")
+    p.add_argument("--data-dir", required=True)
+    p.add_argument("--pairs", default=None, help="image:mask,... (default: every image x each of the four masks)")
+    p.add_argument("--dictionary", default=None)
+    p.add_argument("--atoms", type=int, default=2592)
+    p.add_argument("--iterations", type=int, default=2)
+    p.add_argument("--engine", default="auto")
+    p.add_argument("--denoiser", default="soft", choices=["soft", "nlm", "identity"])
     p = sub.add_parser("learn_dict")
     p.add_argument("--data-dir", required=True)
     p.add_argument("--image", default="base", choices=sorted(PAIRS))
@@ -194,8 +259,13 @@ def main(argv=None):
         print(f"learned {tuple(D.shape)} dictionary from {patches.shape[1]} patches; relative error per round: "
               + " ".join(f"{h:.4f}" for h in hist))
         return
-    noisy, clean, msk = load_case(a.data_dir, a.image, a.mask)
     bb = 36
+    if a.cmd == "lrs_pnp_batch":
+        cases = [(f"{img}+{m}",) + load_pair(a.data_dir, img, m) for img, m in batch_pairs(a.pairs)]
+        D = load_dictionary(a.dictionary or os.path.join(a.data_dir, "trained_dictionary.mat"), bb * bb, a.atoms)
+        run_batch(cases, D, Params(denoiser=a.denoiser), a.iterations, engine=a.engine)
+        return
+    noisy, clean, msk = load_case(a.data_dir, a.image, a.mask)
     D = load_dictionary(a.dictionary or os.path.join(a.data_dir, "trained_dictionary.mat"), bb * bb, a.atoms)
     if a.cmd == "lrs_pnp":
         prm = Params(denoiser=a.denoiser)                                      # main_LRS_PnP.py:218-238

@@ -101,6 +101,28 @@ def col2im(blocks: torch.Tensor, R: int, C: int, bb: int, s: int) -> torch.Tenso
     return out
 
 
+def im2col_batch(X: torch.Tensor, bb: int, s: int, lambda_1: Optional[torch.Tensor] = None, mu_1: float = 1.0) -> torch.Tensor:
+    """Patch matrices of B cubes ``X [B, R, C]`` (or of ``X + lambda_1/mu_1``) side by side: ``[bb², B*P]``, cube b in
+    columns ``[b*P, (b+1)*P)``."""
+    B, R, C = X.shape
+    P = patch_count(R, C, bb, s)
+    out = torch.empty((bb * bb, B * P), dtype=torch.float32, device=X.device)
+    check(lib().lrs_im2col_batch_f32(ptr(X), ptr(lambda_1), float(mu_1), B, R, C, bb, s, ptr(out), stream_ptr()),
+          "lrs_im2col_batch_f32")
+    return out
+
+
+def col2im_batch(blocks: torch.Tensor, B: int, R: int, C: int, bb: int, s: int) -> torch.Tensor:
+    """Overlap sums ``[B, R, C]`` of ``blocks [bb², B*P]`` (cube b in columns ``[b*P, (b+1)*P)``), each bit-exact with
+    :func:`col2im` on its own columns."""
+    blocks = blocks.contiguous()
+    if tuple(blocks.shape) != (bb * bb, B * patch_count(R, C, bb, s)):
+        raise ValueError(f"blocks has shape {tuple(blocks.shape)}, geometry needs {(bb * bb, B * patch_count(R, C, bb, s))}")
+    out = torch.empty((B, R, C), dtype=torch.float32, device=blocks.device)
+    check(lib().lrs_col2im_accum_batch_f32(ptr(blocks), B, R, C, bb, s, ptr(out), stream_ptr()), "lrs_col2im_accum_batch_f32")
+    return out
+
+
 def coverage_weight(R: int, C: int, bb: int, s: int, device="cuda") -> torch.Tensor:
     """``Weight`` of main_LRS_PnP.py:341."""
     require_cuda()
@@ -391,6 +413,72 @@ def sym_eig_jacobi(G: torch.Tensor):
     status = torch.empty(3, dtype=torch.int32, device=G.device)
     check(lib().lrs_sym_eig_jacobi_f64(ptr(G), C, ptr(lam), ptr(Bt), ptr(status), stream_ptr()), "lrs_sym_eig_jacobi_f64")
     return lam, Bt, status
+
+
+def sym_eig_jacobi_batch(G: torch.Tensor):
+    """(lam [B, C], Bt [B, C, C], status [B, 3] int32) of lrs_sym_eig_jacobi_batch_f64 for B symmetric PSD fp64 matrices
+    ``G [B, C, C]``; slice b is what :func:`sym_eig_jacobi` gives for ``G[b]``.  No host synchronisation."""
+    B, C = G.shape[0], G.shape[-1]
+    if G.dtype != torch.float64 or G.dim() != 3 or G.shape[1] != C or not 1 <= C <= JACOBI_MAX_C:
+        raise ValueError("sym_eig_jacobi_batch needs [B, C, C] fp64 matrices of order 1..256")
+    G = G.contiguous()
+    lam = torch.empty((B, C), dtype=torch.float64, device=G.device)
+    Bt = torch.empty((B, C, C), dtype=torch.float64, device=G.device)
+    status = torch.empty((B, 3), dtype=torch.int32, device=G.device)
+    check(lib().lrs_sym_eig_jacobi_batch_f64(ptr(G), B, C, ptr(lam), ptr(Bt), ptr(status), stream_ptr()),
+          "lrs_sym_eig_jacobi_batch_f64")
+    return lam, Bt, status
+
+
+def eig_status_failures(status) -> Tuple[list, list]:
+    """Cubes (indices) whose eigensolve met a non-finite Gram matrix, and those that did not converge, from the host
+    status words ``[B, 3]`` of :func:`sym_eig_jacobi_batch`."""
+    st = np.asarray(status).reshape(-1, 3)
+    return [int(b) for b in np.flatnonzero(st[:, 2])], [int(b) for b in np.flatnonzero((st[:, 1] != 0) & (st[:, 2] == 0))]
+
+
+def svt_weights_batch(G: torch.Tensor, tau: float, solver: str = "auto", status_sink=None) -> torch.Tensor:
+    """W [B, C, C] of :func:`svt_weights` for each of the B Gram matrices ``G [B, C, C]``.  'jacobi' (auto up to
+    JACOBI_AUTO_C): one launch of the batched cluster eigensolver, status words [B, 3] handed to ``status_sink`` (None:
+    checked here); 'library': torch.linalg.eigh on the batch (synchronises)."""
+    B, C = G.shape[0], G.shape[-1]
+    if solver == "auto":
+        solver = "jacobi" if C <= JACOBI_AUTO_C else "library"
+    W = torch.empty((B, C, C), dtype=torch.float32, device=G.device)
+    if solver == "jacobi":
+        lam, Bt, status = sym_eig_jacobi_batch(G)
+        check(lib().lrs_svt_weights_batch_f64(ptr(lam), ptr(Bt), C * C, 1, C, B, C, C, float(tau), 1, ptr(W), stream_ptr()),
+              "lrs_svt_weights_batch_f64")
+        if status_sink is None:
+            raise_for_batch_status(status.cpu())
+        else:
+            status_sink(status)
+        return W
+    if solver != "library":
+        raise ValueError(solver)
+    try:
+        evals, V = torch.linalg.eigh(G)
+    except RuntimeError as e:
+        fin = torch.isfinite(G).flatten(1).all(1).cpu()
+        bad = [b for b in range(B) if not bool(fin[b])]
+        raise _lib.LrsError(f"cube(s) {bad}: {_DIVERGED}" if bad else f"SVT: batched eigh failed: {e}") from e
+    fin = torch.isfinite(evals).all(1).cpu()              # eigh has synchronised on its status words already
+    bad = [b for b in range(B) if not bool(fin[b])]
+    if bad:
+        raise _lib.LrsError(f"cube(s) {bad}: {_DIVERGED}")
+    check(lib().lrs_svt_weights_batch_f64(ptr(evals), ptr(V), V.stride(0), V.stride(1), V.stride(2), B, C, C, float(tau), 0,
+                                          ptr(W), stream_ptr()), "lrs_svt_weights_batch_f64")
+    return W
+
+
+def raise_for_batch_status(status) -> None:
+    """Raise naming the cubes of a batch whose eigensolve met a non-finite Gram matrix or did not converge (host status
+    words [B, 3])."""
+    nonfinite, unconverged = eig_status_failures(status)
+    if nonfinite:
+        raise _lib.LrsError(f"cube(s) {nonfinite}: {_DIVERGED}")
+    if unconverged:
+        raise _lib.LrsError(f"cube(s) {unconverged}: SVT: the Jacobi eigensolver did not converge")
 
 
 def svt_weights(G: torch.Tensor, tau: float, solver: str = "auto", status_sink=None) -> torch.Tensor:

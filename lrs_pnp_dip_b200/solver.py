@@ -669,3 +669,174 @@ class LRSPnP:
             self.step()
         self.validate()
         return self
+
+
+# --------------------------------------------------------------------------------------------------
+# a batch of same-shape cubes in one ADMM loop (explicit engine)
+# --------------------------------------------------------------------------------------------------
+def _batch_inputs(Y_observed, MtM, D, prm: Params, low_rank, engine: str):
+    """Host-side checks of LRSPnPBatch's inputs (no device needed): returns (Y, MtM, D) as tensors, not yet moved."""
+    if low_rank is not None:
+        raise _lib.LrsError("LRSPnPBatch runs the SVT low-rank step only; a low_rank callable (a DIP network) needs one "
+                            "LRSPnP per cube")
+    if prm.step == "spectral_patch":
+        raise _lib.LrsError("LRSPnPBatch serves explicit patch matrices: step='spectral_patch' (bb <= 8 fused engines) is "
+                            "not supported; use step='spectral' or 'frob4', or one LRSPnP per cube")
+    if prm.step not in ("spectral", "frob4"):
+        raise ValueError(f"unknown step mode {prm.step!r}")
+    if prm.denoiser not in _lib.DENOISERS:
+        raise ValueError(f"unknown denoiser {prm.denoiser!r}")
+    if engine not in _lib.ENGINES:
+        raise ValueError(f"unknown engine {engine!r}")
+    Y, M, Dt = (torch.as_tensor(a) for a in (Y_observed, MtM, D))
+    if Y.dim() != 3 or tuple(M.shape) != tuple(Y.shape):
+        raise ValueError(f"Y_observed and MtM must both be [B, R, C] (got {tuple(Y.shape)} and {tuple(M.shape)})")
+    if Y.dtype != M.dtype or not Y.dtype.is_floating_point:
+        raise ValueError(f"Y_observed and MtM must share one floating-point dtype (got {Y.dtype} and {M.dtype})")
+    if Dt.dim() != 2 or not Dt.dtype.is_floating_point:
+        raise ValueError("D must be a floating-point [bb², K] matrix")
+    B, R, C = Y.shape
+    if not 1 <= B <= _lib.MAX_BATCH:
+        raise ValueError(f"a batch holds 1..{_lib.MAX_BATCH} cubes (got B = {B})")
+    if prm.bb < 1 or prm.slidingDis < 1 or prm.bb > min(R, C):
+        raise ValueError(f"invalid geometry: R={R} C={C} bb={prm.bb} stride={prm.slidingDis}")
+    if Dt.shape[0] != prm.bb * prm.bb:
+        raise ValueError(f"dictionary has {Dt.shape[0]} rows, bb² = {prm.bb * prm.bb}")
+    if prm.bb == 8 and Dt.shape[1] in FUSED_K and prm.denoiser == "soft":
+        raise _lib.LrsError(f"bb = 8, K = {Dt.shape[1]} with the soft denoiser runs on the fused engines, which fill the GPU "
+                            "from one cube: use one LRSPnP per cube (LRSPnPBatch serves the explicit engine)")
+    return Y, M, Dt
+
+
+class BatchSparseCoder:
+    """The sparse step of B cubes of one geometry as ONE explicit-engine problem: the patch matrices of all cubes side by
+    side ([n, B*P], cube b in columns [b*P, (b+1)*P)), one ISTA call over all B*P columns, one overlap sum per cube.
+    Step constants come from the concatenated observed patches (patterns shared between cubes: one eigensolve)."""
+
+    def __init__(self, Y_observed: torch.Tensor, D: torch.Tensor, prm: Params):
+        self.Y, self.D, self.prm = Y_observed, D, prm
+        self.B, self.R, self.C = Y_observed.shape
+        self.n, self.K = D.shape
+        self.P = ops.patch_count(self.R, self.C, prm.bb, prm.slidingDis)
+        self.fused = False
+        self.blocks_copy = ops.im2col_batch(self.Y, prm.bb, prm.slidingDis)
+        self.a_patch = ops.step_constants(self.blocks_copy, self.D, prm.step)
+
+    def phi_z(self, X: torch.Tensor, lambda_1: Optional[torch.Tensor]) -> torch.Tensor:
+        """Phi_z [n, B*P] of main_LRS_PnP.py:259-303 for V = X + lambda_1/mu_1 of every cube."""
+        prm = self.prm
+        with _on(X):
+            blocks = ops.im2col_batch(X, prm.bb, prm.slidingDis, lambda_1, prm.mu_1)
+            _, phi = ops.ista_batched(blocks, self.blocks_copy, self.D, self.a_patch, prm.lambda_ista, prm.Nit,
+                                      denoiser=prm.denoiser, h_scale=prm.nlm_h_scale)
+            return phi
+
+    def imout(self, X: torch.Tensor, lambda_1: Optional[torch.Tensor]) -> torch.Tensor:
+        """Overlap sums [B, R, C] (main_LRS_PnP.py:332-339) of every cube."""
+        with _on(X):
+            return ops.col2im_batch(self.phi_z(X, lambda_1), self.B, self.R, self.C, self.prm.bb, self.prm.slidingDis)
+
+
+class LRSPnPBatch:
+    """ADMM driver for B cubes that share one dictionary, one Params and one geometry: ``Y_observed``, ``MtM`` are
+    [B, R, C] and so are ``X``, ``lambda_1``, ``lambda_2``.  Cube b evolves as ``LRSPnP`` would evolve it alone; the
+    batch runs each kernel of an outer iteration once for all cubes.  Served on the explicit engine (shapes where
+    ``SparseCoder.fused`` is false) with the SVT low-rank step, on one GPU."""
+
+    def __init__(self, Y_observed, MtM, D, prm: Params, engine: str = "auto", device=None, low_rank=None):
+        Y, M, Dt = _batch_inputs(Y_observed, MtM, D, prm, low_rank, engine)
+        _lib.require_cuda()
+        device = torch.device(device if device is not None else "cuda")
+        self.prm, self.engine = prm, engine
+        with torch.cuda.device(device):
+            self.Y = Y.to(device=device, dtype=torch.float32).contiguous()
+            self.MtM = M.to(device=device, dtype=torch.float32).contiguous()
+            self.D = Dt.to(device=device, dtype=torch.float32).contiguous()
+            self.coder = BatchSparseCoder(self.Y, self.D, prm)
+            self.X = self.Y.clone()                          # X = Y_observed          (:229)
+            self.lambda_1 = torch.zeros_like(self.Y)         # (:219)
+            self.lambda_2 = torch.zeros_like(self.Y)         # (:220)
+        self.B, self.R, self.C = self.Y.shape
+        self.iterations = 0
+        self._side = None
+        self._pending: list = []
+
+    def reset(self) -> None:
+        """Every cube back to X = Y_observed, λ1 = λ2 = 0 (main_LRS_PnP.py:219-220,229), on the current stream."""
+        with _on(self.X):
+            self.X.copy_(self.Y)
+            self.lambda_1.zero_()
+            self.lambda_2.zero_()
+        self.iterations = 0
+
+    def _defer_status(self, status: torch.Tensor) -> None:
+        """Jacobi status words [B, 3] travel to pinned host memory behind the kernels that produced them (no stall)."""
+        host = torch.empty(tuple(status.shape), dtype=torch.int32).pin_memory()
+        host.copy_(status, non_blocking=True)
+        ev = torch.cuda.Event()
+        ev.record()
+        self._pending.append((host, ev))
+
+    def _check_status(self, wait: bool) -> None:
+        while self._pending:
+            host, ev = self._pending[0]
+            if wait:
+                ev.synchronize()
+            elif not ev.query():
+                return
+            self._pending.pop(0)
+            ops.raise_for_batch_status(host.numpy())
+
+    def _low_rank(self) -> torch.Tensor:
+        """SVT of Z_b = X_b + λ2_b/μ2 with τ = 1/μ2 for every cube (main_LRS_PnP.py:315) on the current stream."""
+        c = 1.0 / self.prm.mu_2
+        B, R, C = self.B, self.R, self.C
+        G = torch.zeros((B, C, C), dtype=torch.float64, device=self.X.device)
+        check(lib().lrs_gram_batch_f64(ptr(self.X), ptr(self.lambda_2), float(c), B, R, C, ptr(G), stream_ptr()),
+              "lrs_gram_batch_f64")
+        W = ops.svt_weights_batch(G, c, status_sink=self._defer_status)
+        U = torch.empty_like(self.X)
+        check(lib().lrs_svt_apply_batch_f32(ptr(self.X), ptr(self.lambda_2), float(c), ptr(W), B, R, C, ptr(U), stream_ptr()),
+              "lrs_svt_apply_batch_f32")
+        return U
+
+    def step(self) -> None:
+        """One outer iteration (main_LRS_PnP.py:259-362) of every cube."""
+        with _on(self.X):
+            self._step()
+
+    def _step(self) -> None:
+        prm = self.prm
+        self._check_status(wait=False)                   # deferred eigensolver verdicts of earlier steps (no stall)
+        main = torch.cuda.current_stream()
+        if self._side is None:
+            self._side = _side_stream(self.X.device)
+        # as LRSPnP's explicit path: the low-rank step runs on the side stream beside the sparse step; with the Jacobi
+        # eigensolver it never blocks the host and is enqueued first, the library eigensolver synchronises and goes second
+        self._side.wait_stream(main)
+        lr_async = self.C <= ops.JACOBI_AUTO_C
+        if lr_async:
+            with torch.cuda.stream(self._side):
+                U = self._low_rank()
+        IMout = self.coder.imout(self.X, self.lambda_1)
+        if not lr_async:
+            with torch.cuda.stream(self._side):
+                U = self._low_rank()
+        main.wait_stream(self._side)
+        U.record_stream(main)
+        check(lib().lrs_admm_update_batch_f32(ptr(self.Y), ptr(self.MtM), ptr(IMout), ptr(U), ptr(self.lambda_1),
+                                              ptr(self.lambda_2), ptr(self.X), float(prm.gamma), float(prm.mu_1),
+                                              float(prm.mu_2), self.B, self.R, self.C, prm.bb, prm.slidingDis, stream_ptr()),
+              "lrs_admm_update_batch_f32")
+        self.iterations += 1
+
+    def validate(self) -> None:
+        """Wait for the deferred eigensolver verdicts; raise naming the cube(s) whose eigensolve met a non-finite Gram
+        matrix (a diverged state) or did not converge."""
+        self._check_status(wait=True)
+
+    def run(self, iteration_num: int) -> "LRSPnPBatch":
+        for _ in range(iteration_num):
+            self.step()
+        self.validate()
+        return self

@@ -94,3 +94,14 @@ def observe(noisy: np.ndarray, pix_mask: np.ndarray) -> np.ndarray:
     else:
         Y[pix_mask.reshape(Y.shape) == 0] = 0
     return Y
+
+
+def cross_masked(Y: np.ndarray, pix_mask: np.ndarray):
+    """Cube (i, m) of the batched experiments: the observed cube ``Y [R, C]`` of image i (already zero on its own
+    missing pixels) with the pixels missing in mask m (``pix_mask [R]``, 0 = missing, unfolded pixel order) zeroed too.
+    Returns ``(Y_im [R, C] f32, MtM [R, C] f32)``; MtM is the row indicator of the pixels still observed (a row of Y
+    that is not all zero, and kept by mask m), replicated over the bands."""
+    Y = np.asarray(Y, dtype=F32)
+    keep = (np.asarray(pix_mask).reshape(-1) != 0) & (Y != 0).any(axis=1)
+    Yim = np.where(keep[:, None], Y, F32(0)).astype(F32)
+    return np.ascontiguousarray(Yim), np.ascontiguousarray(np.repeat(keep.astype(F32)[:, None], Y.shape[1], axis=1))

@@ -204,7 +204,7 @@ def step_constants(blocks_copy: torch.Tensor, D: torch.Tensor, step: str) -> tor
     uniq = m[rep]
     if not bool((uniq[inv] == m).all()):                          # a hash collision merged two patterns: exact fallback
         uniq, inv = torch.unique(m, dim=0, return_inverse=True)
-    if uniq.shape[0] > 4096:
+    if uniq.shape[0] > MAX_SPECTRAL_PATTERNS:
         raise _lib.LrsError(f"{uniq.shape[0]} distinct mask patterns: spectral step constants need one eigensolve "
                             "each; use step='frob4' or pass explicit step constants")
     # One eigensolve per distinct pattern AND dictionary, ever: the value depends on (D, pattern) only, the reference pays an
@@ -227,6 +227,7 @@ def step_constants(blocks_copy: torch.Tensor, D: torch.Tensor, step: str) -> tor
 
 
 _SPECTRAL_CACHE: dict = {}
+MAX_SPECTRAL_PATTERNS = 4096             # distinct mask patterns step_constants solves (one eigensolve each)
 
 
 def row_pattern_table(D: torch.Tensor, bb: int, step: str) -> torch.Tensor:

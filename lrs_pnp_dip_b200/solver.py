@@ -720,7 +720,12 @@ class BatchSparseCoder:
         self.P = ops.patch_count(self.R, self.C, prm.bb, prm.slidingDis)
         self.fused = False
         self.blocks_copy = ops.im2col_batch(self.Y, prm.bb, prm.slidingDis)
-        self.a_patch = ops.step_constants(self.blocks_copy, self.D, prm.step)
+        try:
+            self.a_patch = ops.step_constants(self.blocks_copy, self.D, prm.step)
+        except _lib.LrsError as e:        # too many distinct patterns; a batch takes no explicit step constants
+            raise _lib.LrsError(f"a batch of {self.B} cubes: {e.args[0].split(':')[0]}, more than the "
+                                f"{ops.MAX_SPECTRAL_PATTERNS} that spectral step constants serve (one eigensolve each); use "
+                                "step='frob4', or fewer cubes per batch") from e
 
     def phi_z(self, X: torch.Tensor, lambda_1: Optional[torch.Tensor]) -> torch.Tensor:
         """Phi_z [n, B*P] of main_LRS_PnP.py:259-303 for V = X + lambda_1/mu_1 of every cube."""

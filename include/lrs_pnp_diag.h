@@ -27,6 +27,15 @@ int lrs_tc_timing_read(unsigned long long* out32_host);
  * (the caller zeroes it; a correct walk leaves every entry at 1), tiles_host receives the number of tiles.  bb = 8. */
 int lrs_debug_tile_walk(int64_t R, int64_t C, int bb, int s, int64_t p_begin, int64_t p_end, int sms, int* visits_host,
                         int64_t* tiles_host);
+/* HOST-side replay (no GPU needed) of the launch plan of lrs_ista_pnp_f32 for an [n, K] dictionary and P patches;
+ * out_host = int64 [15] in HOST memory:
+ *   [0]  engine by shape: 1 = tensor-core (ista_tc.cu; LRS_ISTA_ENGINE=simt still forces the FFMA engine), 0 = FFMA
+ *   tensor-core plan (0 when [0] is 0): [1] Np = P rounded up to 16, [2] patch tiles of 256 columns, [3] width of the
+ *   last tile, [4] pipeline stages, [5] S1 / [6] k blocks per split of D alpha, [7] S2 / [8] of D^T r, [9] / [10] k blocks
+ *   of the last split of D alpha / D^T r
+ *   FFMA engine (any shape): [11] / [12] k splits of the residual / gradient GEMM, [13] / [14] their rows per CTA
+ *   (on a 148-SM device). */
+int lrs_debug_ista_plan(int n, int K, int64_t P, int64_t* out_host);
 /* HOST-side replay (no GPU needed) of ONE sweep of the parallel order of lrs_sym_eig_jacobi_f64 (csrc/jacobi_eig.cu) for C
  * columns: meets_host[p*C + q] (p < q; caller zeroes C*C ints) counts how often columns p and q are paired — a correct order
  * leaves every p < q at 1 —, conflicts_host the sub-rounds in which a column was used twice, subrounds_host their number. */

@@ -126,6 +126,9 @@ size_t ista_tc_workspace_bytes(int n, int K, int64_t P);
 int ista_tc_run(const float* blocks, const float* blocks_copy, const float* D, const float* a, float lambda, int Nit, int n,
                 int K, int64_t P, int denoiser, float h_scale, float* coefs, float* phi, void* ws, size_t ws_bytes,
                 cudaStream_t st);
+// ista_generic.cu: split-K count and rows per CTA of the FFMA engine's GEMMs (M x N output, Kd deep)
+int ista_splits(int64_t M, int64_t N, int64_t Kd);
+int ista_row_tile(int64_t M, int64_t N, int splits, int sms);
 // ista_generic.cu: A = NLmeansfilter(G, 3, 3, h_scale * T) column by column (NLmeansfilter.m:18-91)
 int nlm_columns(const char* fn, const float* G, const float* T, float h_scale, int K, int64_t P, float* A, cudaStream_t st);
 

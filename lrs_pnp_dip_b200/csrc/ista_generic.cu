@@ -247,7 +247,7 @@ __global__ void splitk_epilogue_kernel(const float* __restrict__ partial, int sp
 }
 
 // Number of k-splits for an ISTA GEMM: enough CTAs for ~4 per SM on the small-P problems, none on the large ones.
-static int ista_splits(int64_t M, int64_t N, int64_t Kd) {
+int ista_splits(int64_t M, int64_t N, int64_t Kd) {
     const int64_t base = ((M + 31) / 32) * ((N + 47) / 48);
     int64_t sp = (592 + base - 1) / base;
     const int64_t by_k = Kd / (8 * BK);      // at least 8 k-tiles per split
@@ -256,12 +256,18 @@ static int ista_splits(int64_t M, int64_t N, int64_t Kd) {
     return sp < 1 ? 1 : (int)sp;
 }
 
+// Rows per CTA of an ISTA GEMM: 32 when split-K or when 64-row tiles would leave SMs idle, else 64.
+int ista_row_tile(int64_t M, int64_t N, int splits, int sms) {
+    const int64_t ncol = (N + 47) / 48;
+    return (splits > 1 || ((M + 63) / 64) * ncol < 2 * (int64_t)(sms > 0 ? sms : 148)) ? 32 : 64;
+}
+
 __global__ void ista_prepare_kernel(const float* __restrict__ a, float lambda, int64_t P, float* __restrict__ inv_a,
                                     float* __restrict__ T) {
     int64_t p = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (p >= P) return;
     float av = a[p];
-    bool ok = av > 0.0f;
+    bool ok = av > 0.0f && av < INFINITY;   // a <= 0, NaN or +inf: no step, the coefficients stay 0
     inv_a[p] = ok ? __fdiv_rn(1.0f, av) : 0.0f;
     T[p] = ok ? __fdiv_rn(lambda, __fmul_rn(2.0f, av)) : 0.0f;  // T = lambda/(2a), ista.m:17
 }
@@ -275,30 +281,47 @@ __global__ void nlm_column_kernel(const float* __restrict__ G, const float* __re
     const int k = blockIdx.y;
     if (p >= P) return;
     const float kw[7] = {1.0f / 21.0f, 4.0f / 35.0f, 71.0f / 315.0f, 71.0f / 315.0f, 71.0f / 315.0f, 4.0f / 35.0f, 1.0f / 21.0f};
-    float x[13];  // G[k-6 .. k+6] with symmetric (edge-including mirror) extension
+    float x[13];  // G[k-6 .. k+6] with symmetric (edge-including mirror) extension, reflected as often as a short column
+                  // needs (np.pad(..., mode="symmetric")): period 2K, the second half mirrored
 #pragma unroll
     for (int u = 0; u < 13; ++u) {
-        int idx = k - 6 + u;
-        if (idx < 0) idx = -idx - 1;
+        int idx = (k - 6 + u) % (2 * K);
+        if (idx < 0) idx += 2 * K;
         if (idx >= K) idx = 2 * K - 1 - idx;
-        idx = idx < 0 ? 0 : (idx >= K ? K - 1 : idx);
         x[u] = __ldg(G + (int64_t)idx * P + p);
     }
     const float h = h_scale * T[p];
-    const float inv_h2 = h > 0.f ? 1.0f / (h * h) : 0.f;
-    float wmax = 0.f, avg = 0.f, sw = 0.f;
+    const float h2 = h * h, inv_h2 = h2 > 0.f ? 1.0f / h2 : INFINITY;
+    // The reference's weights exp(-d / h^2) (double precision) are computed relative to the nearest window,
+    // exp(-(d - dmin) / h^2): avg / sw is unchanged by the common factor exp(-dmin / h^2), which in fp32 underflows to 0
+    // for every neighbour once dmin / h^2 > 87 and would return the input where the reference still averages.  A weight
+    // is 0 where the reference's double-precision exp underflows (d / h^2 > 745); if all are, the input is returned (:80-84).
+    float d[6];
+    float dmin = INFINITY;
 #pragma unroll
-    for (int dr = -3; dr <= 3; ++dr) {
-        if (dr == 0) continue;
-        const int r = k + dr;
-        if (r < 0 || r >= K) continue;  // the search window is clipped to the real column (:46-49)
-        float d = 0.f;
+    for (int j = 0; j < 6; ++j) {
+        const int dr = j < 3 ? j - 3 : j - 2;
+        d[j] = INFINITY;
+        if (k + dr < 0 || k + dr >= K) continue;  // the search window is clipped to the real column (:46-49)
+        float dd = 0.f;
 #pragma unroll
         for (int u = -3; u <= 3; ++u) {
             float e = x[6 + u] - x[6 + dr + u];
-            d = fmaf(kw[u + 3] * e, e, d);
+            dd = fmaf(kw[u + 3] * e, e, dd);
         }
-        float w = h > 0.f ? __expf(-d * inv_h2) : (d == 0.f ? 1.f : 0.f);
+        d[j] = dd;
+        dmin = fminf(dmin, dd);
+    }
+    float wmax = 0.f, avg = 0.f, sw = 0.f;
+#pragma unroll
+    for (int j = 0; j < 6; ++j) {
+        const int dr = j < 3 ? j - 3 : j - 2;
+        if (k + dr < 0 || k + dr >= K) continue;
+        float w;
+        if (!(h > 0.f)) w = d[j] == 0.f ? 1.f : 0.f;
+        else if (d[j] == 0.f) w = 1.f;                                   // also when h^2 underflows
+        else if (d[j] * inv_h2 > 745.0f) w = 0.f;
+        else w = d[j] == dmin ? 1.f : __expf(-(d[j] - dmin) * inv_h2);
         wmax = fmaxf(wmax, w);
         sw += w;
         avg = fmaf(w, x[6 + dr], avg);
@@ -326,8 +349,8 @@ static int launch_gemm(const char* fn, LoadPlain al, const float* B, int64_t M, 
     static int sms = device_sm_count();
     const int64_t ncol = (N + 47) / 48;
     const int splits = scratch ? ista_splits(M, N, Kd) : 1;
-    const bool small = splits > 1 || ((M + 63) / 64) * ncol < 2 * (int64_t)(sms > 0 ? sms : 148);
-    const int bm = small ? 32 : 64;
+    const int bm = ista_row_tile(M, N, splits, sms);
+    const bool small = bm == 32;
     dim3 grid((unsigned)ncol, (unsigned)((M + bm - 1) / bm), (unsigned)splits);
     if (grid.y > 65535) return fail_arg(fn, "matrix too tall for this engine");
     if (splits > 1) {

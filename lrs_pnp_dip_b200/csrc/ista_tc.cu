@@ -12,8 +12,10 @@
 //   x = x1 + x2, x1 = fp16(x), x2 = fp16(x - x1);   a b ~ a1 b1 + a2 b1 + a1 b2   (fp32 accumulate).
 // The pieces of D (and of D^T, so that both products read a K-major A operand) are made once per call; the pieces of
 // alpha and r are written by the reduce kernels.  Every operand is normalised by an exact power of two first — D by
-// its largest entry, every patch column by its largest observed value — so the fp16 pieces are well scaled whatever
-// the scale of the data, and the products are scaled back exactly in the reduce kernels.
+// its largest entry, every patch column by its largest observed value (blocks_copy != 0; the unobserved entries of
+// `blocks` are the solver's current estimate, not data, and can be far larger) — so the fp16 pieces are well scaled
+// whatever the scale of the data, and the products are scaled back exactly in the reduce kernels.  A subnormal maximum
+// counts as 0 (as in the fused engine) and every exponent is clamped, so all scale factors are finite.
 #include <cuda_fp16.h>
 
 #include <cstdlib>
@@ -65,12 +67,19 @@ __global__ void absmax_kernel(const float* __restrict__ x, int64_t n, unsigned* 
     if ((threadIdx.x & 31) == 0 && m > 0.f && m < INFINITY) atomicMax(out, __float_as_uint(m));
 }
 
-__device__ __forceinline__ float pow2_down_scale(const unsigned* dmax_bits) {   // sd: sd * max|D| in [0.5, 1)
-    const float dmax = __uint_as_float(*dmax_bits);
+__host__ __device__ inline int clamp_int(int x, int lo, int hi) { return x < lo ? lo : (x > hi ? hi : x); }
+
+// ex with x = f 2^ex, f in [0.5, 1), for a normal finite x > 0; 0 for 0, subnormals and inf (2^-ex would overflow)
+__device__ __forceinline__ int pow2_exponent(float x) {
     int ex = 0;
-    if (dmax > 0.f) (void)frexpf(dmax, &ex);
-    return ldexpf(1.0f, -ex);
+    if (x >= 1.17549435e-38f && x < INFINITY) (void)frexpf(x, &ex);
+    return ex;
 }
+
+__device__ __forceinline__ int pow2_down_exp(const unsigned* dmax_bits) {   // sd = 2^-dex: sd * max|D| in [0.5, 1)
+    return pow2_exponent(__uint_as_float(*dmax_bits));
+}
+__device__ __forceinline__ float pow2_down_scale(const unsigned* dmax_bits) { return ldexpf(1.0f, -pow2_down_exp(dmax_bits)); }
 
 // Operand pieces live in global memory as the exact images of the shared-memory stages, so that a stage is ONE
 // contiguous bulk copy:
@@ -104,25 +113,31 @@ __global__ void dict_pieces_kernel(const float* __restrict__ D, int n, int K, co
 //   residual pieces   = fp16 split of  m .* (y - D alpha) * sR ,  sR = 2^-ex(y) / 4       (NOT yet divided by a: with a
 //                       large step constant r / a would fall into fp16's subnormal range)
 //   coefficient pieces = fp16 split of  alpha * sA ,  sA = 2^-ex(y) * 2^ex(sqrt a)          (alpha ~ y / ||d||, a ~ ||d||^2)
-__global__ void column_scales_kernel(const float* __restrict__ Y, int n, int64_t P, const unsigned* __restrict__ dmax_bits,
-                                     const float* __restrict__ a, float lambda, float* __restrict__ sA,
-                                     float* __restrict__ f1, float* __restrict__ f2, float* __restrict__ sR,
-                                     float* __restrict__ T) {
+// ex(y) comes from the largest OBSERVED |y| (BC != 0) only: the residual is zero on the other rows, and an unobserved
+// entry 2^12 times the observed ones would push the residual pieces into fp16's subnormal range.  Exponents are clamped
+// so that sA, sR, f1 and f2 are finite (and sA, sR nonzero) for every finite input and finite a > 0; inside the clamps
+// the factors are exact powers of two (f2: one rounding) and f1 is exactly 1 / (4 sd sA).
+__global__ void column_scales_kernel(const float* __restrict__ Y, const float* __restrict__ BC, int n, int64_t P,
+                                     const unsigned* __restrict__ dmax_bits, const float* __restrict__ a, float lambda,
+                                     float* __restrict__ sA, float* __restrict__ f1, float* __restrict__ f2,
+                                     float* __restrict__ sR, float* __restrict__ T) {
     const int64_t p = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (p >= P) return;
     float amax = 0.f;
-    for (int i = 0; i < n; ++i) amax = fmaxf(amax, fabsf(Y[(int64_t)i * P + p]));
-    int ex = 0;
-    if (amax > 0.f && amax < INFINITY) (void)frexpf(amax, &ex);
-    const float sd = pow2_down_scale(dmax_bits);
+    for (int i = 0; i < n; ++i)
+        if (BC[(int64_t)i * P + p] != 0.0f) amax = fmaxf(amax, fabsf(Y[(int64_t)i * P + p]));
+    const int ex = pow2_exponent(amax);                        // in [-125, 128]
+    const int dex = pow2_down_exp(dmax_bits);                  // sd = 2^-dex, dex in [-125, 128]
     const float av = a[p];
     const bool ok = av > 0.0f && av < INFINITY;
     int ea = 0;
     if (ok) (void)frexpf(sqrtf(av), &ea);
-    sA[p] = ldexpf(1.0f, ea - ex);
+    const int es = clamp_int(ea - ex, -126, 127);              // sA = 2^es
+    sA[p] = ldexpf(1.0f, es);
     sR[p] = ldexpf(TS_R, -ex);
-    f1[p] = ldexpf(1.0f, ex - ea) / (sd * TS_D);                               // D alpha   = (sum of MMAs) * f1
-    f2[p] = ok ? __fdiv_rn(ldexpf(1.0f, ex) / sd, av) : 0.0f;                  // D^T r / a = (sum of MMAs) * f2   (TS_D TS_R = 1)
+    f1[p] = ldexpf(1.0f, clamp_int(dex - 2 - es, -149, 127));                  // D alpha   = (sum of MMAs) * f1
+    f2[p] = ok ? fminf(__fdiv_rn(ldexpf(1.0f, clamp_int(ex + dex, -126, 127)), av), 3.40282347e38f)
+               : 0.0f;                                                         // D^T r / a = (sum of MMAs) * f2   (TS_D TS_R = 1)
     T[p] = ok ? __fdiv_rn(lambda, __fmul_rn(2.0f, av)) : 0.0f;
 }
 
@@ -485,9 +500,11 @@ static int launch_tc_gemm(const char* fn, const GemmArgs& g, int splits, cudaStr
     return rc;
 }
 
+// pipeline stages of the GEMM kernel: 3 while they fit 220 KB of shared memory (Np <= 160), else 2
+static int tc_stages(int64_t Np) { return 3 * (2 * A_PIECE + (size_t)b_slot_halves(Np) * 2) <= 220 * 1024 ? 3 : 2; }
+
 static int tc_gemm(const char* fn, const GemmArgs& g, int splits, cudaStream_t st) {
-    const size_t stage = 2 * A_PIECE + (size_t)b_slot_halves(g.Np) * 2;
-    return 3 * stage <= 220 * 1024 ? launch_tc_gemm<3>(fn, g, splits, st) : launch_tc_gemm<2>(fn, g, splits, st);
+    return tc_stages(g.Np) == 3 ? launch_tc_gemm<3>(fn, g, splits, st) : launch_tc_gemm<2>(fn, g, splits, st);
 }
 
 int ista_tc_run(const float* blocks, const float* blocks_copy, const float* D, const float* a, float lambda, int Nit,
@@ -520,7 +537,8 @@ int ista_tc_run(const float* blocks, const float* blocks_copy, const float* D, c
     LRS_CHECK_LAUNCH(fn);
     dict_pieces_kernel<<<(unsigned)((nD + 255) / 256), 256, 0, st>>>(D, n, K, dmax, A1, pl.Kp1 / TG_BK, A2, pl.Kp2 / TG_BK);
     LRS_CHECK_LAUNCH(fn);
-    column_scales_kernel<<<(unsigned)((P + 63) / 64), 64, 0, st>>>(blocks, n, P, dmax, a, lambda, sA, f1, f2, sR, T);
+    column_scales_kernel<<<(unsigned)((P + 63) / 64), 64, 0, st>>>(blocks, blocks_copy, n, P, dmax, a, lambda, sA, f1, f2,
+                                                                     sR, T);
     LRS_CHECK_LAUNCH(fn);
 
     GemmArgs g1{A1, B1, part, n, P, pl.Mp1, pl.Kp1, pl.Np, pl.kb1, (int)(pl.Kp1 / TG_BK)};   // D alpha
@@ -570,3 +588,35 @@ int ista_tc_run(const float* blocks, const float* blocks_copy, const float* D, c
 }
 
 }  // namespace lrs
+
+#ifdef LRS_DIAGNOSTICS
+#include "../../include/lrs_pnp_diag.h"
+
+// HOST replay of the launch plan of lrs_ista_pnp_f32 (layout of out_host: include/lrs_pnp_diag.h).
+extern "C" int lrs_debug_ista_plan(int n, int K, int64_t P, int64_t* out_host) {
+    using namespace lrs;
+    if (n <= 0 || K <= 0 || P <= 0 || !out_host) return fail_arg("lrs_debug_ista_plan", "bad arguments");
+    for (int i = 0; i < 15; ++i) out_host[i] = 0;
+    const bool tc = ista_tc_shape_ok(n, K, P);
+    out_host[0] = tc ? 1 : 0;
+    if (tc) {
+        const Plan pl = make_plan(n, K, P, PLAN_SMS);
+        out_host[1] = pl.Np;
+        out_host[2] = pl.ntiles;
+        out_host[3] = ptile_width(pl.Np, pl.ntiles - 1);
+        out_host[4] = tc_stages(pl.Np);
+        out_host[5] = pl.S1;
+        out_host[6] = pl.kb1;
+        out_host[7] = pl.S2;
+        out_host[8] = pl.kb2;
+        out_host[9] = pl.Kp1 / TG_BK - (int64_t)(pl.S1 - 1) * pl.kb1;
+        out_host[10] = pl.Kp2 / TG_BK - (int64_t)(pl.S2 - 1) * pl.kb2;
+    }
+    const int s1 = ista_splits(n, P, K), s2 = ista_splits(K, P, n);
+    out_host[11] = s1;
+    out_host[12] = s2;
+    out_host[13] = ista_row_tile(n, P, s1, PLAN_SMS);
+    out_host[14] = ista_row_tile(K, P, s2, PLAN_SMS);
+    return LRS_OK;
+}
+#endif  // LRS_DIAGNOSTICS

@@ -27,6 +27,11 @@ int lrs_tc_timing_read(unsigned long long* out32_host);
  * (the caller zeroes it; a correct walk leaves every entry at 1), tiles_host receives the number of tiles.  bb = 8. */
 int lrs_debug_tile_walk(int64_t R, int64_t C, int bb, int s, int64_t p_begin, int64_t p_end, int sms, int* visits_host,
                         int64_t* tiles_host);
+/* The same replay for the row-pattern tile order of the step-constant table mode: row_obs_host = R bytes, nonzero where
+ * a row of the matrix is observed; order_host (nR ints, may be null) receives the row starts in tile order, which is
+ * the stable sort of the row starts by the Gray rank of their 8-row validity word. */
+int lrs_debug_tile_walk_ordered(int64_t R, int64_t C, int bb, int s, int64_t p_begin, int64_t p_end, int sms,
+                                const unsigned char* row_obs_host, int* visits_host, int64_t* tiles_host, int* order_host);
 /* HOST-side replay (no GPU needed) of the launch plan of lrs_ista_pnp_f32 for an [n, K] dictionary and P patches;
  * out_host = int64 [15] in HOST memory:
  *   [0]  engine by shape: 1 = tensor-core (ista_tc.cu; LRS_ISTA_ENGINE=simt still forces the FFMA engine), 0 = FFMA

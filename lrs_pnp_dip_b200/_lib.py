@@ -69,6 +69,7 @@ DIAG_SIGNATURES = {
     "lrs_tc_probe_f32": (_int, [_p, _p, _p, _int, _int, _int, _int, _int, _p]),
     "lrs_tc_timing_read": (_int, [C.POINTER(C.c_uint64)]),
     "lrs_debug_tile_walk": (_int, [_i64, _i64, _int, _int, _i64, _i64, _int, _p, _p]),
+    "lrs_debug_tile_walk_ordered": (_int, [_i64, _i64, _int, _int, _i64, _i64, _int, _p, _p, _p, _p]),
     "lrs_debug_jacobi_schedule": (_int, [_int, _p, _p, _p]),
     "lrs_debug_ista_plan": (_int, [_int, _int, _i64, _p]),
     "lrs_tc_microbench": (_int, [_int, _int, _int, _int, _int, _int, _int, _int, _int, _p, _p]),

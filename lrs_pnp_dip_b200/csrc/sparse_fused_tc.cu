@@ -4,12 +4,19 @@
 // matrix run Nit soft-ISTA iterations against D and write Phi_z = D alpha (main_LRS_PnP.py:259-303,
 // ista.m:13-24).  Here the two contractions of every iteration run on the 5th-generation tensor cores:
 //
-//   tile        128 consecutive row starts of one column start = the 128 TMEM lanes = MMA M
+//   tile        128 row starts of one column start = the 128 TMEM lanes = MMA M (in the step-constant table mode the
+//               row starts are ordered by their row-validity pattern, so most tiles hold one pattern)
 //   GEMM-B      G[128 x K]    = alpha + r D        A operand = residual pieces in shared memory (SS form), two atom
-//                                                  halves, accumulated IN PLACE onto the fp32 state in TMEM
+//                                                  halves, accumulated IN PLACE onto the fp32 state in TMEM; only the
+//                                                  window rows observed in the tile, two rows per 16-pixel k-step
 //   epilogue    alpha = soft(G, T)                 tcgen05.ld -> registers -> tcgen05.st, 64-atom chunks
 //   GEMM-A      Da[128 x 64]  = alpha D^T          A operand = alpha pieces staged in TMEM (TS form)
 //   epilogue    r = m .* (y - Da / a)              fp16 pieces to shared memory, one 16-pixel k-step at a time
+//
+// Inside the kernel pixel i of a window is 8 * row + col (the reference's order is row + 8 * col), so that an 8-pixel
+// core-matrix group (a K group of GEMM-B, an N group of GEMM-A) is one window row: the residual is exactly zero on a
+// row no patch of the tile observes, and GEMM-B and the residual epilogue skip such rows.  Phi_z is stored in the
+// reference's order.
 //
 // so alpha (128 KB per tile) never leaves TMEM during the Nit iterations; HBM sees 3 gathers and one
 // Phi_z store per patch.
@@ -72,7 +79,7 @@ constexpr float S_D = 4.0f;          // D pieces        = fp16(4 D)
 constexpr float S_R = 0.25f;         // residual pieces = fp16(r / 4)  (S_R * S_D = 1: GEMM-B lands in the state's units)
 
 // D pieces in shared memory, one copy for both GEMMs (bytes):
-//   (k%8)*2 + (i%8)*16 + (8*piece + i/8)*128 + (k/8)*2048       i = pixel (row of D), k = atom
+//   (k%8)*2 + (i%8)*16 + (8*piece + i/8)*128 + (k/8)*2048       i = kernel pixel (8 * row + col), k = atom
 constexpr uint32_t D_SMEM_BYTES = 64 * 1024;
 // GEMM-B takes the residual pieces as the A operand from SHARED memory (SS form) and the 256 atoms in two N = 128
 // halves, so that the soft-threshold of the first half overlaps the MMAs of the second (an N = 128 MMA with A in
@@ -82,7 +89,7 @@ constexpr uint32_t R_SMEM_BYTES = 32 * 1024;
 constexpr uint32_t R_SK = 2048, R_SM = 128, R_PIECE = 16 * 1024;
 constexpr uint32_t D_SK = 2048, D_SI = 128;
 // Next tile's patch values, gathered by the otherwise idle warps 1..3 while the current tile iterates:
-// V = X + L/mu as [pixel][patch] floats (32 KB) and the observed flags as [pixel][patch] bytes (8 KB)
+// V = X + L/mu as [kernel pixel][patch] floats (32 KB) and the observed flags as [kernel pixel][patch] bytes (8 KB)
 constexpr uint32_t G_SMEM_BYTES = 64 * TILE * 4 + 64 * TILE;
 constexpr int NLOAD = 32 * (FIRST_EPI - 1);   // loader threads
 
@@ -102,7 +109,8 @@ struct __align__(8) Shared {
     uint32_t walk_done;       // set after the last announcement
     float xmax[NCG][TILE];    // per-patch partial max |y| of the pixel groups
     float xsum[NCG][TILE];    // per-patch partial sum of valid row norms (in-kernel 4||H||_F^2)
-    uint32_t xrow[TILE];      // validity bits of window column 0 (pixels 0..7)
+    uint32_t xrow[NCG][TILE]; // validity bits of window column 0, the rows of each column group
+    uint32_t rowor[2][FIRST_EPI - 1];   // per gather warp, by tile parity: window rows observed by a patch of the tile
     float rn[64];             // ||Dh[i,:]||^2 (normalised dictionary)
     uint32_t dmax_bits;       // max |D| as float bits
 };
@@ -192,7 +200,40 @@ struct TilePlan {
     int64_t items;         // rblocks * cchunks
     int cchunks, cpc;      // chunks per row block, column starts per chunk
     unsigned* counter;     // device word, zero at launch: next unclaimed work item (nullptr: static round-robin deal)
+    const int* order;      // row starts in tile order, nR of them (nullptr: ascending)
 };
+
+// Row starts are ordered by the rank of their 8-row validity word in the reflected Gray code, so that consecutive
+// patterns differ in one row and a tile that straddles two patterns observes at most one row more than either.
+__host__ __device__ __forceinline__ uint32_t pattern_rank(uint32_t w) {
+    w ^= w >> 1;
+    w ^= w >> 2;
+    w ^= w >> 4;
+    return w;
+}
+
+// Window rows of a tile, from the OR w of the observed flags of its patches: the observed rows ascending, padded with
+// unobserved rows to an even count of at least 2, then the other rows; nibble j holds the j-th row.  GEMM-B k-step s
+// (s < nks = half the padded count) takes the rows of nibbles 2s, 2s+1.  Padding rows are unobserved by every patch of
+// the tile, so their residual is exactly zero.
+__device__ __forceinline__ uint32_t tile_rows(uint32_t w, int& nks) {
+    w &= 0xFFu;
+    int c = __popc(w);
+    while (c < 2 || (c & 1)) {
+        w |= ~w & (w + 1);            // lowest unobserved row
+        ++c;
+    }
+    nks = c >> 1;
+    uint32_t list = 0;
+    int j = 0;
+#pragma unroll
+    for (int r = 0; r < 8; ++r)
+        if ((w >> r) & 1u) list |= (uint32_t)r << (4 * j++);
+#pragma unroll
+    for (int r = 0; r < 8; ++r)
+        if (!((w >> r) & 1u)) list |= (uint32_t)r << (4 * j++);
+    return list;
+}
 
 // The walker also compiles for the host (lrs_debug_tile_walk below replays a launch's tile order on the CPU, so the
 // no-GPU test suite covers this integer logic); on the device the CTA index and the grid size stay special registers.
@@ -268,28 +309,42 @@ struct TileWalk {
                     continue;
                 }
             }
-            const int64_t r0 = (int64_t)rb * TILE, r1 = r0 + TILE < nR ? r0 + TILE : nR;
+            // an ordered tile holds row starts from anywhere in its column: it is walked when the column meets the range
+            int64_t r0 = 0, r1 = nR;
+            if (!pl.order) {
+                r0 = (int64_t)rb * TILE;
+                r1 = r0 + TILE < nR ? r0 + TILE : nR;
+            }
             if (ci * nR + r1 > prm.p_begin && ci * nR + r0 < prm.p_end) return true;
         }
     }
 };
 
-// Lane m of the current tile: its patch (clamped to some patch of the range when the lane is idle, so that it computes
-// finite garbage and stores nothing), the window origin and the Phi_z column.
+// Lane m of the current tile: its patch, the window origin and the Phi_z column.  A lane is idle (stores nothing) when its
+// patch lies outside [p_begin, p_end): it still computes its own patch, whose observed rows join the tile's row set, so
+// that the row set, and with it every result, does not depend on the launch's range.  A lane past the last row start
+// computes some patch of the range (finite garbage) and adds nothing to the row set.
 struct PatchRef {
     int64_t p, pi, rs, cs;
     bool valid;
 };
-__host__ __device__ __forceinline__ PatchRef tile_patch(const FusedParams& prm, const TileWalk& tw, int m) {
+__host__ __device__ __forceinline__ PatchRef tile_patch(const FusedParams& prm, const TilePlan& pl, const TileWalk& tw, int m) {
     const int64_t nR = prm.g.row.n;
     int64_t ci = tw.ci, ri = (int64_t)tw.rb * TILE + m;
+    if (pl.order && ri < nR) {
+#ifdef __CUDA_ARCH__
+        ri = __ldg(pl.order + ri);
+#else
+        ri = pl.order[ri];
+#endif
+    }
     int64_t p = ci * nR + ri;
     PatchRef r;
     r.valid = ri < nR && p >= prm.p_begin && p < prm.p_end;
     r.pi = p - prm.p_begin;
-    if (!r.valid) {
+    if (ri >= nR) {
         p = p < prm.p_begin ? prm.p_begin : prm.p_end - 1;
-        if (ri >= nR && tw.ci * nR + nR - 1 >= prm.p_begin && tw.ci * nR + nR - 1 < prm.p_end) p = tw.ci * nR + nR - 1;
+        if (tw.ci * nR + nR - 1 >= prm.p_begin && tw.ci * nR + nR - 1 < prm.p_end) p = tw.ci * nR + nR - 1;
         ci = p / nR;
         ri = p - ci * nR;
     }
@@ -348,7 +403,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) sparse_fused_tc_kernel(FusedParam
     }
     const float sd = ldexpf(1.0f, -dex);
     for (int e = tid; e < 64 * KATOMS; e += NTHREADS) {
-        int i = e / KATOMS, k = e % KATOMS;
+        const int ir = e / KATOMS, k = e % KATOMS, i = 8 * (ir % 8) + ir / 8;   // reference pixel row + 8 col -> kernel pixel
         float v = prm.D[e] * (sd * S_D);
         __half h1 = __float2half_rn(v);
         __half h2 = __float2half_rn(v - __half2float(h1));
@@ -362,7 +417,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) sparse_fused_tc_kernel(FusedParam
             float d = prm.D[tid * KATOMS + k] * sd;
             s = fmaf(d, d, s);
         }
-        sh.rn[tid] = s;                                  // ||Dh[i,:]||^2
+        sh.rn[8 * (tid % 8) + tid / 8] = s;              // ||Dh[i,:]||^2, kernel pixel order
     }
     if (tid == 0) {
         mbar_init(&sh.bar_B[0], 1);
@@ -397,8 +452,9 @@ __global__ void __launch_bounds__(NTHREADS, 1) sparse_fused_tc_kernel(FusedParam
         const uint32_t idescA128 = make_idesc_f16(128, 128, false);
         const uint32_t idescA64 = make_idesc_f16(128, 64, false);
         // GEMM-B: B = D as (N = atoms, K = pixels), MN-major: 16-byte atom chunks SBO = D_SK apart, 8-pixel groups
-        //         LBO = D_SI apart; k-step ks covers pixel groups 2ks, 2ks+1 of piece p.
-        const uint64_t descB0 = make_smem_desc(dbase, /*lbo=*/D_SI, /*sbo=*/D_SK);
+        //         LBO = D_SI apart; k-step s covers the pixel groups (window rows) a < b of the tile's row list: its
+        //         descriptor starts at group a with LBO = (b - a) D_SI.
+        const uint64_t descB0 = make_smem_desc(dbase, /*lbo=*/0, /*sbo=*/D_SK);
         // GEMM-A: B = D as (N = pixels [D1;D2], K = atoms), K-major: 16-byte atom chunks LBO = D_SK apart, 8-pixel
         //         groups SBO = D_SI apart; k-step covers atom groups 2g, 2g+1.
         const uint64_t descA0 = make_smem_desc(dbase, /*lbo=*/D_SK, /*sbo=*/D_SI);
@@ -408,7 +464,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) sparse_fused_tc_kernel(FusedParam
         // Dynamic instance: the MMA warp does not walk the tiles (it needs no coordinates); the gather warps announce every tile
         // they find and the vote makes the loop condition warp-uniform.  Static instance: the walker itself (all uniform).
         TileWalk twm;
-        uint32_t nt = 0;
+        uint32_t nt = 0, tcount = 0;
         auto more_tiles = [&]() -> bool {
             if constexpr (DYN) {
                 uint32_t have;
@@ -428,15 +484,20 @@ __global__ void __launch_bounds__(NTHREADS, 1) sparse_fused_tc_kernel(FusedParam
                 return twm.next<false>(plan, prm);
             }
         };
-        while (more_tiles()) {
+        for (; more_tiles(); ++tcount) {
+            // The tile's row list: its row word was published with the gather, before the epilogue staged this tile's
+            // first residual k-step (at least one k-step is always issued).
+            mbar_wait(&sh.bar_R[0], gi & 1);
+            int nks;
+            const uint32_t rl = tile_rows(sh.rowor[tcount & 1][0] | sh.rowor[tcount & 1][1] | sh.rowor[tcount & 1][2], nks);
             for (int it = 0; it < Nit; ++it, ++gi) {
                 const uint32_t par = gi & 1;
-                // ---- GEMM-B: state += r D; k-step ks (16 pixels) starts as soon as its residual quarter is staged ----
+                // ---- GEMM-B: state += r D; k-step ks (two window rows) starts as soon as its residual is staged ----
                 {
                     const uint32_t idescB128 = make_idesc_f16(128, KH, /*b_mn_major=*/true);
                     const uint64_t descR0 = make_smem_desc(smem_u32(Rsm), /*lbo=*/R_SK, /*sbo=*/R_SM);
                     // Half 0 takes every k-step as soon as its residual quarter is staged (its completion releases the first
-                    // soft-threshold chunks), then half 1 runs all four k-steps.
+                    // soft-threshold chunks), then half 1 runs the tile's nks k-steps.
 #pragma unroll
                     for (int half = 0; half < 2; ++half) {
 #pragma unroll
@@ -447,20 +508,25 @@ __global__ void __launch_bounds__(NTHREADS, 1) sparse_fused_tc_kernel(FusedParam
                                 if (DBG) dbg[1 + ks] += clock64() - w0;
                                 tc_fence_after();
                             }
-                            const uint64_t d1 = descB0 + (uint64_t)(((0 * 8 + 2 * ks) * D_SI + half * (KH / 8) * D_SK) >> 4);
-                            const uint64_t d2 = descB0 + (uint64_t)(((1 * 8 + 2 * ks) * D_SI + half * (KH / 8) * D_SK) >> 4);
-                            const uint64_t r1 = descR0 + (uint64_t)((2 * ks * R_SK) >> 4);
-                            const uint64_t r2 = descR0 + (uint64_t)((R_PIECE + 2 * ks * R_SK) >> 4);
-                            const uint32_t acc = tbase + COL_ALPHA + KH * half;
-                            if (leader) {
-                                mma_f16_ss(acc, r1, d1, idescB128, !(it == 0 && ks == 0));
-                                mma_f16_ss(acc, r2, d1, idescB128, true);
-                                mma_f16_ss(acc, r1, d2, idescB128, true);
+                            if (ks < nks) {
+                                const uint32_t ra = (rl >> (8 * ks)) & 15u, rw = (rl >> (8 * ks + 4)) & 15u;
+                                const uint64_t dk = (uint64_t)((ra * D_SI + half * (KH / 8) * D_SK) >> 4) |
+                                                    ((uint64_t)(((rw - ra) * D_SI) >> 4) << 16);   // LBO: group b
+                                const uint64_t d1 = descB0 + dk;
+                                const uint64_t d2 = descB0 + dk + (uint64_t)((8 * D_SI) >> 4);
+                                const uint64_t r1 = descR0 + (uint64_t)((2 * ks * R_SK) >> 4);
+                                const uint64_t r2 = descR0 + (uint64_t)((R_PIECE + 2 * ks * R_SK) >> 4);
+                                const uint32_t acc = tbase + COL_ALPHA + KH * half;
+                                if (leader) {
+                                    mma_f16_ss(acc, r1, d1, idescB128, !(it == 0 && ks == 0));
+                                    mma_f16_ss(acc, r2, d1, idescB128, true);
+                                    mma_f16_ss(acc, r1, d2, idescB128, true);
+                                }
                             }
                             __syncwarp();
-                            if (ks == 3 && leader) mma_commit(&sh.bar_B[half]);     // last group of the half
-                            __syncwarp();
                         }
+                        if (leader) mma_commit(&sh.bar_B[half]);
+                        __syncwarp();
                     }
                 }
                 // ---- GEMM-A: Da = state D^T, chunk by chunk as the soft-threshold epilogue releases them ----
@@ -525,45 +591,60 @@ __global__ void __launch_bounds__(NTHREADS, 1) sparse_fused_tc_kernel(FusedParam
         const long long e_begin = TSTAMP();
         for (TileWalk tw; tw.next<DYN>(plan, prm, &sh);) {
             const long long tp0 = TSTAMP();
-            // ---- tile prologue: gather my CW pixels, mask, step constant, scale.  Register slot c holds pixel
-            //      16*(c/8) + 8*cg + c%8 = window row c%8, column 2*(c/8) + cg: every 16-pixel GEMM-B k-step is shared by
-            //      the two column groups, so that all warps finish quarter ks together and its MMAs start early ----
-            const PatchRef pr = tile_patch(prm, tw, m);
+            // ---- tile prologue: gather my CW pixels, mask, step constant, scale.  Register slot c holds window row
+            //      row(2*(c/8) + cg) of the tile's row list, column c%8: GEMM-B k-step s is shared by the two column
+            //      groups (one row each), so that all warps finish it together and its MMAs start early ----
+            const PatchRef pr = tile_patch(prm, plan, tw, m);
             const bool valid = pr.valid;
             const int64_t pi = pr.pi, p = pr.p;                 // Phi_z column; patch for the step constant
             float ysc[CW];
             uint32_t mbits = 0;
             float amax = 0.f, nsum = 0.f;
             mbar_wait(&sh.bar_G_full, tcount & 1);              // gathered by warps 1..3 during the previous tile
+            // byte s of rlc: my row of k-step s in bits 0-3, bit 7 set when the tile issues k-step s
+            uint32_t rlc;
+            {
+                int nks;
+                const uint32_t rl = tile_rows(sh.rowor[tcount & 1][0] | sh.rowor[tcount & 1][1] | sh.rowor[tcount & 1][2], nks);
+                rlc = (rl >> (4 * cg)) & 0x0F0F0F0Fu;
+#pragma unroll
+                for (int s4 = 0; s4 < 4; ++s4)
+                    if (s4 < nks) rlc |= 0x80u << (8 * s4);
+            }
 #pragma unroll
             for (int c = 0; c < CW; ++c) {
-                const int pix = 16 * (c >> 3) + NPX * cg + (c & 7);
+                const int pix = 8 * (int)((rlc >> (8 * (c >> 3))) & 15u) + (c & 7);
                 const float v = Gv[pix * TILE + m];
                 const bool ok = Gok[pix * TILE + m] != 0;
                 ysc[c] = v;
                 if (ok) {
                     mbits |= 1u << c;
                     amax = fmaxf(amax, fabsf(v));
-                    nsum += sh.rn[16 * (c >> 3) + NPX * cg + (c & 7)];
+                    nsum += sh.rn[pix];
                 }
             }
+            uint32_t xr = 0;                                    // window column 0 of my rows
+#pragma unroll
+            for (int s4 = 0; s4 < 4; ++s4) xr |= ((mbits >> (8 * s4)) & 1u) << ((rlc >> (8 * s4)) & 15u);
             __syncwarp();
             if (lane == 0) mbar_arrive(&sh.bar_G_free);         // the loader may fetch the next tile
             ++tcount;
             sh.xmax[cg][m] = amax;
             sh.xsum[cg][m] = nsum;
-            if (cg == 0) sh.xrow[m] = mbits & 0xFFu;
+            sh.xrow[cg][m] = xr;
             epi_barrier();
             float a = 0.f;
             amax = 0.f;
+            uint32_t xrow = 0;
 #pragma unroll
             for (int g2 = 0; g2 < NCG; ++g2) {
                 amax = fmaxf(amax, sh.xmax[g2][m]);
                 a += sh.xsum[g2][m];
+                xrow |= sh.xrow[g2][m];
             }
             a *= 4.0f;                                              // 4 ||H||_F^2 (main_LRS_PnP_DIP_pro.py:190)
             if (prm.a_patch) a = __ldg(prm.a_patch + p) * (sd * sd);          // caller's a refers to D: a_h = a sd^2
-            else if (prm.a_table) a = __ldg(prm.a_table + sh.xrow[m]) * (sd * sd);
+            else if (prm.a_table) a = __ldg(prm.a_table + xrow) * (sd * sd);
             epi_barrier();  // exchange buffers are free for the next tile
             const bool ok_a = a > 0.0f;
             const float inv_a = ok_a ? __fdiv_rn(1.0f, a) : 0.0f;
@@ -579,11 +660,13 @@ __global__ void __launch_bounds__(NTHREADS, 1) sparse_fused_tc_kernel(FusedParam
 #pragma unroll
             for (int c = 0; c < CW; ++c) ysc[c] = ((mbits >> c) & 1u) ? ysc[c] * c1 : 0.f;    // y' stored masked
             const uint64_t nc2 = pk2(-c2, -c2);
-            // slot c holds window row c % 8 (see above): with a band-replicated mask bit c % 8 speaks for slot c
-            uint64_t nc2m[NPX / 2];
+            // slots 8s .. 8s+7 hold one window row (see above): with a band-replicated mask bit 8s speaks for all of them
+            uint64_t nc2m[4];
 #pragma unroll
-            for (int c = 0; c < NPX / 2; ++c)
-                nc2m[c] = pk2(((mbits >> (2 * c)) & 1u) ? -c2 : 0.f, ((mbits >> (2 * c + 1)) & 1u) ? -c2 : 0.f);
+            for (int s4 = 0; s4 < 4; ++s4) {
+                const float v = ((mbits >> (8 * s4)) & 1u) ? -c2 : 0.f;
+                nc2m[s4] = pk2(v, v);
+            }
             if (DBG) ed[7] += clock64() - tp0;
 
             for (int it = 0; it < Nit; ++it, ++gi) {
@@ -597,42 +680,47 @@ __global__ void __launch_bounds__(NTHREADS, 1) sparse_fused_tc_kernel(FusedParam
                     tc_fence_after();
                 }
                 // FOLD: band-replicated masks (validity depends on the window row only), so the mask is folded into four
-                // packed constants nc2m[row pair] = -c2 .* m and into y' itself: r = y'm - (c2 m) Da needs no per-element
+                // packed constants nc2m[s] = -c2 .* m and into y' itself: r = y'm - (c2 m) Da needs no per-element
                 // select (the selects run on the half-rate ALU pipe that bounds the epilogue).
+                // K-steps past the tile's nks are not issued: their barriers are only arrived on, so that every quarter
+                // barrier keeps one phase per iteration.
 #pragma unroll
-                for (int ks = 0; ks < 4; ++ks) {             // pixel quarter = GEMM-B k-step; my NPX pixels of it
-                    uint32_t p1[NPX / 2], p2[NPX / 2];
-                    if (it > 0) {
-                        uint32_t b0[NPX], b1[NPX];
-                        tmem_ld8(lane_addr + COL_ACC + 16 * ks + NPX * cg, b0);
-                        tmem_ld8(lane_addr + COL_ACC + 64 + 16 * ks + NPX * cg, b1);
-                        tmem_wait_ld();
+                for (int ks = 0; ks < 4; ++ks) {             // GEMM-B k-step = two window rows; my row of it
+                    if ((rlc >> (8 * ks + 7)) & 1u) {
+                        uint32_t p1[NPX / 2], p2[NPX / 2];
+                        if (it > 0) {
+                            uint32_t b0[NPX], b1[NPX];
+                            const uint32_t col = COL_ACC + 8 * ((rlc >> (8 * ks)) & 15u);
+                            tmem_ld8(lane_addr + col, b0);
+                            tmem_ld8(lane_addr + col + 64, b1);
+                            tmem_wait_ld();
 #pragma unroll
-                        for (int c = 0; c < NPX / 2; ++c) {
-                            const int e = NPX * ks + 2 * c;
-                            const uint64_t sm2 = add2(pk2(__uint_as_float(b0[2 * c]), __uint_as_float(b0[2 * c + 1])),
-                                                      pk2(__uint_as_float(b1[2 * c]), __uint_as_float(b1[2 * c + 1])));
-                            float r0, r1;
-                            upk2(fma2(FOLD ? nc2m[c] : nc2, sm2, pk2(ysc[e], ysc[e + 1])), r0, r1);
-                            if (!FOLD) {
-                                r0 = ((mbits >> e) & 1u) ? r0 : 0.f;
-                                r1 = ((mbits >> (e + 1)) & 1u) ? r1 : 0.f;
+                            for (int c = 0; c < NPX / 2; ++c) {
+                                const int e = NPX * ks + 2 * c;
+                                const uint64_t sm2 = add2(pk2(__uint_as_float(b0[2 * c]), __uint_as_float(b0[2 * c + 1])),
+                                                          pk2(__uint_as_float(b1[2 * c]), __uint_as_float(b1[2 * c + 1])));
+                                float r0, r1;
+                                upk2(fma2(FOLD ? nc2m[ks] : nc2, sm2, pk2(ysc[e], ysc[e + 1])), r0, r1);
+                                if (!FOLD) {
+                                    r0 = ((mbits >> e) & 1u) ? r0 : 0.f;
+                                    r1 = ((mbits >> (e + 1)) & 1u) ? r1 : 0.f;
+                                }
+                                split_pair(r0, r1, p1[c], p2[c]);
                             }
-                            split_pair(r0, r1, p1[c], p2[c]);
-                        }
-                    } else {
+                        } else {
 #pragma unroll
-                        for (int c = 0; c < NPX / 2; ++c) {
-                            const int e = NPX * ks + 2 * c;
-                            split_pair(ysc[e], ysc[e + 1], p1[c], p2[c]);   // y' is stored masked
+                            for (int c = 0; c < NPX / 2; ++c) {
+                                const int e = NPX * ks + 2 * c;
+                                split_pair(ysc[e], ysc[e + 1], p1[c], p2[c]);   // y' is stored masked
+                            }
                         }
+                        // my 8 pixels = k-group 2ks + cg of my row m: one 16-byte store per piece (a warp covers 512
+                        // contiguous bytes per store: conflict-free), then publish to the async proxy
+                        uint8_t* rrow = Rsm + (uint32_t)(m >> 3) * R_SM + (uint32_t)(m & 7) * 16 + (uint32_t)(NCG * ks + cg) * R_SK;
+                        *reinterpret_cast<uint4*>(rrow) = make_uint4(p1[0], p1[1], p1[2], p1[3]);
+                        *reinterpret_cast<uint4*>(rrow + R_PIECE) = make_uint4(p2[0], p2[1], p2[2], p2[3]);
+                        fence_async_smem();
                     }
-                    // my 8 pixels = k-group 2ks + cg of my row m: one 16-byte store per piece (a warp covers 512 contiguous
-                    // bytes per store: conflict-free), then publish to the async proxy
-                    uint8_t* rrow = Rsm + (uint32_t)(m >> 3) * R_SM + (uint32_t)(m & 7) * 16 + (uint32_t)(NCG * ks + cg) * R_SK;
-                    *reinterpret_cast<uint4*>(rrow) = make_uint4(p1[0], p1[1], p1[2], p1[3]);
-                    *reinterpret_cast<uint4*>(rrow + R_PIECE) = make_uint4(p2[0], p2[1], p2[2], p2[3]);
-                    fence_async_smem();
                     tc_fence_before();
                     __syncwarp();
                     if (lane == 0) mbar_arrive(&sh.bar_R[ks]);
@@ -734,9 +822,10 @@ __global__ void __launch_bounds__(NTHREADS, 1) sparse_fused_tc_kernel(FusedParam
                 tc_fence_before();   // order these loads before the next tile's MMAs (via bar_R)
                 const float sc = up * inv_a / (S_ALPHA * S_D);
                 if (valid) {
+                    // slot c = kernel pixel 16*(c/8) + NPX*cg + c%8 = window row 2*(c/8) + cg, column c%8
 #pragma unroll
                     for (int c = 0; c < CW; ++c)
-                        __stcs(prm.phi + (int64_t)(16 * (c >> 3) + NPX * cg + (c & 7)) * total + pi,
+                        __stcs(prm.phi + (int64_t)(2 * (c >> 3) + cg + 8 * (c & 7)) * total + pi,
                                (__uint_as_float(a0[c]) + __uint_as_float(a1[c])) * sc);   // streaming: keep the cube in L2
                 }
             }
@@ -756,13 +845,15 @@ __global__ void __launch_bounds__(NTHREADS, 1) sparse_fused_tc_kernel(FusedParam
         for (TileWalk tw; tw.next<DYN>(plan, prm, &sh); ++t) {
             if (DYN && tid == 32) *(volatile uint32_t*)&sh.tiles_pub = t + 1;      // announce the tile to the MMA warp
             if (t > 0) mbar_wait(&sh.bar_G_free, (t - 1) & 1);
+            uint32_t rows = 0;                            // window rows with an observed entry in a patch of the tile
             for (int m = lt; m < TILE; m += NLOAD) {
-                const PatchRef pr = tile_patch(prm, tw, m);
+                const PatchRef pr = tile_patch(prm, plan, tw, m);
+                const bool own = (int64_t)tw.rb * TILE + m < prm.g.row.n;   // the lane holds a patch of the tile
                 const float* xs = prm.X + pr.rs * C + pr.cs;
                 const float* ys = prm.Yobs + pr.rs * C + pr.cs;
                 const float* ls = prm.L ? prm.L + pr.rs * C + pr.cs : nullptr;
 #pragma unroll 2
-                for (int j = 0; j < 8; ++j) {            // window column j: pixels 8j .. 8j+7 = rows 0..7
+                for (int j = 0; j < 8; ++j) {            // window column j: kernel pixels j, 8 + j, .. 56 + j = rows 0..7
                     float v[8], o[8];
 #pragma unroll
                     for (int i = 0; i < 8; ++i) {
@@ -775,11 +866,14 @@ __global__ void __launch_bounds__(NTHREADS, 1) sparse_fused_tc_kernel(FusedParam
                     }
 #pragma unroll
                     for (int i = 0; i < 8; ++i) {
-                        Gv[(8 * j + i) * TILE + m] = v[i];
-                        Gok[(8 * j + i) * TILE + m] = o[i] != 0.0f ? 1 : 0;
+                        Gv[(8 * i + j) * TILE + m] = v[i];
+                        Gok[(8 * i + j) * TILE + m] = o[i] != 0.0f ? 1 : 0;
+                        if (own && o[i] != 0.0f) rows |= 1u << i;
                     }
                 }
             }
+            rows = __reduce_or_sync(0xffffffffu, rows);
+            if (lane == 0) sh.rowor[t & 1][warp - 1] = rows;   // tile t-2, the last reader of this slot, is done
             __syncwarp();
             if (lane == 0) mbar_arrive(&sh.bar_G_full);
         }
@@ -791,6 +885,75 @@ __global__ void __launch_bounds__(NTHREADS, 1) sparse_fused_tc_kernel(FusedParam
     tc_fence_before();
     __syncthreads();
     if (warp == 1) tmem_dealloc(tbase, 512);
+}
+
+// ---- tile order of the step-constant table mode: row starts sorted by the Gray rank of their row-validity word ----
+// The word uses the same bits as the table index (Yobs != 0 in the window's rows, column 0: table mode asserts
+// band-replicated masks).  The order only decides which patches share a tile, never a result: the kernel derives a
+// tile's row set from the gathered flags themselves.
+__global__ void row_pattern_keys_kernel(const float* __restrict__ Yobs, Geom g, uint8_t* __restrict__ key) {
+    const int64_t ri = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (ri >= g.row.n) return;
+    const float* y = Yobs + g.row.start(ri) * g.C;
+    uint32_t w = 0;
+#pragma unroll
+    for (int i = 0; i < 8; ++i) w |= (__ldg(y + i * g.C) != 0.0f ? 1u : 0u) << i;
+    key[ri] = (uint8_t)pattern_rank(w);
+}
+
+// Stable counting sort of n one-byte keys: CTA k writes the row starts with key k, ascending, after the count of smaller
+// keys.  Thread t of every CTA reads the t-th contiguous share of the key array (the array is padded to a multiple of 16)
+// twice, 16 keys per load: ~0.5 MB per CTA from L2 for the 262137 row starts of a 512 x 512 cube.  The result does not
+// depend on timing, so every launch of a range sees the same tiles.
+constexpr int SORT_THREADS = 1024;
+__device__ __forceinline__ uint32_t key_matches(const uint8_t* key, int64_t n, int64_t i0, uint32_t k, bool below) {
+    const uint4 v = __ldg(reinterpret_cast<const uint4*>(key + i0));
+    const uint32_t w[4] = {v.x, v.y, v.z, v.w};
+    uint32_t bits = 0;
+#pragma unroll
+    for (int j = 0; j < 16; ++j) {
+        const uint32_t kj = (w[j >> 2] >> (8 * (j & 3))) & 0xFFu;
+        if (i0 + j < n && (below ? kj < k : kj == k)) bits |= 1u << j;
+    }
+    return bits;
+}
+// exclusive prefix of v over the CTA; total receives the sum (every thread)
+__device__ __forceinline__ uint32_t cta_exclusive_scan(uint32_t v, uint32_t* wsum, uint32_t& total) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    uint32_t inc = v;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+        const uint32_t t = __shfl_up_sync(0xffffffffu, inc, d);
+        if (lane >= d) inc += t;
+    }
+    if (lane == 31) wsum[warp] = inc;
+    __syncthreads();
+    uint32_t before = 0;
+    total = 0;
+    for (int w = 0; w < SORT_THREADS / 32; ++w) {
+        const uint32_t t = wsum[w];
+        before += w < warp ? t : 0u;
+        total += t;
+    }
+    __syncthreads();   // wsum is reused by the next call
+    return before + inc - v;
+}
+__global__ void __launch_bounds__(SORT_THREADS) row_order_kernel(const uint8_t* __restrict__ key, int64_t n, int* __restrict__ order) {
+    __shared__ uint32_t wsum[SORT_THREADS / 32];
+    const uint32_t k = blockIdx.x;
+    const int64_t share = ((n + 16 * SORT_THREADS - 1) / (16 * SORT_THREADS)) * 16;
+    const int64_t b = share * threadIdx.x, e = b + share < n ? b + share : n;
+    uint32_t below = 0, mine = 0, total, base;
+    for (int64_t i0 = b; i0 < e; i0 += 16) {
+        below += __popc(key_matches(key, n, i0, k, true));
+        mine += __popc(key_matches(key, n, i0, k, false));
+    }
+    uint32_t pos = cta_exclusive_scan(mine, wsum, total);
+    if (total == 0) return;
+    (void)cta_exclusive_scan(below, wsum, base);
+    pos += base;
+    for (int64_t i0 = b; i0 < e; i0 += 16)
+        for (uint32_t bits = key_matches(key, n, i0, k, false); bits; bits &= bits - 1) order[pos++] = (int)(i0 + __ffs(bits) - 1);
 }
 
 }  // namespace
@@ -817,6 +980,7 @@ static TilePlan make_tile_plan(const FusedParams& prm, int sms) {
     plan.cchunks = (int)((ncols + plan.cpc - 1) / plan.cpc);   // no empty chunks: every work item holds tiles
     plan.items = rblocks * plan.cchunks;
     plan.counter = nullptr;
+    plan.order = nullptr;
     return plan;
 }
 
@@ -870,9 +1034,29 @@ static int launch_tc(const FusedParams& prm, bool dynamic_tiles, cudaStream_t st
     unsigned grid = (unsigned)(plan.items < sms ? plan.items : sms);
     plan.counter = dynamic_tiles ? claim_counter(st) : nullptr;
     if (dynamic_tiles && !plan.counter) return fail_arg(fn, "no claim counter for the dynamic tile schedule");
+    // table mode: tiles of row starts with one row-validity pattern, so that GEMM-B and the residual skip the rows none of
+    // a tile's patches observes.  Scratch is stream-ordered on the launch stream.
+    const int64_t nR = prm.g.row.n;
+    void* scratch = nullptr;
+    if (fold) {
+        if (nR >= ((int64_t)1 << 30)) return fail_arg(fn, "too many row starts for the row-pattern tile order");
+        const int64_t nkey = (nR + 15) / 16 * 16;
+        rc = check_cuda(fn, cudaMallocAsync(&scratch, (size_t)nkey * 5, st));
+        if (rc != LRS_OK) return rc;
+        int* order = static_cast<int*>(scratch);
+        uint8_t* key = reinterpret_cast<uint8_t*>(order + nkey);
+        row_pattern_keys_kernel<<<(unsigned)((nR + 255) / 256), 256, 0, st>>>(prm.Yobs, prm.g, key);
+        row_order_kernel<<<256, SORT_THREADS, 0, st>>>(key, nR, order);
+        plan.order = order;
+    }
     kern<<<grid, NTHREADS, smem, st>>>(prm, plan);
     note_launch();
-    return check_cuda(fn, cudaGetLastError());
+    rc = check_cuda(fn, cudaGetLastError());
+    if (scratch) {
+        const int rc2 = check_cuda(fn, cudaFreeAsync(scratch, st));
+        if (rc == LRS_OK) rc = rc2;
+    }
+    return rc;
 }
 
 int sparse_fused_tc_launch(const FusedParams& prm, int K, bool dynamic_tiles, cudaStream_t st) {
@@ -895,34 +1079,68 @@ int tc_timing_read(unsigned long long* out32) {
 }  // namespace lrs
 
 #ifdef LRS_DIAGNOSTICS
+#include <algorithm>
+#include <numeric>
+#include <vector>
+
 #include "../../include/lrs_pnp_diag.h"
 
 // Replays on the HOST the tile order a launch with `sms` SMs would use and counts how often every patch of
-// [p_begin, p_end) is owned by a valid lane (must be exactly once); idle lanes must point at a patch of the range.
-extern "C" int lrs_debug_tile_walk(int64_t R, int64_t C, int bb, int s, int64_t p_begin, int64_t p_end, int sms,
-                                   int* visits_host, int64_t* tiles_host) {
-    const char* fn = "lrs_debug_tile_walk";
+// [p_begin, p_end) is owned by a valid lane (must be exactly once); idle lanes must point at a patch of the matrix.
+// row_obs_host (R bytes, or null: ascending row starts) gives the observed rows of the table mode's row-pattern order,
+// which is returned in order_host (nR ints) when that is not null.
+static int tile_walk_replay(const char* fn, int64_t R, int64_t C, int bb, int s, int64_t p_begin, int64_t p_end, int sms,
+                            const uint8_t* row_obs_host, int* visits_host, int64_t* tiles_host, int* order_host) {
     lrs::FusedParams prm{};
     if (bb != 8 || !lrs::make_geom(R, C, bb, s, prm.g)) return lrs::fail_arg(fn, "need bb = 8 and a valid geometry");
     if (p_begin < 0 || p_end > prm.g.P || p_begin >= p_end || sms < 1 || !visits_host || !tiles_host)
         return lrs::fail_arg(fn, "bad range, sms or null pointer");
     prm.p_begin = p_begin;
     prm.p_end = p_end;
-    const lrs::TilePlan plan = lrs::make_tile_plan(prm, sms);
+    lrs::TilePlan plan = lrs::make_tile_plan(prm, sms);
+    std::vector<int> order;
+    if (row_obs_host) {
+        const int64_t nR = prm.g.row.n;
+        std::vector<uint8_t> key(nR);
+        for (int64_t ri = 0; ri < nR; ++ri) {
+            uint32_t w = 0;
+            for (int i = 0; i < 8; ++i) w |= (row_obs_host[prm.g.row.start(ri) + i] ? 1u : 0u) << i;
+            key[ri] = (uint8_t)lrs::pattern_rank(w);
+        }
+        order.resize(nR);
+        std::iota(order.begin(), order.end(), 0);
+        std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return key[a] < key[b]; });
+        if (order_host) std::copy(order.begin(), order.end(), order_host);
+        plan.order = order.data();
+    }
     const int64_t grid = plan.items < sms ? plan.items : sms;
     int64_t tiles = 0;
     for (int64_t cta = 0; cta < grid; ++cta) {
         for (lrs::TileWalk tw(cta, grid); tw.next(plan, prm); ++tiles) {
             for (int m = 0; m < lrs::TILE; ++m) {
-                const lrs::PatchRef pr = lrs::tile_patch(prm, tw, m);
+                const lrs::PatchRef pr = lrs::tile_patch(prm, plan, tw, m);
                 if (pr.valid) ++visits_host[pr.pi];
-                if (pr.p < p_begin || pr.p >= p_end || pr.rs < 0 || pr.rs + bb > R || pr.cs < 0 || pr.cs + bb > C)
-                    return lrs::fail_arg(fn, "a lane points outside the patch range or the matrix");
+                if (pr.p < 0 || pr.p >= prm.g.P || pr.rs < 0 || pr.rs + bb > R || pr.cs < 0 || pr.cs + bb > C)
+                    return lrs::fail_arg(fn, "a lane points outside the matrix");
             }
         }
     }
     *tiles_host = tiles;
     return LRS_OK;
+}
+
+extern "C" int lrs_debug_tile_walk(int64_t R, int64_t C, int bb, int s, int64_t p_begin, int64_t p_end, int sms,
+                                   int* visits_host, int64_t* tiles_host) {
+    return tile_walk_replay("lrs_debug_tile_walk", R, C, bb, s, p_begin, p_end, sms, nullptr, visits_host, tiles_host,
+                            nullptr);
+}
+
+extern "C" int lrs_debug_tile_walk_ordered(int64_t R, int64_t C, int bb, int s, int64_t p_begin, int64_t p_end, int sms,
+                                           const uint8_t* row_obs_host, int* visits_host, int64_t* tiles_host,
+                                           int* order_host) {
+    const char* fn = "lrs_debug_tile_walk_ordered";
+    if (!row_obs_host) return lrs::fail_arg(fn, "null row mask");
+    return tile_walk_replay(fn, R, C, bb, s, p_begin, p_end, sms, row_obs_host, visits_host, tiles_host, order_host);
 }
 
 extern "C" int lrs_tc_timing_read(unsigned long long* out32_host) {

@@ -281,7 +281,7 @@ class SparseCoder:
     # needs ~4 % more cycles: that first range is kept just long enough to cover the eigensolver (~2 ms), judged by the
     # kernel's rate on a B200.
     SHARED_START_SECONDS = 2.5e-3
-    FUSED_PATCH_ITERS_PER_S = 6.5e9
+    FUSED_PATCH_ITERS_PER_S = 6.7e9
 
     def _ranges(self, shared_start: bool = False):
         """Column-start ranges [(c0, c1), ...] of one sparse step, ascending and contiguous."""
